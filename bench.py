@@ -7,6 +7,9 @@ inequality example batched (n=50, p=1, 65,536 independent instances per GPU, see
     e2e   : the same through the host-buffer C-ABI call (pinned host memory; H2D + kernel + D2H inside the timed region)
 Multi-GPU: the path shards by instances with no collective (weak scaling: every rank solves its own B instances).
 `--impl reference` times the CPU oracle port of the reference (Julia is absent from this image) on all host cores.
+`--dump-outputs DIR` writes what the last timed step returned for rank 0's instances (x, obj_values, obj_len, lambda,
+term_*) as DIR/<name>.npy in float64, about 39 MB, all finite; the inputs are seeded, so two builds can be compared file
+for file.
 """
 import argparse
 import json
@@ -35,6 +38,19 @@ def make_inputs(rank, B):
     coeff = rng.standard_normal((B, N_VARS))
     x0 = np.zeros((B, N_VARS))
     return coeff, x0
+
+
+def dump_outputs(d, x, obj, olen, lam, term):
+    """One batched solve's results as float64 .npy files.  The solver leaves obj entries past an instance's history
+    length unwritten (it always records f(x0), so the length is at least 1): they are stored as the last recorded
+    objective, which keeps every value finite and loses nothing next to obj_len."""
+    os.makedirs(d, exist_ok=True)
+    H = obj.shape[1]
+    obj = obj[np.arange(obj.shape[0])[:, None], np.minimum(np.arange(H)[None, :], np.minimum(olen, H)[:, None] - 1)]
+    out = {"x": x, "obj_values": obj, "obj_len": olen, "lambda": lam}
+    out.update({"term_" + k: term[k] for k in term.dtype.names})
+    for k, v in out.items():
+        np.save(os.path.join(d, k + ".npy"), np.asarray(v, dtype=np.float64))
 
 
 def host_cores():
@@ -376,9 +392,11 @@ def run_reference(args):
     t0 = time.perf_counter()
     for k in range(args.steps):
         lo = (k * S) % (B_PER_GPU - S + 1)
-        O.optimize_batched("readme_ineq", n, 0, 1, x0[lo:lo + S], xl=-inf, xu=inf, fam_params=coeff[lo:lo + S],
-                           fam_stride=n, H=HIST, nthreads=nthreads)
+        res = O.optimize_batched("readme_ineq", n, 0, 1, x0[lo:lo + S], xl=-inf, xu=inf, fam_params=coeff[lo:lo + S],
+                                 fam_stride=n, H=HIST, nthreads=nthreads)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, *res[:5])
     value = S * args.steps / dt
     sample = "%d of the %d instances per step, %d steps, %d host threads" % (S, B_PER_GPU, args.steps, nthreads)
     line = {"impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
@@ -415,7 +433,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--skip-large", action="store_true", help="skip the secondary large-n (C5) section")
     ap.add_argument("--no-numa-bind", action="store_true", help="N > 1: do not bind each rank to the CPUs next to its GPU (A/B)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's results for rank 0's instances as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
         return
@@ -521,6 +542,9 @@ def main():
     step_ms = [a.elapsed_time(b) for a, b in ev]
     total_ms = max_over_ranks(float(sum(step_ms)))
     value = world * B * K / (total_ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, d_x.cpu().numpy(), d_obj.cpu().numpy(), d_len.cpu().numpy(), d_lam.cpu().numpy(),
+                     np.frombuffer(d_term.cpu().numpy().tobytes(), dtype=_lib.TERM_DTYPE))
 
     # ---- end-to-end through the host-buffer C-ABI call (pinned host memory, copies inside the timed region)
     for _ in range(2):

@@ -2,6 +2,7 @@
 slack wrapper of src/optimize.jl:13-71 with explicit derivatives (checked against the oracle's family callbacks and by
 finite differences), method dispatch, and the loud failure without a GPU (no CPU fallback)."""
 import ctypes
+import multiprocessing as mp
 
 import numpy as np
 import pytest
@@ -86,11 +87,8 @@ def test_slack_wrapper_finite_differences():
     assert np.allclose(out, hfd, atol=1e-5 * max(1.0, np.abs(hfd).max()))
 
 
-def test_explicit_core_dispatch_and_no_cpu_fallback():
-    import torch
+def _explicit_core_dispatch_and_no_cpu_fallback():
     import lfpsqp.jl_b200 as L
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
     f = lambda x: float(x @ x)
     def grad(g, x): g[:] = 2 * x
     def hlv(dest, src, x, lam): dest[:] = 2 * src
@@ -103,3 +101,12 @@ def test_explicit_core_dispatch_and_no_cpu_fallback():
         L.optimize(f, grad, None, None, hlv, np.ones(3), None, None, 1)
     with pytest.raises(TypeError):                                                        # device-family path still demands a family handle
         L.optimize(f, np.ones(3))
+
+
+def test_explicit_core_dispatch_and_no_cpu_fallback(monkeypatch):
+    # in a child process that sees no GPU, so that the check runs on a GPU machine as well
+    monkeypatch.setenv("CUDA_VISIBLE_DEVICES", "")
+    p = mp.get_context("spawn").Process(target=_explicit_core_dispatch_and_no_cpu_fallback)
+    p.start()
+    p.join(300)
+    assert p.exitcode == 0
