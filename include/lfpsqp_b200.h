@@ -137,6 +137,10 @@ int lfpsqp_ctx_set_noise(lfpsqp_ctx *ctx, const double *noise, int64_t T, int64_
 /* device time (ms, CUDA events on the launching stream) and launch count of the kernels of the last solve call */
 double lfpsqp_last_kernel_ms(lfpsqp_ctx *ctx);
 int64_t lfpsqp_last_launches(lfpsqp_ctx *ctx);
+/* which batched kernel the last lfpsqp_solve_batched* call launched: out4 = {kind, LW, NPL, SPARSE} with kind 0 = one thread
+ * per instance (LW = 1), 1 = shared-memory warp solver (LW = 32), 2 = register-resident solver (LW lanes per instance, NPL
+ * elements per lane, SPARSE = 1 for the one-exception-per-lane bound layout); kind = -1 when the last call launched none */
+int lfpsqp_last_kernel(lfpsqp_ctx *ctx, int *out4);
 
 /*
  * Batched mode: B independent instances of optimize(f, c!, d!, x0, xl, xu, m, p, param)  (src/optimize.jl:83-85 and

@@ -34,7 +34,7 @@ EXPORTS = [
     "lfpsqp_comm_unique_id", "lfpsqp_comm_init", "lfpsqp_comm_destroy", "lfpsqp_large_retract", "lfpsqp_large_pcg",
     "lfpsqp_ineq_op", "lfpsqp_large_phase_ms", "lfpsqp_comm_ipc_export", "lfpsqp_comm_ipc_import", "lfpsqp_comm_mode",
     "lfpsqp_large_set_bounds", "lfpsqp_solve_host", "lfpsqp_linesearch", "lfpsqp_aug_hess_vec", "lfpsqp_large_projcg_general",
-    "lfpsqp_ctx_create_multi", "lfpsqp_ctx_device_count", "lfpsqp_ctx_set_noise",
+    "lfpsqp_ctx_create_multi", "lfpsqp_ctx_device_count", "lfpsqp_ctx_set_noise", "lfpsqp_last_kernel",
 ]
 
 _lib = None
@@ -55,6 +55,7 @@ def load():
         lib.lfpsqp_last_kernel_ms.argtypes = [C.c_void_p]
         lib.lfpsqp_last_launches.restype = C.c_int64
         lib.lfpsqp_last_launches.argtypes = [C.c_void_p]
+        lib.lfpsqp_last_kernel.argtypes = [C.c_void_p, C.POINTER(C.c_int)]
         lib.lfpsqp_ctx_create.argtypes = [C.c_int, C.POINTER(C.c_void_p)]
         lib.lfpsqp_ctx_destroy.argtypes = [C.c_void_p]
         lib.lfpsqp_ctx_create_multi.argtypes = [C.POINTER(C.c_int), C.c_int, C.POINTER(C.c_void_p)]
@@ -139,6 +140,14 @@ class Context:
     @property
     def last_launches(self):
         return self.lib.lfpsqp_last_launches(self.h)
+
+    @property
+    def last_kernel(self):
+        """(kind, LW, NPL, SPARSE) of the last batched launch: kind 0 thread per instance, 1 warp solver, 2 register
+        solver, -1 none"""
+        out = (C.c_int * 4)()
+        self.check(self.lib.lfpsqp_last_kernel(self.h, out))
+        return tuple(out)
 
 
 class MultiContext(Context):

@@ -121,6 +121,11 @@ extern "C" int lfpsqp_ctx_set_noise(lfpsqp_ctx *c, const double *noise, int64_t 
 }
 extern "C" double lfpsqp_last_kernel_ms(lfpsqp_ctx *c) { return c ? c->last_ms : -1.0; }
 extern "C" int64_t lfpsqp_last_launches(lfpsqp_ctx *c) { return c ? c->last_launches : 0; }
+extern "C" int lfpsqp_last_kernel(lfpsqp_ctx *c, int *out4) {
+  if (!c || !out4) return LFPSQP_ERR_ARG;
+  memcpy(out4, c->last_kernel, sizeof(c->last_kernel));
+  return LFPSQP_OK;
+}
 
 // ------------------------------------------------------------------ family registry
 namespace {
@@ -215,6 +220,7 @@ int launch_warp(lfpsqp_ctx *c, BatchedArgs &A, int use_nr) {
   cudaEventRecord(c->ev1, c->stream);
   c->last_launches = 1;
   c->last_cfg_warps = warps; c->last_cfg_grid = (int)grid; c->last_cfg_smem = (int)smem; c->last_cfg_resident = resident;
+  c->last_kernel[0] = 1; c->last_kernel[1] = 32; c->last_kernel[2] = 0; c->last_kernel[3] = 0;
   e = cudaGetLastError();
   if (e != cudaSuccess) return c->cuda_fail(e, "batched_warp_kernel launch");
   return LFPSQP_OK;
@@ -230,6 +236,7 @@ int launch_tiny(lfpsqp_ctx *c, BatchedArgs &A) {
   batched_tiny_kernel<Fam, NT><<<(unsigned)grid, threads, 0, c->stream>>>(A);
   cudaEventRecord(c->ev1, c->stream);
   c->last_launches = 1;
+  c->last_kernel[0] = 0; c->last_kernel[1] = 1; c->last_kernel[2] = 0; c->last_kernel[3] = 0;
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return c->cuda_fail(e, "batched_tiny_kernel launch");
   return LFPSQP_OK;
@@ -282,6 +289,7 @@ static int prepare_batched(lfpsqp_ctx *c, int family, int64_t n, int64_t m, int6
                            const double *xu, const lfpsqp_params *prm, int64_t H, BatchedArgs &A) {
   int rc = check_common(c, family, n, m, p, B, prm, H);
   if (rc) return rc;
+  c->last_kernel[0] = -1; c->last_kernel[1] = c->last_kernel[2] = c->last_kernel[3] = 0;
   cudaSetDevice(c->device);
   std::vector<double> &bnd = c->bnd_host;   // kept for the launcher (kernel selection looks at the bound kinds)
   bnd.clear();

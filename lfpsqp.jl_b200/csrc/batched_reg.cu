@@ -30,6 +30,7 @@ int launch(lfpsqp_ctx *c, BatchedArgs &A) {
   cudaEventRecord(c->ev1, c->stream);
   c->last_launches = 1;
   c->last_cfg_warps = NT / 32; c->last_cfg_grid = (int)grid; c->last_cfg_smem = (int)smem; c->last_cfg_resident = resident;
+  c->last_kernel[0] = 2; c->last_kernel[1] = LW; c->last_kernel[2] = NPL; c->last_kernel[3] = SPARSE ? 1 : 0;
   e = cudaGetLastError();
   if (e != cudaSuccess) return c->cuda_fail(e, "batched_reg_kernel launch");
   return LFPSQP_OK;

@@ -60,5 +60,6 @@ int solve_batched_multi(lfpsqp_ctx *c, int family, int64_t n, int64_t m, int64_t
     launches += c->children[g]->last_launches;
   }
   c->last_ms = ms_max; c->last_launches = launches;
+  std::copy(c->children[0]->last_kernel, c->children[0]->last_kernel + 4, c->last_kernel);   // every device runs the same kernel
   return rc;
 }
