@@ -90,6 +90,30 @@ enum {
 };
 
 /*
+ * Dense QCQP (batched mode only; lfpsqp_solve_large / lfpsqp_large_setup return LFPSQP_ERR_FAMILY for it):
+ *   f(x)   = 1/2 x'P x + q.x + r
+ *   c_i(x) = 1/2 x'Qc_i x + Ac_i.x - bc_i = 0      i < m
+ *   d_k(x) = 1/2 x'Qd_k x + Ad_k.x - bd_k <= 0     k < p
+ * Each array has a batch stride in doubles: 0 = shared by the whole batch, otherwise instance k reads ptr + k*stride
+ * (stride >= the array's element count).  NULL = all zero.  Matrices are n x n, symmetric, row-major (identical to
+ * column-major); stacks are m (or p) such matrices back to back.  Ac / Ad are m x n / p x n row-major (row i = a_i).
+ * lfpsqp_solve_batched takes host pointers and checks that every matrix is exactly symmetric; lfpsqp_solve_batched_dev
+ * takes device pointers and requires symmetric matrices.  The struct itself is host memory in both cases.
+ */
+typedef struct {
+  const double *P;  int64_t P_stride;    /* n*n   */
+  const double *q;  int64_t q_stride;    /* n     */
+  const double *r;  int64_t r_stride;    /* 1     */
+  const double *Qc; int64_t Qc_stride;   /* m*n*n */
+  const double *Ac; int64_t Ac_stride;   /* m*n   */
+  const double *bc; int64_t bc_stride;   /* m     */
+  const double *Qd; int64_t Qd_stride;   /* p*n*n */
+  const double *Ad; int64_t Ad_stride;   /* p*n   */
+  const double *bd; int64_t bd_stride;   /* p     */
+} lfpsqp_qcqp;
+#define LFPSQP_FAM_QCQP 101   /* fam_params = (const double*)(const lfpsqp_qcqp*), fam_stride must be 0 */
+
+/*
  * Host callbacks of the explicit-derivative core optimize(f, grad!, c!, jac!, hess_lag_vec!, x0, xl, xu, m, param)
  * (src/optimize.jl:119-143).  Conventions are the reference's (src/autodiff_generators.jl:7-9, :40-42, :80-104):
  * x is the first n entries of the working vector (optimize.jl:259 passes view(x, 1:n)); jac! fills Jc (m x n,
@@ -146,7 +170,8 @@ int lfpsqp_last_kernel(lfpsqp_ctx *ctx, int *out4);
  * Batched mode: B independent instances of optimize(f, c!, d!, x0, xl, xu, m, p, param)  (src/optimize.jl:83-85 and
  * the methods it forwards to, :13-71, :88-104, :119-443), solved in lockstep on one GPU, one warp (or one thread for
  * tiny unconstrained problems) per instance.
- *   fam_params : per-instance parameter blobs, instance k at fam_params + k*fam_stride (fam_stride 0 = shared)
+ *   fam_params : per-instance parameter blobs, instance k at fam_params + k*fam_stride (fam_stride 0 = shared);
+ *                LFPSQP_FAM_QCQP: a const lfpsqp_qcqp* cast to const double*, with fam_stride = 0
  *   x0         : n x B ; xl, xu : n (shared by the batch) or NULL (= `nothing`)
  *   x_out      : n x B ; obj_hist : H x B (first min(len,H) objective values) ; obj_len : B (iters+1)
  *   lambda     : (m+p) x B (untruncated, optimize.jl:67-70) ; term : B ; stats : B or NULL
@@ -166,7 +191,7 @@ int lfpsqp_solve_batched_dev(lfpsqp_ctx *ctx, int family, int64_t n, int64_t m, 
  * Large-n mode: ONE instance with a dense m x n constraint Jacobian, host-orchestrated whole-GPU kernels
  * (FP64 DMMA Gram + blocked Cholesky replace ksvd!, src/la_helper.jl:8-34 / optimize.jl:291-293; streaming passes over
  * J replace kgemv!, la_helper.jl:36-44).  Families: LFPSQP_FAM_DIAGQUAD, LFPSQP_FAM_THOMSON,
- * LFPSQP_FAM_HOST (params = const lfpsqp_host_callbacks*).  Finite bounds xl <= x <= xu run the reference's 2n-variable
+ * LFPSQP_FAM_HOST (params = const lfpsqp_host_callbacks*); LFPSQP_FAM_QCQP is LFPSQP_ERR_FAMILY here.  Finite bounds xl <= x <= xu run the reference's 2n-variable
  * embedding (src/inequality_helper.jl): lfpsqp_large_set_bounds after lfpsqp_large_setup, or the xl/xu arguments of
  * lfpsqp_solve_large / lfpsqp_solve_host.  projcg! on diagonal Lagrangian Hessians and pcg! run as persistent cooperative
  * kernels (large_fused.cu); LFPSQP_FUSED_PROJCG=0 in the environment selects the launch-per-phase loops.

@@ -20,6 +20,13 @@ class CParams(C.Structure):  # lfpsqp_params == LFPSQPParams, src/LFPSQP.jl:57-8
                 ("tn_maxiter", C.c_int64), ("tn_kappa", C.c_double), ("callback_period", C.c_int64)]
 
 
+QCQP_FIELDS = ("P", "q", "r", "Qc", "Ac", "bc", "Qd", "Ad", "bd")
+
+
+class CQcqp(C.Structure):  # lfpsqp_qcqp: nine {const double*, int64 batch stride} pairs
+    _fields_ = [f for name in QCQP_FIELDS for f in ((name, C.c_void_p), (name + "_stride", C.c_int64))]
+
+
 TERM_DTYPE = np.dtype([("condition", "<i4"), ("status", "<i4"), ("f_diff", "<f8"), ("step_diff", "<f8"),
                        ("kkt_diff", "<f8"), ("iter", "<i8")])
 STATS_FIELDS = ("projcg_iters", "projcg_negcurv", "armijo_trials", "retract_outer", "retract_pcg", "pp_backtracks",

@@ -6,7 +6,7 @@ from typing import NamedTuple
 import numpy as np
 
 from . import _lib
-from .families import DeviceCallback
+from .families import QCQP, DeviceCallback
 
 # LinesearchOption / DisplayOption (src/LFPSQP.jl:27-35)
 armijo, exact = 0, 1
@@ -143,12 +143,7 @@ def optimize_batched(*args, ctx=None, history=64, return_stats=False, noise=None
             raise _lib.LFPSQPError("xl, xu, and x0 must all be the same length")      # optimize.jl:144-148
     ctx = ctx or _lib.default_context()
     cp = param.to_c()
-    fp = fam.params
-    stride = 0
-    if fp is not None and fam.batched_params:
-        if fp.shape[0] != B:
-            raise _lib.LFPSQPError("per-instance family parameters must have B rows")
-        stride = fp.shape[1]
+    fp, stride, keep = fam.batched_args(B)
     H = int(history)
     x = np.empty((B, n)); obj = np.empty((B, H)); olen = np.zeros(B, dtype=np.int64)
     lam = np.zeros((B, m + p)); term = np.zeros(B, dtype=_lib.TERM_DTYPE)
@@ -158,9 +153,10 @@ def optimize_batched(*args, ctx=None, history=64, return_stats=False, noise=None
         if noise.ndim != 3 or noise.shape[0] != B:
             raise _lib.LFPSQPError("noise must have shape (B, T, N_working)")
         ctx.check(ctx.lib.lfpsqp_ctx_set_noise(ctx.h, _lib.ptr(noise), noise.shape[1], noise.shape[2], B))
-    rc = ctx.lib.lfpsqp_solve_batched(ctx.h, fam.id, n, m, p, B, _lib.ptr(fp), stride, _lib.ptr(x0), _lib.ptr(xl),
+    rc = ctx.lib.lfpsqp_solve_batched(ctx.h, fam.id, n, m, p, B, fp, stride, _lib.ptr(x0), _lib.ptr(xl),
                                       _lib.ptr(xu), C.cast(C.pointer(cp), C.c_void_p), _lib.ptr(x), _lib.ptr(obj), H,
                                       _lib.ptr(olen), _lib.ptr(lam), _lib.ptr(term), _lib.ptr(stats))
+    del keep
     if noise is not None:
         ctx.lib.lfpsqp_ctx_set_noise(ctx.h, None, 0, 0, 0)
     ctx.check(rc)
@@ -190,6 +186,9 @@ def optimize(*args, ctx=None, history=None, return_stats=False, noise=None):
     idx = {2: 1, 4: 2, 6: 2, 8: 3, 10: 5}.get(len(a))
     if idx is None:
         raise TypeError("no method matching optimize with %d positional arguments" % len(a))
+    if isinstance(a[0], DeviceCallback) and a[0].family.id == QCQP and a[0].family.batched_params:
+        raise _lib.LFPSQPError("optimize solves one instance: give every qcqp array at its own shape (no batch axis), "
+                               "or call optimize_batched")
     a[idx] = np.asarray(a[idx], dtype=np.float64)[None, :]
     if param is not None:
         a.append(param)

@@ -150,8 +150,62 @@ bool fam_valid(int family, int64_t n, int64_t m, int64_t p) {
     case LFPSQP_FAM_DIAGQUAD: return FamDiagQuad::valid(n, m, p);
     case LFPSQP_FAM_SIN: return FamSin::valid(n, m, p);
     case LFPSQP_FAM_BOXQUAD: return FamBoxQuad::valid(n, m, p);
+    case LFPSQP_FAM_QCQP: return FamQCQP::valid(n, m, p);
     default: return false;
   }
+}
+
+// lfpsqp_qcqp viewed as its nine {pointer, batch stride} pairs, in declaration order
+struct QcqpField { const double *ptr; int64_t stride; };
+static_assert(sizeof(lfpsqp_qcqp) == 9 * sizeof(QcqpField), "lfpsqp_qcqp is nine {pointer, stride} pairs");
+const char *const kQcqpNames[9] = {"P", "q", "r", "Qc", "Ac", "bc", "Qd", "Ad", "bd"};
+
+// element count of each array and how many n x n matrices it stacks
+void qcqp_counts(int64_t n, int64_t m, int64_t p, int64_t cnt[9], int64_t nmat[9]) {
+  const int64_t c[9] = {n * n, n, 1, m * n * n, m * n, m, p * n * n, p * n, p}, k[9] = {1, 0, 0, m, 0, 0, p, 0, 0};
+  for (int i = 0; i < 9; i++) { cnt[i] = c[i]; nmat[i] = k[i]; }
+}
+
+// Argument checks of the QCQP descriptor shared by both entry points.  out = the descriptor with the arrays of
+// zero elements (Qc when m = 0, ...) set to NULL, so that nothing downstream reads them.
+int qcqp_check(lfpsqp_ctx *c, const double *fam_params, int64_t fam_stride, int64_t n, int64_t m, int64_t p,
+               lfpsqp_qcqp &out) {
+  if (!fam_params) return c->fail(LFPSQP_ERR_ARG, "LFPSQP_FAM_QCQP: fam_params must point to a lfpsqp_qcqp descriptor");
+  if (fam_stride != 0) return c->fail(LFPSQP_ERR_ARG, "LFPSQP_FAM_QCQP: fam_stride must be 0 (each array has its own stride)");
+  out = *(const lfpsqp_qcqp *)fam_params;
+  QcqpField *F = (QcqpField *)&out;
+  int64_t cnt[9], nmat[9];
+  qcqp_counts(n, m, p, cnt, nmat);
+  for (int i = 0; i < 9; i++) {
+    if (cnt[i] == 0) { F[i].ptr = nullptr; F[i].stride = 0; continue; }
+    if (F[i].ptr && (F[i].stride < 0 || (F[i].stride != 0 && F[i].stride < cnt[i])))
+      return c->fail(LFPSQP_ERR_ARG, "LFPSQP_FAM_QCQP: %s_stride = %lld; it must be 0 (shared) or >= %lld", kQcqpNames[i],
+                     (long long)F[i].stride, (long long)cnt[i]);
+  }
+  if (m > 0 && !out.Qc && !out.Ac) return c->fail(LFPSQP_ERR_ARG, "LFPSQP_FAM_QCQP: m > 0 needs Qc or Ac");
+  if (p > 0 && !out.Qd && !out.Ad) return c->fail(LFPSQP_ERR_ARG, "LFPSQP_FAM_QCQP: p > 0 needs Qd or Ad");
+  return LFPSQP_OK;
+}
+
+// exact symmetry of every n x n matrix the host entry point stages (instances [0, B) of a per-instance array)
+int qcqp_check_symmetric(lfpsqp_ctx *c, const lfpsqp_qcqp &qp, int64_t n, int64_t m, int64_t p, int64_t B) {
+  const QcqpField *F = (const QcqpField *)&qp;
+  int64_t cnt[9], nmat[9];
+  qcqp_counts(n, m, p, cnt, nmat);
+  for (int i = 0; i < 9; i++) {
+    if (!F[i].ptr || nmat[i] == 0) continue;
+    const int64_t copies = F[i].stride ? B : 1;
+    for (int64_t k = 0; k < copies; k++)
+      for (int64_t t = 0; t < nmat[i]; t++) {
+        const double *M = F[i].ptr + k * F[i].stride + t * n * n;
+        for (int64_t a = 1; a < n; a++)
+          for (int64_t b = 0; b < a; b++)
+            if (!(M[a * n + b] == M[b * n + a]))
+              return c->fail(LFPSQP_ERR_ARG, "LFPSQP_FAM_QCQP: %s is not symmetric (instance %lld, matrix %lld, entry %lld,%lld)",
+                             kQcqpNames[i], (long long)k, (long long)t, (long long)a, (long long)b);
+      }
+  }
+  return LFPSQP_OK;
 }
 
 // InequalityData (src/inequality_helper.jl:39-85) for the slack-augmented bound vectors (optimize.jl:30-36).
@@ -258,6 +312,7 @@ int dispatch_batched(lfpsqp_ctx *c, BatchedArgs &A) {
     case LFPSQP_FAM_DIAGQUAD: return launch_warp<FamDiagQuad>(c, A, use_nr);
     case LFPSQP_FAM_SIN: return launch_warp<FamSin>(c, A, use_nr);
     case LFPSQP_FAM_BOXQUAD: return launch_warp<FamBoxQuad>(c, A, use_nr);
+    case LFPSQP_FAM_QCQP: return launch_warp<FamQCQP>(c, A, use_nr);   // not separable: no register-resident solver
     default: return c->fail(LFPSQP_ERR_FAMILY, "unknown family %d", A.family);
   }
 }
@@ -320,6 +375,11 @@ extern "C" int lfpsqp_solve_batched_dev(lfpsqp_ctx *c, int family, int64_t n, in
   int rc = prepare_batched(c, family, n, m, p, B, xl, xu, prm, H, A);
   if (rc) return rc;
   c->last_ms = 0; c->last_launches = 0;
+  if (family == LFPSQP_FAM_QCQP) {   // descriptor in host memory, arrays in device memory (symmetry is a precondition)
+    rc = qcqp_check(c, fam_params_dev, fam_stride, n, m, p, A.qcqp);
+    if (rc) return rc;
+    fam_params_dev = nullptr;
+  }
   if (B == 0) return LFPSQP_OK;
   if (fam_param_count(family, n, m, p) > 0 && !fam_params_dev) return c->fail(LFPSQP_ERR_ARG, "family needs a parameter blob");
   A.fam_params = fam_params_dev; A.fam_stride = fam_stride; A.x0 = x0_dev;
@@ -353,7 +413,27 @@ extern "C" int lfpsqp_solve_batched(lfpsqp_ctx *c, int family, int64_t n, int64_
   BatchedArgs A0;
   int rc = prepare_batched(c, family, n, m, p, B, xl, xu, prm, H, A0);
   if (rc) return rc;
+  // QCQP: host arrays of the descriptor; qf = the device copies (arena slots 10..18, same batch strides as the caller's)
+  lfpsqp_qcqp qh{}, qd{};
+  QcqpField *qf = (QcqpField *)&qd;
+  const QcqpField *hf = (const QcqpField *)&qh;
+  int64_t qcnt[9] = {0}, qmat[9];
+  if (family == LFPSQP_FAM_QCQP) {
+    rc = qcqp_check(c, fam_params, fam_stride, n, m, p, qh);
+    if (rc) return rc;
+    rc = qcqp_check_symmetric(c, qh, n, m, p, B);
+    if (rc) return rc;
+    fam_params = nullptr;
+    qcqp_counts(n, m, p, qcnt, qmat);
+  }
   if (B == 0) return LFPSQP_OK;
+  for (int i = 0; i < 9; i++) {
+    if (!hf[i].ptr) continue;
+    const int64_t elems = hf[i].stride ? (B - 1) * hf[i].stride + qcnt[i] : qcnt[i];   // never reads past the last instance
+    qf[i].ptr = (const double *)c->arena(10 + i, (size_t)elems * 8);
+    qf[i].stride = hf[i].stride;
+    if (!qf[i].ptr) return c->fail(LFPSQP_ERR_NOMEM, "device allocation failed");
+  }
   const int64_t npar = fam_param_count(family, n, m, p);
   if (npar > 0 && !fam_params) return c->fail(LFPSQP_ERR_ARG, "family needs a parameter blob");
   if (npar > 0 && fam_stride != 0 && fam_stride < npar) return c->fail(LFPSQP_ERR_ARG, "fam_stride smaller than the family's blob");
@@ -419,6 +499,12 @@ extern "C" int lfpsqp_solve_batched(lfpsqp_ctx *c, int family, int64_t n, int64_
   unsigned long long *counter0 = c->work_counter;
   if (nchunk > 1) cudaStreamSynchronize(user_stream);   // earlier work on the caller's stream is done before the pipeline starts
   if (npar && fam_stride == 0) cudaMemcpyAsync(d_par, fam_params, par_bytes, cudaMemcpyHostToDevice, user_stream), cudaStreamSynchronize(user_stream);
+  {  // QCQP arrays shared by the batch: copied once, before any chunk's kernel
+    bool any = false;
+    for (int i = 0; i < 9; i++)
+      if (hf[i].ptr && !hf[i].stride) { cudaMemcpyAsync((void *)qf[i].ptr, hf[i].ptr, (size_t)qcnt[i] * 8, cudaMemcpyHostToDevice, user_stream); any = true; }
+    if (any) cudaStreamSynchronize(user_stream);
+  }
   c->last_launches = 0;
   int64_t launches = 0;
   for (int ci = 0; ci < nchunk && rc == 0; ci++) {
@@ -429,6 +515,14 @@ extern "C" int lfpsqp_solve_batched(lfpsqp_ctx *c, int family, int64_t n, int64_
     cudaMemsetAsync(d_obj + lo * H, 0xff, (size_t)H * nb * 8, s);  // NaN-fill the unused tail of the history
     BatchedArgs A = A0;
     A.B = nb;
+    QcqpField *af = (QcqpField *)&A.qcqp;
+    for (int i = 0; i < 9; i++) {
+      af[i] = qf[i];
+      if (!hf[i].ptr || !hf[i].stride) continue;
+      const int64_t off = lo * hf[i].stride;   // per-instance array: this chunk's instances, rebased to the chunk
+      cudaMemcpyAsync((void *)(qf[i].ptr + off), hf[i].ptr + off, (size_t)((nb - 1) * hf[i].stride + qcnt[i]) * 8, cudaMemcpyHostToDevice, s);
+      af[i].ptr = qf[i].ptr + off;
+    }
     if (noise_row) {
       cudaMemcpyAsync(d_noise + lo * noise_row, c->noise_host + lo * noise_row, noise_row * nb * 8, cudaMemcpyHostToDevice, s);
       A.noise = d_noise + lo * noise_row; A.noise_T = c->noise_T;

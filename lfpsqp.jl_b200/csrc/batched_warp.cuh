@@ -713,6 +713,7 @@ struct Solver {
   // ------------------------------------------------------------ the driver (optimize.jl:176-443)
   LFPSQP_DEV void run(const BatchedArgs &A, int64_t k) {
     fc.prm = A.fam_params ? A.fam_params + k * A.fam_stride : nullptr;
+    if constexpr (Fam::kId == LFPSQP_FAM_QCQP) { fc.k = k; fc.qp = A.qcqp; }
     st = lfpsqp_stats{}; status = 0;
     for (int i = g.lane; i < L.total; i += G::SIZE) sm[i] = 0.0;
     g.sync();

@@ -43,6 +43,8 @@ struct WarpGroup {
 struct FamCtx {
   int n, m, p;            // user sizes: variables, equalities c, inequalities d
   const double *prm;      // this instance's parameter blob (global memory)
+  int64_t k;              // this instance's index in the launch (FamQCQP: array base + k * stride)
+  lfpsqp_qcqp qp;         // FamQCQP: device pointers + batch strides (the other families ignore it)
 };
 
 struct BatchedArgs {
@@ -59,6 +61,7 @@ struct BatchedArgs {
   // stochastic perturbation of optimize.jl:264-273 with a caller-supplied noise sequence (lfpsqp_ctx_set_noise): instance k,
   // outer iteration i < noise_T uses the N working entries at noise + (k * noise_T + i) * N ; nullptr when beta == 0
   const double *noise; int64_t noise_T;
+  lfpsqp_qcqp qcqp;       // LFPSQP_FAM_QCQP: device pointers rebased to this launch's first instance, batch strides
 };
 
 // coefficient of the noise term at outer iteration i (optimize.jl:267-271); 0 beyond the supplied rows

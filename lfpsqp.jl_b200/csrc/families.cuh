@@ -302,4 +302,103 @@ struct FamBoxQuad {
   }
 };
 
+// ---------------------------------------------------------------- dense QCQP given by data (lfpsqp_qcqp)
+// f = 1/2 x'Px + q.x + r ; c_i = 1/2 x'Qc_i x + Ac_i.x - bc_i ; d_k = 1/2 x'Qd_k x + Ad_k.x - bd_k.
+// The matrices are symmetric, so (M v)_j = sum_i M_ij v_i reads row i coalesced across the lanes (lane = column j),
+// through L2 with __ldg.  A NULL array is skipped, not read as zeros; the test is group-uniform (the descriptor is a
+// kernel parameter).  A quadratic's value is sum_j (0.5 (Mx)_j + a_j) x_j: with M = 2I and a = NULL every term is
+// x_j x_j exactly, which is what makes the README families' encodings give their registered results bit for bit.
+struct FamQCQP {
+  static constexpr int kId = LFPSQP_FAM_QCQP;
+  static constexpr bool kSparseJac = false;
+  static __host__ bool valid(int64_t n, int64_t m, int64_t p) { return n >= 1 && m >= 0 && p >= 0; }
+  // this instance's copy of one array (NULL stays NULL)
+  static LFPSQP_DEV const double *arr(const FamCtx &fc, const double *base, int64_t stride) {
+    return base ? base + fc.k * stride : nullptr;
+  }
+  // (M v)_j of a symmetric n x n matrix
+  static LFPSQP_DEV double mv(const double *M, const double *v, int n, int j) {
+    double s = 0;
+#pragma unroll 4
+    for (int i = 0; i < n; i++) s += __ldg(M + (size_t)i * n + j) * v[i];
+    return s;
+  }
+  // 1/2 x'Mx + a.x - b (M, a, b may be NULL, not both M and a); with row != NULL also writes the gradient Mx + a
+  template <class G>
+  static LFPSQP_DEV double quad(const G &g, int n, const double *M, const double *a, const double *b, double *row,
+                                const double *x) {
+    double s = 0;
+    for (int j = g.lane; j < n; j += G::SIZE) {
+      double gj, w;
+      if (M) {
+        const double u = mv(M, x, n, j);
+        gj = u; w = 0.5 * u;
+        if (a) { const double aj = __ldg(a + j); gj += aj; w += aj; }
+      } else {
+        gj = w = __ldg(a + j);
+      }
+      if (row) row[j] = gj;
+      s += w * x[j];
+    }
+    s = g.sum(s);
+    return b ? s - __ldg(b) : s;
+  }
+  template <class G> static LFPSQP_DEV double f(const G &g, const FamCtx &fc, const double *x) {
+    const double *P = arr(fc, fc.qp.P, fc.qp.P_stride), *q = arr(fc, fc.qp.q, fc.qp.q_stride);
+    const double *r = arr(fc, fc.qp.r, fc.qp.r_stride);
+    const double v = (P || q) ? quad(g, fc.n, P, q, nullptr, nullptr, x) : 0.0;
+    return r ? v + __ldg(r) : v;
+  }
+  template <class G> static LFPSQP_DEV void grad(const G &g, const FamCtx &fc, double *out, const double *x) {
+    const double *P = arr(fc, fc.qp.P, fc.qp.P_stride), *q = arr(fc, fc.qp.q, fc.qp.q_stride);
+    for (int j = g.lane; j < fc.n; j += G::SIZE) {
+      double gj = 0.0;
+      if (P) { gj = mv(P, x, fc.n, j); if (q) gj += __ldg(q + j); }
+      else if (q) gj = __ldg(q + j);
+      out[j] = gj;
+    }
+  }
+  // rows of one constraint block (cnt quadratics): values into cv, gradients into J (row stride ld) when J != NULL
+  template <class G>
+  static LFPSQP_DEV void block(const G &g, const FamCtx &fc, int cnt, const double *Q, int64_t Qs, const double *A,
+                               int64_t As, const double *b, int64_t bs, double *J, int ld, double *cv, const double *x) {
+    const int n = fc.n;
+    Q = arr(fc, Q, Qs); A = arr(fc, A, As); b = arr(fc, b, bs);
+    for (int i = 0; i < cnt; i++) {
+      const double v = quad(g, n, Q ? Q + (size_t)i * n * n : nullptr, A ? A + (size_t)i * n : nullptr,
+                            b ? b + i : nullptr, J ? J + (size_t)i * ld : nullptr, x);
+      if (g.lane == 0) cv[i] = v;
+    }
+  }
+  template <class G> static LFPSQP_DEV void c(const G &g, const FamCtx &fc, double *cv, const double *x) {
+    block(g, fc, fc.m, fc.qp.Qc, fc.qp.Qc_stride, fc.qp.Ac, fc.qp.Ac_stride, fc.qp.bc, fc.qp.bc_stride, nullptr, 0, cv, x);
+  }
+  template <class G>
+  static LFPSQP_DEV void jac(const G &g, const FamCtx &fc, double *J, int ld, double *cv, const double *x) {
+    block(g, fc, fc.m, fc.qp.Qc, fc.qp.Qc_stride, fc.qp.Ac, fc.qp.Ac_stride, fc.qp.bc, fc.qp.bc_stride, J, ld, cv, x);
+  }
+  template <class G> static LFPSQP_DEV void d(const G &g, const FamCtx &fc, double *dv, const double *x) {
+    block(g, fc, fc.p, fc.qp.Qd, fc.qp.Qd_stride, fc.qp.Ad, fc.qp.Ad_stride, fc.qp.bd, fc.qp.bd_stride, nullptr, 0, dv, x);
+  }
+  template <class G>
+  static LFPSQP_DEV void jacd(const G &g, const FamCtx &fc, double *J, int ld, double *dv, const double *x) {
+    block(g, fc, fc.p, fc.qp.Qd, fc.qp.Qd_stride, fc.qp.Ad, fc.qp.Ad_stride, fc.qp.bd, fc.qp.bd_stride, J, ld, dv, x);
+  }
+  // dest = (P + sum_i lam_i Qc_i + sum_k lam_d_k Qd_k) v, one pass over every matrix's rows
+  template <class G>
+  static LFPSQP_DEV void hess(const G &g, const FamCtx &fc, double *dest, const double *v, const double *,
+                              const double *lam, const double *lam_d) {
+    const int n = fc.n;
+    const size_t nn = (size_t)n * n;
+    const double *P = arr(fc, fc.qp.P, fc.qp.P_stride), *Qc = arr(fc, fc.qp.Qc, fc.qp.Qc_stride);
+    const double *Qd = arr(fc, fc.qp.Qd, fc.qp.Qd_stride);
+    for (int j = g.lane; j < n; j += G::SIZE) {
+      double s = P ? mv(P, v, n, j) : 0.0;
+      if (Qc) for (int i = 0; i < fc.m; i++) s += lam[i] * mv(Qc + i * nn, v, n, j);
+      if (Qd) for (int k = 0; k < fc.p; k++) s += lam_d[k] * mv(Qd + k * nn, v, n, j);
+      dest[j] = s;
+    }
+  }
+};
+
 }  // namespace lfpsqp

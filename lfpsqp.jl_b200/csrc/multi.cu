@@ -45,7 +45,17 @@ int solve_batched_multi(lfpsqp_ctx *c, int family, int64_t n, int64_t m, int64_t
     if (nb == 0) { rcs[g] = 0; ch->last_ms = 0; ch->last_launches = 0; return; }
     if (c->noise_host) { ch->noise_host = c->noise_host + lo * c->noise_T * c->noise_N; ch->noise_T = c->noise_T; ch->noise_N = c->noise_N; ch->noise_B = nb; }
     else { ch->noise_host = nullptr; ch->noise_T = ch->noise_N = ch->noise_B = 0; }
-    rcs[g] = lfpsqp_solve_batched(ch, family, n, m, p, nb, fam_params ? fam_params + (fam_stride ? lo * fam_stride : 0) : nullptr, fam_stride,
+    const double *shard_params = fam_params ? fam_params + (fam_stride ? lo * fam_stride : 0) : nullptr;
+    lfpsqp_qcqp qs;
+    if (family == LFPSQP_FAM_QCQP && fam_params) {   // the descriptor is shared; each per-instance array moves to the shard's first instance
+      qs = *(const lfpsqp_qcqp *)fam_params;
+      struct Field { const double *ptr; int64_t stride; };
+      static_assert(sizeof(lfpsqp_qcqp) == 9 * sizeof(Field), "lfpsqp_qcqp is nine {pointer, stride} pairs");
+      Field *F = (Field *)&qs;
+      for (int i = 0; i < 9; i++) if (F[i].ptr && F[i].stride > 0) F[i].ptr += lo * F[i].stride;
+      shard_params = (const double *)&qs;
+    }
+    rcs[g] = lfpsqp_solve_batched(ch, family, n, m, p, nb, shard_params, fam_stride,
                                   x0 ? x0 + lo * n : nullptr, xl, xu, prm, x_out ? x_out + lo * n : nullptr, obj_hist ? obj_hist + lo * H : nullptr, H,
                                   obj_len ? obj_len + lo : nullptr, lambda ? lambda + lo * ME : nullptr, term ? term + lo : nullptr,
                                   stats ? stats + lo : nullptr);

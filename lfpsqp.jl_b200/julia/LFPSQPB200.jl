@@ -8,7 +8,7 @@ import Random
 
 export optimize, optimize_batched, optimize_large, LFPSQPParams, TerminationInfo, DeviceFamily, DeviceCallback, callbacks, use_devices!,
        rosenbrock, readme_equality,
-       readme_inequality, thomson, diagquad
+       readme_inequality, thomson, diagquad, qcqp, QCQPFamily
 
 const lib = joinpath(@__DIR__, "..", "liblfpsqp_b200.so")
 
@@ -65,6 +65,55 @@ function optimize_batched(fam::DeviceFamily, X0::Matrix{Float64}, xl, xu, param:
                      Ptr{Float64}, Ref{LFPSQPParams}, Ptr{Float64}, Ptr{Float64}, Int64, Ptr{Int64}, Ptr{Float64},
                      Ptr{CTerm}, Ptr{Cvoid}),
                     context(), fam.id, n, fam.m, fam.p, B, fam.params, fam.stride, X0, pl, pu, param, x, obj, history,
+                    len, λ, term, C_NULL))
+    end
+    x, obj, len, λ, term
+end
+
+# dense QCQP given by data (LFPSQP_FAM_QCQP = 101): lfpsqp_qcqp is nine {pointer, batch stride} pairs
+struct CQcqp
+    P::Ptr{Float64}; P_stride::Int64; q::Ptr{Float64}; q_stride::Int64; r::Ptr{Float64}; r_stride::Int64
+    Qc::Ptr{Float64}; Qc_stride::Int64; Ac::Ptr{Float64}; Ac_stride::Int64; bc::Ptr{Float64}; bc_stride::Int64
+    Qd::Ptr{Float64}; Qd_stride::Int64; Ad::Ptr{Float64}; Ad_stride::Int64; bd::Ptr{Float64}; bd_stride::Int64
+end
+struct QCQPFamily
+    n::Int64; m::Int64; p::Int64; arrays::Vector{Any}; strides::Vector{Int64}   # P q r Qc Ac bc Qd Ad bd (nothing = zero)
+end
+const _QCQP_NDIMS = (2, 1, 0, 3, 2, 1, 3, 2, 1)   # own dims: P n x n, q n, r scalar, Qc n x n x m, Ac n x m (column i = a_i), bc m, ...
+"""qcqp(; P, q, r, Qc, Ac, bc, Qd, Ad, bd): each array at its own shape (shared by the batch) or with a trailing batch
+dimension B (per instance); nothing = zero.  Matrices are symmetrised as (M + M')/2."""
+function qcqp(; P=nothing, q=nothing, r=nothing, Qc=nothing, Ac=nothing, bc=nothing, Qd=nothing, Ad=nothing, bd=nothing)
+    arrays = Any[P, q, r, Qc, Ac, bc, Qd, Ad, bd]; strides = zeros(Int64, 9)
+    for i in 1:9
+        a = arrays[i]
+        isnothing(a) && continue
+        a = Array{Float64}(a isa Number ? fill(Float64(a)) : a)
+        if i in (1, 4, 7)   # symmetrise every n x n slice
+            a = (a .+ permutedims(a, (2, 1, (3:ndims(a))...))) ./ 2
+        end
+        ndims(a) == _QCQP_NDIMS[i] + 1 && (strides[i] = prod(size(a)[1:end-1]))
+        ndims(a) in (_QCQP_NDIMS[i], _QCQP_NDIMS[i] + 1) || error("qcqp: array $i has $(ndims(a)) dimensions")
+        arrays[i] = a
+    end
+    n = something(map(a -> isnothing(a) ? nothing : size(a, 1), arrays[[1, 2, 4, 5, 7, 8]])..., 0)
+    m = isnothing(bc) ? (isnothing(Ac) ? (isnothing(Qc) ? 0 : size(arrays[4], 3)) : size(arrays[5], 2)) : size(arrays[6], 1)
+    p = isnothing(bd) ? (isnothing(Ad) ? (isnothing(Qd) ? 0 : size(arrays[7], 3)) : size(arrays[8], 2)) : size(arrays[9], 1)
+    QCQPFamily(n, m, p, arrays, strides)
+end
+
+function optimize_batched(fam::QCQPFamily, X0::Matrix{Float64}, xl, xu, param::LFPSQPParams=LFPSQPParams(); history::Int=64)
+    n, B = size(X0); me = fam.m + fam.p
+    x = Matrix{Float64}(undef, n, B); obj = Matrix{Float64}(undef, history, B); len = Vector{Int64}(undef, B)
+    λ = Matrix{Float64}(undef, me, B); term = Vector{CTerm}(undef, B)
+    pl = isnothing(xl) ? Ptr{Float64}(C_NULL) : pointer(xl); pu = isnothing(xu) ? Ptr{Float64}(C_NULL) : pointer(xu)
+    GC.@preserve X0 xl xu x obj len λ term fam begin
+        ptrs = [isnothing(a) ? Ptr{Float64}(C_NULL) : pointer(a) for a in fam.arrays]
+        desc = Ref(CQcqp(collect(Iterators.flatten(zip(ptrs, fam.strides)))...))
+        check(ccall((:lfpsqp_solve_batched, lib), Cint,
+                    (Ptr{Cvoid}, Cint, Int64, Int64, Int64, Int64, Ref{CQcqp}, Int64, Ptr{Float64}, Ptr{Float64},
+                     Ptr{Float64}, Ref{LFPSQPParams}, Ptr{Float64}, Ptr{Float64}, Int64, Ptr{Int64}, Ptr{Float64},
+                     Ptr{CTerm}, Ptr{Cvoid}),
+                    context(), 101, n, fam.m, fam.p, B, desc, 0, X0, pl, pu, param, x, obj, history,
                     len, λ, term, C_NULL))
     end
     x, obj, len, λ, term
