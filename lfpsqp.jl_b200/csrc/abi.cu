@@ -10,6 +10,7 @@
 #include "ctx.h"
 #include "batched_tiny.cuh"
 #include "batched_warp.cuh"
+#include "launch.cuh"
 
 using namespace lfpsqp;
 
@@ -261,39 +262,15 @@ int launch_warp(lfpsqp_ctx *c, BatchedArgs &A, int use_nr) {
   }
   if (resident < 1) return c->fail(LFPSQP_ERR_CUDA, "batched_warp_kernel cannot be made resident");
   const size_t smem = bnd_bytes + warps * per_warp;
-  c->round_instances = (int64_t)c->sm_count * resident * warps;
-  if (c->query_round) return LFPSQP_OK;
-  int64_t grid = (int64_t)c->sm_count * resident;
-  int64_t need = (A.B + warps - 1) / warps;
-  if (grid > need) grid = need;
-  if (grid < 1) grid = 1;
-  cudaMemsetAsync(c->work_counter, 0, 8, c->stream);
-  A.work_counter = c->work_counter;
-  cudaEventRecord(c->ev0, c->stream);
-  kern<<<(unsigned)grid, warps * 32, smem, c->stream>>>(A, use_nr);
-  cudaEventRecord(c->ev1, c->stream);
-  c->last_launches = 1;
-  c->last_cfg_warps = warps; c->last_cfg_grid = (int)grid; c->last_cfg_smem = (int)smem; c->last_cfg_resident = resident;
-  c->last_kernel[0] = 1; c->last_kernel[1] = 32; c->last_kernel[2] = 0; c->last_kernel[3] = 0;
-  e = cudaGetLastError();
-  if (e != cudaSuccess) return c->cuda_fail(e, "batched_warp_kernel launch");
-  return LFPSQP_OK;
+  const int64_t grid = persistent_grid(c, A, resident, warps);
+  return launch_batched_kernel(c, kern, grid, warps * 32, smem, {1, 32, 0, 0}, "batched_warp_kernel launch", A, use_nr);
 }
 
 template <class Fam, int NT>
-int launch_tiny(lfpsqp_ctx *c, BatchedArgs &A) {
+int launch_tiny(lfpsqp_ctx *c, BatchedArgs &A) {   // one thread per instance, not persistent
   const int threads = 128;
-  int64_t grid = (A.B + threads - 1) / threads;
-  c->round_instances = 0;   // one thread per instance, not persistent: no round structure
-  if (c->query_round) return LFPSQP_OK;
-  cudaEventRecord(c->ev0, c->stream);
-  batched_tiny_kernel<Fam, NT><<<(unsigned)grid, threads, 0, c->stream>>>(A);
-  cudaEventRecord(c->ev1, c->stream);
-  c->last_launches = 1;
-  c->last_kernel[0] = 0; c->last_kernel[1] = 1; c->last_kernel[2] = 0; c->last_kernel[3] = 0;
-  cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) return c->cuda_fail(e, "batched_tiny_kernel launch");
-  return LFPSQP_OK;
+  return launch_batched_kernel(c, batched_tiny_kernel<Fam, NT>, (A.B + threads - 1) / threads, threads, 0, {0, 1, 0, 0},
+                               "batched_tiny_kernel launch", A);
 }
 
 int dispatch_batched(lfpsqp_ctx *c, BatchedArgs &A) {
@@ -449,52 +426,22 @@ extern "C" int lfpsqp_solve_batched(lfpsqp_ctx *c, int family, int64_t n, int64_
   double *d_noise = noise_row ? (double *)c->arena(9, noise_row * B * 8) : nullptr;
   if (!d_par || !d_x0 || !d_x || !d_obj || !d_lam || !d_len || !d_term || (stats && !d_stats) || (noise_row && !d_noise))
     return c->fail(LFPSQP_ERR_NOMEM, "device allocation failed");
-  // chunking: keep every chunk big enough to fill the GPU several times over
+  // chunking: keep every chunk big enough to fill the GPU several times over.  The first chunk's H2D and the last chunk's
+  // D2H are the only copies the kernels cannot hide, so those two chunks are half the size of the others (measured at C2,
+  // 65,536 instances: 8 equal chunks 2.050 ms, halved ends 2.009 ms, 16 chunks 2.06-2.09 ms, 4 chunks 2.24 ms;
+  // device-resident kernel 1.74 ms).  Chunks cut in whole rounds of the persistent kernels (resident CTAs x instances per
+  // CTA) measured slower (2.11 ms): a partly filled last round costs nothing, because the idle CTAs exit and the next
+  // chunk's CTAs take their place, while whole rounds end all CTAs at once and expose the launch gap.
   int nchunk = 1;
   if (B >= 16384) nchunk = (int)std::min<int64_t>(8, B / 8192);
-  // pipeline shape: the first chunk's H2D and the last chunk's D2H are the only copies the kernels cannot hide, so those two
-  // chunks are half the size of the others (measured at C2, 65,536 instances: 8 equal chunks 2.050 ms, halved ends 2.009 ms,
-  // 16 chunks 2.06-2.09 ms, 4 chunks 2.24 ms; device-resident kernel 1.74 ms).  LFPSQP_PIPE_CHUNKS / LFPSQP_PIPE_RAMP override
-  // (tools/e2e_pipe.py).  LFPSQP_PIPE_ROUNDS=1 cuts the chunks in whole rounds of the persistent kernels (resident CTAs x
-  // instances per CTA) instead: measured SLOWER (2.11 ms) -- a partly filled last round costs nothing, because the idle CTAs
-  // exit and the next chunk's CTAs take their place, while whole rounds end all CTAs at once and expose the launch gap.
-  double ramp = 0.5;
-  bool shaped = true;
-  if (const char *e = getenv("LFPSQP_PIPE_ROUNDS")) shaped = !(e[0] == '1');
-  if (const char *e = getenv("LFPSQP_PIPE_CHUNKS")) { int v = atoi(e); if (v >= 1 && v <= 64 && B >= 2 * v) { nchunk = v; shaped = true; } }
-  if (const char *e = getenv("LFPSQP_PIPE_RAMP")) { double v = atof(e); if (v > 0.05 && v <= 1.0) ramp = v; }
-  std::vector<int64_t> cut(nchunk + 1, 0);
-  int64_t q = 0;
-  if (nchunk > 1 && !shaped) {
-    BatchedArgs Aq = A0; Aq.B = B;
-    c->query_round = 1; c->round_instances = 0;
-    const int qrc = dispatch_batched(c, Aq);
-    c->query_round = 0;
-    if (qrc == LFPSQP_OK) q = c->round_instances;
-  }
-  if (q > 0 && B >= 4 * q) {
-    const int64_t R = B / q, rem = B - R * q;
-    int64_t mid = 2 * q;
-    while ((R - 1 + mid / q - 1) / (mid / q) > 12) mid += 2 * q;   // at most 12 middle chunks
-    std::vector<int64_t> c2; c2.push_back(0); c2.push_back(q);
-    int64_t left = (R - 1) * q;
-    while (left > 0) { const int64_t t = std::min(mid, left); c2.push_back(c2.back() + t); left -= t; }
-    if (rem > 0) c2.push_back(B);
-    cut = c2; nchunk = (int)cut.size() - 1;
-  } else {
-    const double tot = (nchunk > 2) ? (nchunk - 2) + 2 * ramp : (double)nchunk;
-    double acc = 0;
-    for (int ci = 0; ci < nchunk; ci++) {
-      acc += (nchunk > 2 && (ci == 0 || ci == nchunk - 1)) ? ramp : 1.0;
-      cut[ci + 1] = std::min<int64_t>(B, (int64_t)(B * (acc / tot) + 0.5));
-    }
-    cut[nchunk] = B;
-    for (int ci = 0; ci < nchunk; ci++) if (cut[ci + 1] <= cut[ci]) { nchunk = 1; cut.assign(2, 0); cut[1] = B; break; }
-  }
   const int NS = 3;
   if (nchunk > 1 && !c->pipe[0]) {
     for (int i = 0; i < NS; i++) if (cudaStreamCreateWithFlags(&c->pipe[i], cudaStreamNonBlocking) != cudaSuccess) { cudaGetLastError(); nchunk = 1; break; }
   }
+  // chunk ci = instances [cut[ci], cut[ci + 1]); chunk sizes in the ratio 1/2 : 1 : ... : 1 : 1/2 (two halves when nchunk = 2)
+  std::vector<int64_t> cut(nchunk + 1, B);
+  cut[0] = 0;
+  for (int ci = 1; ci < nchunk; ci++) cut[ci] = (int64_t)(B * ((ci - 0.5) / (nchunk - 1)) + 0.5);
   cudaStream_t user_stream = c->stream;
   unsigned long long *counter0 = c->work_counter;
   if (nchunk > 1) cudaStreamSynchronize(user_stream);   // earlier work on the caller's stream is done before the pipeline starts

@@ -26,20 +26,10 @@
 #pragma once
 #include "common.cuh"
 
-// A/B switches of the register kernel; defaults = measured best on B200 (C2, LW = 8: 1.687 ms for 65,536 instances;
-// MASKS=1: 1.82, FIXUP=1: 1.76, both: 1.83, DXS=1: 2.04, EPCACHE=0: 1.72; gpurun_out/r2f_ab.log)
-#ifndef LFPSQP_F_MASKS
-#define LFPSQP_F_MASKS 0     // 1: per-thread bit masks for "slot holds a user variable / a slack" instead of index compares (measured slower)
-#endif
-#ifndef LFPSQP_F_FIXUP
-#define LFPSQP_F_FIXUP 0     // 1: line formula for every slot + one fix-up branch per lane, instead of one branch per slot (measured slower)
-#endif
-#ifndef LFPSQP_F_DXS
-#define LFPSQP_F_DXS 0       // wide lanes: accumulate pcg!'s dx in the stash instead of registers
-#endif
-#ifndef LFPSQP_F_EPCACHE
-#define LFPSQP_F_EPCACHE 1   // keep per-element family parameters in registers (0: re-read through the L1 on demand)
-#endif
+// Alternatives measured against this kernel on a B200 (C2, LW = 8: 1.687 ms for 65,536 instances) and dropped: bit masks
+// for "slot holds a user variable / a slack" instead of index compares 1.82 ms; the line formula for every slot plus one
+// fix-up branch per lane 1.76 ms; pcg!'s dx accumulated in the stash 2.04 ms; family parameters re-read through the L1
+// instead of cached in registers 1.72 ms (profiles/r2_c2_ab_feature_switches.log).
 
 namespace lfpsqp {
 
@@ -47,7 +37,6 @@ namespace lfpsqp {
 // row a < m is an equality c_a, row a >= m an inequality d_{a-m}; ep = this element's cached parameters (KP doubles)
 struct SepReadmeIneq {  // f = coeff.x ; d = x.x - 1     (README.md:57-76)
   static constexpr int kId = LFPSQP_FAM_README_INEQ, KP = 1;
-  static constexpr bool kCache = LFPSQP_F_EPCACHE != 0;   // 0: re-read the one read-only parameter per element through the L1 instead of pinning NPL registers
   static LFPSQP_DEV void load(const FamCtx &fc, int j, double *ep) { ep[0] = __ldg(fc.prm + j); }
   static LFPSQP_DEV double f(const FamCtx &, int, double x, const double *ep) { return ep[0] * x; }
   static LFPSQP_DEV double g(const FamCtx &, int, double, const double *ep) { return ep[0]; }
@@ -58,7 +47,6 @@ struct SepReadmeIneq {  // f = coeff.x ; d = x.x - 1     (README.md:57-76)
 };
 struct SepReadmeEq {  // f = x.x ; c = x[1] - 0.75          (README.md:41-54)
   static constexpr int kId = LFPSQP_FAM_README_EQ, KP = 0;
-  static constexpr bool kCache = true;
   static LFPSQP_DEV void load(const FamCtx &, int, double *) {}
   static LFPSQP_DEV double f(const FamCtx &, int, double x, const double *) { return x * x; }
   static LFPSQP_DEV double g(const FamCtx &, int, double x, const double *) { return 2.0 * x; }
@@ -69,7 +57,6 @@ struct SepReadmeEq {  // f = x.x ; c = x[1] - 0.75          (README.md:41-54)
 };
 struct SepBoxQuad {  // f = |x-t|^2 ; optional c = a.x - b ; params [t(n), a(n), b]
   static constexpr int kId = LFPSQP_FAM_BOXQUAD, KP = 2;
-  static constexpr bool kCache = true;
   static LFPSQP_DEV void load(const FamCtx &fc, int j, double *ep) { ep[0] = __ldg(fc.prm + j); ep[1] = __ldg(fc.prm + fc.n + j); }
   static LFPSQP_DEV double f(const FamCtx &, int, double x, const double *ep) { double u = x - ep[0]; return u * u; }
   static LFPSQP_DEV double g(const FamCtx &, int, double x, const double *ep) { return 2.0 * (x - ep[0]); }
@@ -125,9 +112,8 @@ struct RegSolver {
   static constexpr int MEA = ME > 0 ? ME : 1;
   static constexpr int NAP = NPL * LW;                       // padded vector length (bound tables are zero-padded to it)
   static constexpr int VECD = (INEQ ? 2 : 1) * NAP;          // doubles of one stashed vector
-  static constexpr bool DXS = (LFPSQP_F_DXS != 0) && NPL >= 6;                      // wide lanes: pcg!'s solution dx accumulates in the stash, not in registers
   static constexpr int NGR = SPARSE ? 1 : NPL;
-  enum { SV_X = 0, SV_D, SV_XTIL, SV_XNEW, SV_GV, SV_DX, SV_COUNT };
+  enum { SV_X = 0, SV_D, SV_XTIL, SV_XNEW, SV_GV, SV_COUNT };
   static constexpr int STASH_DOUBLES = SV_COUNT * VECD;      // per group
   struct Vec { double x[NPL]; double y[INEQ ? NPL : 1]; };
 
@@ -140,11 +126,9 @@ struct RegSolver {
   // (kind: 0 line, 1 parabola, 2 circle); padded elements have q = s = r = t = 0 and x = y = 0 throughout
   const double *bnd;
   unsigned kinds;        // 2 bits per slot: this lane's bound kinds (bkind without the shared-memory read)
-  unsigned umask;        // bit k: slot k holds a user variable (idx(k) < n); fixed for the whole batch
-  unsigned sbits;        // bit 8a + k: slot k of this lane holds the slack of constraint row a (a >= m)
   double pcg_rho_stop;   // largest rho with sqrt(rho) <= eps_c: pcg!'s test norm(r) > tol (retractions.jl:207) without the sqrt
   double *stash;         // this group's parking area
-  double ep[Fam::kCache ? NPL : 1][KP];    // cached per-element family parameters (kCache families)
+  double ep[NPL][KP];    // cached per-element family parameters
   // instance state
   Vec x;
   double J[MEA][NPL], Lc[MEA][MEA], cval[MEA], lam[MEA];
@@ -160,12 +144,8 @@ struct RegSolver {
   LFPSQP_DEV RegSolver(int lane_, unsigned gmask_, const lfpsqp_params &prm_, int n_, int m_, int p_, const double *bnd_, double *stash_)
       : lane(lane_), gmask(gmask_), prm(prm_), n(n_), m(m_), p(p_), NA(n_ + p_), bnd(bnd_), stash(stash_) {
     fc.n = n_; fc.m = m_; fc.p = p_; fc.prm = nullptr;
-    kinds = 0; umask = 0;
-    LF_UNROLL for (int k = 0; k < NPL; k++) if (k * LW + lane < n_) umask |= 1u << k;
+    kinds = 0;
     exc = -1;
-    sbits = 0;
-    LF_UNROLL for (int a = 0; a < ME; a++)
-      LF_UNROLL for (int k = 0; k < NPL; k++) if (a >= m_ && k * LW + lane == n_ + (a - m_)) sbits |= 1u << (8 * a + k);
     if (INEQ) { LF_UNROLL for (int k = 0; k < NPL; k++) { const unsigned kd = (unsigned)(int)bnd[k * LW + lane] & 3u; kinds |= kd << (2 * k); if (kd != 0u) exc = k; } }
     // sqrt is correctly rounded and monotone: {rho : sqrt(rho) <= eps_c} is an interval [0, t]; find t once
     const double e = prm.eps_c;
@@ -180,22 +160,14 @@ struct RegSolver {
   }
 
   LFPSQP_DEV int idx(int s) const { return s * LW + lane; }
-#if LFPSQP_F_MASKS
-  LFPSQP_DEV bool user(int k) const { return (umask >> k) & 1u; }
-  LFPSQP_DEV bool slack(int a, int k) const { return (sbits >> (8 * a + k)) & 1u; }
-#else
   LFPSQP_DEV bool user(int k) const { return idx(k) < n; }
   LFPSQP_DEV bool slack(int a, int k) const { return a >= m && idx(k) == n + (a - m); }
-#endif
   LFPSQP_DEV double gS(int k) const { if (!SPARSE) return S[SPARSE ? 0 : k]; return (k == exc) ? S[0] : sqrt(2.0); }
   LFPSQP_DEV double gDx(int k) const { if (!SPARSE) return Dx[SPARSE ? 0 : k]; return (k == exc) ? Dx[0] : 1.0 * (1.0 / sqrt(2.0)); }
   LFPSQP_DEV double gDy(int k) const { if (!SPARSE) return Dy[SPARSE ? 0 : k]; return (k == exc) ? Dy[0] : -1.0 * (1.0 / sqrt(2.0)); }
   LFPSQP_DEV void eload(int k, double *e) const {   // family parameters of user slot k
-    if (Fam::kCache) { LF_UNROLL for (int q = 0; q < KP; q++) e[q] = ep[Fam::kCache ? k : 0][q]; }
-    else Fam::load(fc, idx(k), e);
+    LF_UNROLL for (int q = 0; q < KP; q++) e[q] = ep[k][q];
   }
-  LFPSQP_DEV double &dxx(Vec &dx, int k) const { return DXS ? sx(SV_DX, k) : dx.x[k]; }
-  LFPSQP_DEV double &dxy(Vec &dx, int k) const { return DXS ? sy(SV_DX, k) : dx.y[k]; }
   LFPSQP_DEV int bkind(int k) const { return INEQ ? (int)((kinds >> (2 * k)) & 3u) : 0; }
   LFPSQP_DEV double bq(int k) const { return INEQ ? bnd[NAP + idx(k)] : 0.0; }
   LFPSQP_DEV double br(int k) const { return INEQ ? bnd[2 * NAP + idx(k)] : 0.0; }
@@ -326,7 +298,6 @@ struct RegSolver {
       v.y[k] = (idx(k) < NA) ? yv : 0.0;
     }
   }
-#if !LFPSQP_F_FIXUP
   LFPSQP_DEV void calculate_h(double *out, const Vec &v) const {  // :112-122
     LF_UNROLL for (int k = 0; k < NPL; k++) {
       // line pairs (and the padded elements) have q = s = r = t = 0: the general formula reduces EXACTLY to x - y there
@@ -348,36 +319,6 @@ struct RegSolver {
       S[SPARSE ? 0 : k] = sv; Dx[SPARSE ? 0 : k] = dx * inv; Dy[SPARSE ? 0 : k] = dy * inv;
     }
   }
-#else
-  LFPSQP_DEV void calculate_h(double *out, const Vec &v) const {  // :112-122
-    // line pairs (and the padded elements) have q = s = r = t = 0: the general formula reduces EXACTLY to x - y there
-    // (0 (dx dx) + 1 x + 0 (dy dy) - 1 y - 0).  Lanes that hold a parabola / circle pair redo those slots.
-    LF_UNROLL for (int k = 0; k < NPL; k++) out[k] = v.x[k] - v.y[k];
-    if (kinds != 0u) {
-      LF_UNROLL for (int k = 0; k < NPL; k++) {
-        if (bkind(k) == 0) continue;
-        double q = bq(k), s = bs(k), r = br(k), dx = v.x[k] - r, dy = v.y[k] - r;
-        out[k] = q * (dx * dx) + (1.0 - q * q) * v.x[k] + s * (dy * dy) - (1.0 - s * s) * v.y[k] - bt(k);
-      }
-    }
-  }
-  // line pairs (q = s = 0): dx = 1, dy = -1 whatever (x, y) is, so S = sqrt(2), Dx = 1/S, Dy = -1/S -- the values the
-  // general formula computes -- never change: set once per instance (init_line_gradients), refreshed nowhere
-  LFPSQP_DEV void init_line_gradients() {
-    LF_UNROLL for (int k = 0; k < NGR; k++) { const double sv = sqrt(2.0), inv = 1.0 / sv; S[k] = sv; Dx[k] = 1.0 * inv; Dy[k] = -1.0 * inv; }
-  }
-  LFPSQP_DEV void inequality_gradient(const Vec &v) {  // :125-141 (parabola / circle pairs; see init_line_gradients)
-    if (kinds == 0u) return;
-    LF_UNROLL for (int k = 0; k < NPL; k++) {
-      if (bkind(k) == 0) continue;
-      double q = bq(k), s = bs(k), r = br(k);
-      double dx = 2.0 * q * (v.x[k] - r) + (q == 0.0 ? 1.0 : 0.0);
-      double dy = 2.0 * s * (v.y[k] - r) - (s == 0.0 ? 1.0 : 0.0);
-      double sv = sqrt(dx * dx + dy * dy), inv = 1.0 / sv;   // one reciprocal instead of two divisions (<= 1 ulp apart)
-      S[SPARSE ? 0 : k] = sv; Dx[SPARSE ? 0 : k] = dx * inv; Dy[SPARSE ? 0 : k] = dy * inv;
-    }
-  }
-#endif
   LFPSQP_DEV void y_retract_elem(int k, double &xn, double &yn, double xb, double yb) const {  // retractions.jl:451-500
     if (idx(k) >= NA) return;
     const int kind = bkind(k);
@@ -599,7 +540,7 @@ struct RegSolver {
       {
         Vec r, pv;
         r = gv; zero(pv);
-        LF_UNROLL for (int k = 0; k < NPL; k++) { dxx(dx, k) = 0.0; if (INEQ) dxy(dx, k) = 0.0; }
+        LF_UNROLL for (int k = 0; k < NPL; k++) { dx.x[k] = 0.0; if (INEQ) dx.y[k] = 0.0; }
         bool go = true;                                              // norm_res = Inf before the first iteration (:205)
         double rho_prev = 1.0, rho, Jr[MEA], Jp[MEA];
         {
@@ -633,10 +574,10 @@ struct RegSolver {
           const double alpha = rho / sum(pz);
           double a0 = 0.0, b0 = 0.0, b1 = 0.0;
           LF_UNROLL for (int k = 0; k < NPL; k++) {
-            dxx(dx, k) += alpha * pv.x[k]; r.x[k] -= alpha * z.x[k]; a0 += r.x[k] * r.x[k];
+            dx.x[k] += alpha * pv.x[k]; r.x[k] -= alpha * z.x[k]; a0 += r.x[k] * r.x[k];
             if (ME > 0) b0 += J[0][k] * r.x[k];
             if (ME > 1) b1 += J[MEA - 1][k] * r.x[k];
-            if (INEQ) { dxy(dx, k) += alpha * pv.y[k]; r.y[k] -= alpha * z.y[k]; a0 += r.y[k] * r.y[k]; }
+            if (INEQ) { dx.y[k] += alpha * pv.y[k]; r.y[k] -= alpha * z.y[k]; a0 += r.y[k] * r.y[k]; }
           }
           if (ME == 2) { sum3(a0, b0, b1); Jr[0] = b0; Jr[MEA - 1] = b1; } else if (ME == 1) { sum2(a0, b0); Jr[0] = b0; } else a0 = sum(a0);
           rho_prev = rho; rho = a0;
@@ -648,11 +589,11 @@ struct RegSolver {
       if (pi == prm.maxiter_pcg) { get(SV_XNEW, xnew); flag = 2; break; }   // :240-243, :377-381
       // inner Armijo (:384-426): p = xnew (stays in the stash) ; xnew -= dx ; g = xnew - xtilde
       double ard = 0.0, s2 = 0.0;
-      LF_UNROLL for (int k = 0; k < NPL; k++) ard += sx(SV_GV, k) * dxx(dx, k);
-      if (INEQ) { LF_UNROLL for (int k = 0; k < NPL; k++) ard += sy(SV_GV, k) * dxy(dx, k); }
+      LF_UNROLL for (int k = 0; k < NPL; k++) ard += sx(SV_GV, k) * dx.x[k];
+      if (INEQ) { LF_UNROLL for (int k = 0; k < NPL; k++) ard += sy(SV_GV, k) * dx.y[k]; }
       LF_UNROLL for (int k = 0; k < NPL; k++) {
-        xnew.x[k] = sx(SV_XNEW, k) - 1.0 * dxx(dx, k); { const double t = xnew.x[k] - sx(SV_XTIL, k); s2 += t * t; }
-        if (INEQ) { xnew.y[k] = sy(SV_XNEW, k) - 1.0 * dxy(dx, k); const double t = xnew.y[k] - sy(SV_XTIL, k); s2 += t * t; }
+        xnew.x[k] = sx(SV_XNEW, k) - 1.0 * dx.x[k]; { const double t = xnew.x[k] - sx(SV_XTIL, k); s2 += t * t; }
+        if (INEQ) { xnew.y[k] = sy(SV_XNEW, k) - 1.0 * dx.y[k]; const double t = xnew.y[k] - sy(SV_XTIL, k); s2 += t * t; }
       }
       double alpha = 1.0;
       c_partial(cpart, xnew);                                           // :392
@@ -678,8 +619,8 @@ struct RegSolver {
         if (!((h2 + c2) + mu * dist2 > prev_obj + 1e-4 * alpha * ar_dot)) break;   // :403
         alpha /= 2; s2 = 0.0;
         LF_UNROLL for (int k = 0; k < NPL; k++) {
-          xnew.x[k] = sx(SV_XNEW, k) - alpha * dxx(dx, k); { const double t = xnew.x[k] - sx(SV_XTIL, k); s2 += t * t; }
-          if (INEQ) { xnew.y[k] = sy(SV_XNEW, k) - alpha * dxy(dx, k); const double t = xnew.y[k] - sy(SV_XTIL, k); s2 += t * t; }
+          xnew.x[k] = sx(SV_XNEW, k) - alpha * dx.x[k]; { const double t = xnew.x[k] - sx(SV_XTIL, k); s2 += t * t; }
+          if (INEQ) { xnew.y[k] = sy(SV_XNEW, k) - alpha * dx.y[k]; const double t = xnew.y[k] - sy(SV_XTIL, k); s2 += t * t; }
         }
         h2 = 0.0;
         if (INEQ) { calculate_h(cvh, xnew); LF_UNROLL for (int k = 0; k < NPL; k++) h2 += cvh[k] * cvh[k]; sum2(s2, h2); }   // :410-417: only the bound part is refreshed, the c-part stays frozen
@@ -746,10 +687,8 @@ struct RegSolver {
     rank = ME; pinv = false;
     LF_UNROLL for (int s = 0; s < NPL; s++) {
       int j = idx(s);
-      if (Fam::kCache) {
-        LF_UNROLL for (int q = 0; q < KP; q++) ep[Fam::kCache ? s : 0][q] = 0.0;
-        if (j < n) Fam::load(fc, j, ep[Fam::kCache ? s : 0]);
-      }
+      LF_UNROLL for (int q = 0; q < KP; q++) ep[s][q] = 0.0;
+      if (j < n) Fam::load(fc, j, ep[s]);
       x.x[s] = (j < n) ? A.x0[k * n + j] : 0.0;
       if (INEQ) x.y[s] = 0.0;
       cvh[s] = 0.0; lamy[s] = 0.0;
@@ -881,12 +820,13 @@ struct RegSolver {
   }
 };
 
-// Persistent CTAs of 128 threads = 128 / LW lane groups; every group pulls instance indices from a global counter until the
-// batch is drained (absorbs the per-instance iteration-count variance).  The groups of a warp leave the loop together.
-// MINB = resident CTAs per SM the register allocation is capped for (3 -> 168 registers, 2 -> 255).
-// SPARSE: see RegSolver; NT = threads per CTA.
-template <class Fam, int LW, int NPL, int ME, bool INEQ, bool SPARSE, int NT, int MINB>
-__global__ void __launch_bounds__(NT, MINB) batched_reg_kernel(const BatchedArgs A) {
+// Persistent CTAs of REG_NT threads = REG_NT / LW lane groups; every group pulls instance indices from a global counter
+// until the batch is drained (absorbs the per-instance iteration-count variance).  The groups of a warp leave the loop
+// together.  MINB = resident CTAs per SM the register allocation is capped for (3 -> 168 registers, 2 -> 255).
+// SPARSE: see RegSolver.
+constexpr int REG_NT = 128;
+template <class Fam, int LW, int NPL, int ME, bool INEQ, bool SPARSE, int MINB>
+__global__ void __launch_bounds__(REG_NT, MINB) batched_reg_kernel(const BatchedArgs A) {
   using RS = RegSolver<Fam, LW, NPL, ME, INEQ, SPARSE>;
   extern __shared__ double smem[];
   const int lane32 = threadIdx.x & 31;

@@ -27,12 +27,7 @@ struct lfpsqp_ctx {
   unsigned long long *work_counter = nullptr;
   double last_ms = 0.0;
   int64_t last_launches = 0;
-  int last_cfg_warps = 0, last_cfg_grid = 0, last_cfg_smem = 0, last_cfg_resident = 0;
   int last_kernel[4] = {-1, 0, 0, 0};   // lfpsqp_last_kernel: {kind, LW, NPL, SPARSE} of the last batched launch
-  // persistent batched kernels work in ROUNDS of round_instances = resident CTAs x instances per CTA; query_round = 1 makes
-  // the launchers fill it in and return without launching (the host pipeline sizes its chunks in whole rounds)
-  int query_round = 0;
-  int64_t round_instances = 0;
   std::string err;
   std::vector<void *> bufs;  // grow-only device arena, one slot per role (no allocation inside solve loops)
   std::vector<size_t> caps;

@@ -417,7 +417,7 @@ def test_instances_do_not_depend_on_the_batch(L, which):
 
 # ----------------------------------------------------------------------- host pipeline vs device-resident entry point
 @pytest.mark.parametrize("B", [16383, 16384, 16385, 65536 + 7])
-def test_host_pipeline_matches_device_entry(L, monkeypatch, B):
+def test_host_pipeline_matches_device_entry(L, B):
     import torch
     import bench
     from lfpsqp.jl_b200 import _lib
@@ -454,11 +454,6 @@ def test_host_pipeline_matches_device_entry(L, monkeypatch, B):
     assert np.all(np.isnan(ref[1][np.arange(H)[None, :] >= olen[:, None]]))   # the NaN tail past obj_len
     assert _identical(device_entry(False)[:5], ref[:5]) == -1
     runs = {"host": host_entry(True), "host stats=NULL": host_entry(False)}
-    monkeypatch.setenv("LFPSQP_PIPE_ROUNDS", "1")
-    try:
-        runs["host PIPE_ROUNDS=1"] = host_entry(True)
-    finally:
-        monkeypatch.delenv("LFPSQP_PIPE_ROUNDS")
     for label, out in runs.items():
         assert _kernel(L) == REG(8, 7, 1)
         bad = _identical(tuple(out[:5]) + ((out[5],) if len(out) > 5 else (None,)), ref)

@@ -1,6 +1,6 @@
 #!/bin/bash
-# Round-2 evidence on ONE B200 (run under gpurun): sanitizer passes on the new paths, ncu --set full of the final C2 register
-# kernel and of the fused pcg! kernel (reports are reduced to CSV here: the .ncu-rep files are too large to bring back), and
+# Round-2 evidence on ONE B200: sanitizer passes on the new paths, ncu --set full of the fused pcg! and
+# projcg kernels (reports are reduced to CSV here: the .ncu-rep files are too large to bring back), and
 # the launch list of the bench command.
 set -x
 OUT=gpurun_out
@@ -8,10 +8,6 @@ for tool in memcheck racecheck synccheck; do
   compute-sanitizer --tool $tool python tools/sanitize_small.py r2 > $OUT/r2_sanitizer_$tool.log 2>&1
   tail -3 $OUT/r2_sanitizer_$tool.log
 done
-ncu --set full --clock-control none --import-source on -k regex:batched_reg -s 3 -c 1 -o /tmp/r2_c2 python tools/c2_variants.py 0 > $OUT/r2_ncu_c2.log 2>&1
-ncu -i /tmp/r2_c2.ncu-rep --page details --csv > $OUT/r2_c2_batched_reg_details.csv 2>/dev/null
-ncu -i /tmp/r2_c2.ncu-rep --page raw --csv > $OUT/r2_c2_batched_reg_raw.csv 2>/dev/null
-ncu -i /tmp/r2_c2.ncu-rep --page source --csv > $OUT/r2_c2_batched_reg_source.csv 2>/dev/null
 ncu --set full --clock-control none -k regex:fused_pcg -s 1 -c 1 -o /tmp/r2_pcg python tools/c5_quick.py > $OUT/r2_ncu_pcg.log 2>&1
 ncu -i /tmp/r2_pcg.ncu-rep --page details --csv > $OUT/r2_fused_pcg_details.csv 2>/dev/null
 ncu -i /tmp/r2_pcg.ncu-rep --page raw --csv > $OUT/r2_fused_pcg_raw.csv 2>/dev/null
