@@ -252,6 +252,18 @@ int lfpsqp_large_pcg(lfpsqp_ctx *ctx, const double *x_point_loc, double mu, cons
 /* host wall-clock split (ms) of the last lfpsqp_large_solve: [factorisation (jac!, Gram, Cholesky, first projection),
  * projcg!, line search incl. retractions, total] */
 int lfpsqp_large_phase_ms(lfpsqp_ctx *ctx, double *out4);
+/* what the last large-n call (factor, project, projcg, projcg_general, retract, pcg, solve) enqueued, recorded on the host
+ * (read-only; no kernel changes).  out8 =
+ *   [0] mask of dgemm_nt instantiations: 1 <128> lean, 2 <128> with extras (block-structure flags, batches), 4 <64> (N <= 64),
+ *       8 <128, SKIP> (zero-slab skipping); bits 0-3 for the Gram's SYRK, bits 4-7 for every other product
+ *   [1] largest split-K factor of a product with fewer than SMs / 2 tiles (0: none)
+ *   [2] largest wave-quantisation split-K factor of a lower SYRK (0: none)
+ *   [3] mask of rows_dot kernels: bits 0-2 R = 1, 2, 4 rows per CTA; bits 3-5 the same with zero-slab skipping
+ *   [4] launches of the single-GPU explicit-inverse fused projcg kernel, [5] of the general fused projcg kernel,
+ *   [6] launches of the fused pcg! kernel
+ *   [7] mask of the forms the Gram solves took: 1 explicit inverse, 2 triangular solves, 4 truncated pseudo-inverse
+ * LFPSQP_ERR_ARG before lfpsqp_large_setup. */
+int lfpsqp_large_last_dispatch(lfpsqp_ctx *ctx, int64_t *out8);
 
 /* Unit-level bound embedding (src/inequality_helper.jl; y_retract! src/retractions.jl:451-500) on one instance; runs the
  * device code of the batched solver.  J: m x n row-major (== Jct column-major), may be NULL when m = 0.

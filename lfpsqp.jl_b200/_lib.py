@@ -32,6 +32,7 @@ TERM_DTYPE = np.dtype([("condition", "<i4"), ("status", "<i4"), ("f_diff", "<f8"
 STATS_FIELDS = ("projcg_iters", "projcg_negcurv", "armijo_trials", "retract_outer", "retract_pcg", "pp_backtracks",
                 "newton_accepted", "factorizations", "f_evals", "flag_last")
 STATS_DTYPE = np.dtype([(k, "<i8") for k in STATS_FIELDS])
+LARGE_DISPATCH_FIELDS = ("gemm", "ksplit_grid", "ksplit_wave", "rows_dot", "fused_single", "fused_general", "fused_pcg", "solve")
 
 EXPORTS = [
     "lfpsqp_version", "lfpsqp_default_params", "lfpsqp_ctx_create", "lfpsqp_ctx_destroy", "lfpsqp_last_error",
@@ -42,6 +43,7 @@ EXPORTS = [
     "lfpsqp_ineq_op", "lfpsqp_large_phase_ms", "lfpsqp_comm_ipc_export", "lfpsqp_comm_ipc_import", "lfpsqp_comm_mode",
     "lfpsqp_large_set_bounds", "lfpsqp_solve_host", "lfpsqp_linesearch", "lfpsqp_aug_hess_vec", "lfpsqp_large_projcg_general",
     "lfpsqp_ctx_create_multi", "lfpsqp_ctx_device_count", "lfpsqp_ctx_set_noise", "lfpsqp_last_kernel",
+    "lfpsqp_large_last_dispatch",
 ]
 
 _lib = None
@@ -88,6 +90,7 @@ def load():
         lib.lfpsqp_large_pcg.argtypes = [P, P, C.c_double, P, C.c_double, I, P, P, P, P]
         lib.lfpsqp_ineq_op.argtypes = [P, C.c_int, I, I, P, P, P, P, I, P, I]
         lib.lfpsqp_large_phase_ms.argtypes = [P, P]
+        lib.lfpsqp_large_last_dispatch.argtypes = [P, C.POINTER(C.c_int64)]
         lib.lfpsqp_comm_ipc_export.argtypes = [P, P]
         lib.lfpsqp_comm_ipc_import.argtypes = [P, P]
         lib.lfpsqp_comm_mode.argtypes = [P]
@@ -155,6 +158,17 @@ class Context:
         out = (C.c_int * 4)()
         self.check(self.lib.lfpsqp_last_kernel(self.h, out))
         return tuple(out)
+
+    @property
+    def large_dispatch(self):
+        """What the last large-n call enqueued (lfpsqp_large_last_dispatch): gemm = mask of dgemm_nt instantiations (1 <128>
+        lean, 2 <128> with extras, 4 <64>, 8 <128, SKIP>; bits 0-3 the Gram's SYRK, 4-7 other products), ksplit_grid /
+        ksplit_wave = largest split-K factors (0 none), rows_dot = mask (bits 0-2 R = 1, 2, 4; bits 3-5 with zero-slab
+        skipping), fused_single / fused_general / fused_pcg = fused kernel launches, solve = mask (1 explicit inverse,
+        2 triangular, 4 pseudo-inverse)"""
+        out = (C.c_int64 * 8)()
+        self.check(self.lib.lfpsqp_large_last_dispatch(self.h, out))
+        return dict(zip(LARGE_DISPATCH_FIELDS, (int(v) for v in out)))
 
 
 class MultiContext(Context):

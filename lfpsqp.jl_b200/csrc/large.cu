@@ -55,7 +55,8 @@ static int read_ctrl(lfpsqp_ctx *c, LargeState &S) {
   if (S.gdep_pending) { S.gdep_pending = false; S.g_blockdiag = (S.hctrl->g_dependent == 0) ? 1 : 0; }
   if (S.nz_pending) {       // density of the zero-slab map of J -> keep skipping (block-sparse J) or use the plain SYRK from now on
     S.nz_pending = false;
-    const double total = (double)S.nz_rows * (double)std::max<int64_t>(S.nz_ld, 1);
+    // out of the (64-row slab, K chunk) pairs the scan visits; nz_ld is padded past the last chunk and does not count
+    const double total = (double)S.nz_rows * (double)std::max<int64_t>((S.n_loc + GM_BK - 1) / GM_BK, 1);
     S.gram_mode = ((double)S.hctrl->nz_count > 0.5 * total) ? 2 : 1;
   }
   if (S.guard_pending) {    // pivots of the factor just computed -> which solve the fused projcg kernel may use
@@ -72,6 +73,10 @@ static void write_ctrl_fields(LargeState &S) {  // push the host copy (tolerance
   cudaMemcpyAsync(S.ctrl, S.hctrl, sizeof(LargeCtrl), cudaMemcpyHostToDevice, S.stream);
 }
 
+// lfpsqp_large_last_dispatch bits of a dgemm_nt instantiation: 1 <128> lean, 2 <128> with the extras' prologue, 4 <64>,
+// 8 <128, SKIP>; bits 0-3 for the Gram's SYRK, bits 4-7 for every other product
+static void note_gemm(LargeState &S, int bit) { S.disp[LARGE_DISP_GEMM] |= (int64_t)bit << (S.disp_syrk ? 0 : 4); }
+
 // C (op)= A B' with optional split-K through S.gemm_ws
 static void gemm_nt(LargeState &S, int M, int N, int K, const double *A, int64_t lda, const double *B, int64_t ldb, double *C,
                     int64_t ldc, int mode, int lower, const GemmExt *ext = nullptr) {
@@ -87,6 +92,7 @@ static void gemm_nt(LargeState &S, int M, int N, int K, const double *A, int64_t
     grid.z = X.batch;
     if (narrow) dgemm_nt_kernel<64><<<grid, 256, dgemm_smem_bytes<64>(), S.stream>>>(M, N, K, A, lda, B, ldb, C, ldc, mode, lower, 1, 0, X);
     else dgemm_nt_kernel<128><<<grid, 256, dgemm_smem_bytes<128>(), S.stream>>>(M, N, K, A, lda, B, ldb, C, ldc, mode, lower, 1, 0, X);
+    note_gemm(S, narrow ? 4 : 2);
     S.launches++;
     return;
   }
@@ -94,6 +100,7 @@ static void gemm_nt(LargeState &S, int M, int N, int K, const double *A, int64_t
     ksplit = std::min(std::min(16, S.sm_count / tiles), K / 256);
     while (ksplit > 1 && (size_t)ksplit * M * (N + 1) * 8 > S.gemm_ws_bytes) ksplit--;
     if (ksplit < 1) ksplit = 1;
+    if (ksplit > 1) S.disp[LARGE_DISP_KSPLIT_GRID] = std::max<int64_t>(S.disp[LARGE_DISP_KSPLIT_GRID], ksplit);
   } else if (mode == GEMM_ASSIGN && lower && K >= 8192 && tiles < S.sm_count) {
     // wave quantisation of a SYRK that does not fill one wave (C5: 136 lower tiles on 148 SMs = 92 %): split K so that
     // tiles x ksplit fills whole waves (C5: 13 -> 1768 CTAs = 11.95 waves; measured 27.2 -> 28.9 TFLOP/s).  With several
@@ -105,12 +112,14 @@ static void gemm_nt(LargeState &S, int M, int N, int K, const double *A, int64_t
       if (eff(ks) > eff(best) + 0.02) best = ks;
     }
     ksplit = best;
+    if (ksplit > 1) S.disp[LARGE_DISP_KSPLIT_WAVE] = std::max<int64_t>(S.disp[LARGE_DISP_KSPLIT_WAVE], ksplit);
   }
   // zero-slab skipping (SYRK of a block-sparse J): the chunk list of one K slice must fit behind the tiles in shared memory
   const int kchunks = (K + GM_BK - 1) / GM_BK, per = (kchunks + ksplit - 1) / ksplit;
   const size_t skip_smem = dgemm_smem_bytes<128>() + (size_t)per * sizeof(int);
   const bool skip = X.nz && !narrow && skip_smem <= (size_t)S.max_dyn_smem;
   const bool lean = !ext;   // plain product: the instantiation without the extras' prologue
+  note_gemm(S, skip ? 8 : narrow ? 4 : lean ? 1 : 2);
   if (ksplit == 1) {
     if (skip) dgemm_nt_kernel<128, true><<<grid, 256, skip_smem, S.stream>>>(M, N, K, A, lda, B, ldb, C, ldc, mode, lower, 1, 0, X);
     else if (narrow) dgemm_nt_kernel<64><<<grid, 256, dgemm_smem_bytes<64>(), S.stream>>>(M, N, K, A, lda, B, ldb, C, ldc, mode, lower, 1, 0, X);
@@ -146,12 +155,14 @@ static void rows_dot(LargeState &S, const double *Jm, int64_t ld, int m, int64_t
     if (m >= 8 * S.sm_count) rows_dot_kernel<4, true><<<(m + 3) / 4, 256, 0, S.stream>>>(Jm, ld, m, ncols, v, t, S.ctrl, pred, S.nzmap, S.nz_ld);
     else if (m >= 2 * S.sm_count) rows_dot_kernel<2, true><<<(m + 1) / 2, 256, 0, S.stream>>>(Jm, ld, m, ncols, v, t, S.ctrl, pred, S.nzmap, S.nz_ld);
     else rows_dot_kernel<1, true><<<m, 256, 0, S.stream>>>(Jm, ld, m, ncols, v, t, S.ctrl, pred, S.nzmap, S.nz_ld);
+    S.disp[LARGE_DISP_ROWS_DOT] |= (m >= 8 * S.sm_count ? 4 : m >= 2 * S.sm_count ? 2 : 1) << 3;
     S.launches++;
     return;
   }
   if (m >= 8 * S.sm_count) rows_dot_kernel<4><<<(m + 3) / 4, 256, 0, S.stream>>>(Jm, ld, m, ncols, v, t, S.ctrl, pred);
   else if (m >= 2 * S.sm_count) rows_dot_kernel<2><<<(m + 1) / 2, 256, 0, S.stream>>>(Jm, ld, m, ncols, v, t, S.ctrl, pred);
   else rows_dot_kernel<1><<<m, 256, 0, S.stream>>>(Jm, ld, m, ncols, v, t, S.ctrl, pred);
+  S.disp[LARGE_DISP_ROWS_DOT] |= m >= 8 * S.sm_count ? 4 : m >= 2 * S.sm_count ? 2 : 1;   // bits 0-2: R = 1, 2, 4 ; 3-5: SKIP
   S.launches++;
 }
 static void cols_dot(LargeState &S, const double *Jm, int64_t ld, int m, int64_t ncols, const double *u, int pred) {
@@ -168,12 +179,14 @@ static void gram_solve(LargeState &S, const double *t, double *u, double *u_copy
   const int m = S.m;
   if (S.pinv_active) {   // rank-deficient: u = G^+ t (one dense m x m pass; optimize.jl:297-302 equivalent, large_eig.cu)
     rows_dot(S, S.Ginv, S.ldm, m, m, t, u, pred);
+    S.disp[LARGE_DISP_SOLVE] |= LARGE_SOLVE_PINV;
     if (u_copy) vec(S, m, [=] __device__(int64_t a, double *) { u_copy[a] = u[a]; });
     S.launches++;
     return;
   }
   tri_gemv_kernel<<<(m + 7) / 8, 256, m * sizeof(double), S.stream>>>(S.Linv, S.ldm, m, t, S.ty, 0, nullptr, S.ctrl, pred, S.invflag_valid ? S.invflag : nullptr, S.nz_rows);
   tri_gemv_kernel<<<(m + 7) / 8, 256, m * sizeof(double), S.stream>>>(S.XT, S.ldm, m, S.ty, u, 1, u_copy, S.ctrl, pred, S.invflag_valid ? S.invflag : nullptr, S.nz_rows);
+  S.disp[LARGE_DISP_SOLVE] |= LARGE_SOLVE_TRIANGULAR;
   S.launches += 2;
 }
 
@@ -367,7 +380,9 @@ static void gram_syrk(LargeState &S, const double *Jg) {
     if (S.gram_mode == 0) S.nz_pending = true;
     S.jmap_valid = (Jg == S.J);   // with bounds the map describes J diag(Dy), whose zeros are not J's
   } else S.jmap_valid = false;
+  S.disp_syrk = true;
   gemm_nt(S, m, m, (int)S.n_loc, Jg, S.ldj, Jg, S.ldj, S.G, S.ldm, GEMM_ASSIGN, 1, ext);
+  S.disp_syrk = false;
 }
 static void gram_only(LargeState &S) {   // S.G (lower tiles) = J W J', all-reduced
   const int m = S.m;
@@ -1259,6 +1274,7 @@ static int need_large(lfpsqp_ctx *c) {
   if (!c->large) return c->fail(LFPSQP_ERR_ARG, "call lfpsqp_large_setup first");
   cudaSetDevice(c->device);
   c->large->stream = c->stream;
+  std::fill(c->large->disp, c->large->disp + 8, (int64_t)0);   // every entry call starts a new dispatch record
   return 0;
 }
 static int prep_params(lfpsqp_ctx *c, LargeState &S, const lfpsqp_params *prm) {
@@ -1379,7 +1395,9 @@ extern "C" int lfpsqp_large_factor(lfpsqp_ctx *c, const double *x_loc, double *G
   memset(S.hctrl, 0, sizeof(LargeCtrl)); write_ctrl_fields(S);
   fam_c_jac(S, S.J, S.cval, S.x);
   if (G_out) {  // G before it is overwritten by L
+    S.disp_syrk = true;
     gemm_nt(S, m, m, (int)S.n_loc, S.J, S.ldj, S.J, S.ldj, S.G, ldm, GEMM_ASSIGN, 1);
+    S.disp_syrk = false;
     if (S.world > 1) comm_allreduce(S, S.G, (size_t)m * ldm);
     CK(cudaMemcpy2DAsync(G_out, m * 8, S.G, ldm * 8, m * 8, m, cudaMemcpyDeviceToHost, S.stream));
   }
@@ -1533,6 +1551,13 @@ extern "C" int lfpsqp_large_pcg(lfpsqp_ctx *c, const double *x_point_loc, double
   if (flag) *flag = (S.hctrl->pcg_iter == maxiter) ? 1 : 0;
   { float ms = 0; cudaEventElapsedTime(&ms, c->ev0, c->ev1); c->last_ms = ms; }   // device time of the pcg! loop (lfpsqp_last_kernel_ms)
   c->last_launches = S.launches;
+  return LFPSQP_OK;
+}
+
+// what the last large-n entry call enqueued (LargeState::disp, large_state.h): read-only, recorded on the host
+extern "C" int lfpsqp_large_last_dispatch(lfpsqp_ctx *c, int64_t *out8) {
+  if (!c || !c->large || !out8) return LFPSQP_ERR_ARG;
+  std::copy(c->large->disp, c->large->disp + 8, out8);
   return LFPSQP_OK;
 }
 

@@ -656,6 +656,7 @@ int fused_projcg_chunk(LargeState &S, int iters, int first, double *xs, double *
                                               dim3(FT), args, smem, S.stream);
   if (e != cudaSuccess) { cudaGetLastError(); S.fused_ok = false; return 1; }
   S.launches++;
+  S.disp[LARGE_DISP_FUSED_GENERAL]++; S.disp[LARGE_DISP_SOLVE] |= a.solve_mode == 0 ? large_ginv_form(S) : (int64_t)LARGE_SOLVE_TRIANGULAR;
   if (want_prof) {
     double h[8];
     cudaMemcpyAsync(h, a.prof, sizeof(h), cudaMemcpyDeviceToHost, S.stream);
@@ -693,6 +694,7 @@ int fused_pcg(LargeState &S, double *dx, double *r, double *pv, double *z) {
   cudaError_t e = cudaLaunchCooperativeKernel(kern, dim3(S.fused_grid), dim3(FT), args, smem, S.stream);
   if (e != cudaSuccess) { cudaGetLastError(); return 1; }
   S.launches++;
+  S.disp[LARGE_DISP_FUSED_PCG]++;
   return 0;
 }
 

@@ -419,6 +419,7 @@ int fused_projcg_chunk_single(LargeState &S, int iters, int first, double *xs, d
   cudaError_t e = cudaLaunchCooperativeKernel((void *)fused_projcg_kernel, dim3(S.fused_grid), dim3(FT), args, smem, S.stream);
   if (e != cudaSuccess) { cudaGetLastError(); S.fused_ok = false; return 1; }
   S.launches++;
+  S.disp[LARGE_DISP_FUSED_SINGLE]++; S.disp[LARGE_DISP_SOLVE] |= large_ginv_form(S);
   if (want_prof) {
     double h[8];
     cudaMemcpyAsync(h, a.prof, sizeof(h), cudaMemcpyDeviceToHost, S.stream);

@@ -107,7 +107,9 @@ __global__ void __launch_bounds__(256) cols_dot_kernel(const double *__restrict_
       if (SKIP && !nzc[(int64_t)((i0 + i) >> 6) * nz_ld]) continue;
       double2 q = ld_stream2(base + (int64_t)i * ld); double w = us[i]; a0 += q.x * w; a1 += q.y * w;
     }
-    *reinterpret_cast<double2 *>(cpart + (int64_t)rs * ncols + c) = make_double2(a0, a1);
+    double *dst = cpart + (int64_t)rs * ncols + c;
+    if (ncols & 1) { dst[0] = a0; dst[1] = a1; }   // odd row pitch: the rows of splits rs >= 1 start at odd offsets
+    else *reinterpret_cast<double2 *>(dst) = make_double2(a0, a1);
   } else {
     for (; i < nr; i++) a0 += base[(int64_t)i * ld] * us[i];
     cpart[(int64_t)rs * ncols + c] = a0;

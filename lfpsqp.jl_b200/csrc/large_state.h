@@ -81,6 +81,10 @@ struct LargeState {
   cudaStream_t side_stream = nullptr;                  // look-ahead of the blocked Cholesky (large.cu::factorize)
   cudaEvent_t ev_panel = nullptr, ev_potf = nullptr;
   std::vector<void *> owned;
+  // lfpsqp_large_last_dispatch: what the last large-n entry call enqueued, recorded on the host where the launches are made and
+  // cleared by every entry call (LARGE_DISP_* below).  disp_syrk: the product being enqueued is the Gram's SYRK.
+  int64_t disp[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+  bool disp_syrk = false;
   // counters
   int64_t collectives = 0, launches = 0, projcg_iters = 0, projcg_negcurv = 0, armijo_trials = 0, retract_outer = 0, retract_pcg = 0,
           pp_backtracks = 0, newton_accepted = 0, factorizations = 0, f_evals = 0;
@@ -91,6 +95,21 @@ struct LargeState {
     newton_accepted = factorizations = f_evals = 0;
   }
 };
+
+// entries of LargeState::disp (the layout of lfpsqp_large_last_dispatch, include/lfpsqp_b200.h)
+enum {
+  LARGE_DISP_GEMM = 0,          // mask of dgemm_nt instantiations
+  LARGE_DISP_KSPLIT_GRID = 1,   // largest split-K factor of a product with too few tiles for the GPU (0: none)
+  LARGE_DISP_KSPLIT_WAVE = 2,   // largest wave-quantisation split-K factor of a SYRK (0: none)
+  LARGE_DISP_ROWS_DOT = 3,      // mask of rows_dot_kernel instantiations
+  LARGE_DISP_FUSED_SINGLE = 4,  // launches of the single-GPU explicit-inverse fused projcg kernel (large_fused_single.cu)
+  LARGE_DISP_FUSED_GENERAL = 5, // launches of the general fused projcg kernel (large_fused.cu)
+  LARGE_DISP_FUSED_PCG = 6,     // launches of the fused pcg! kernel
+  LARGE_DISP_SOLVE = 7,         // mask of the forms u = G^-1 t was applied in
+};
+enum { LARGE_SOLVE_EXPLICIT = 1, LARGE_SOLVE_TRIANGULAR = 2, LARGE_SOLVE_PINV = 4 };
+// the solve form of a fused kernel that applies S.Ginv: G^-1, or G^+ once the factorisation lost rank (large.cu::factorize_pinv)
+inline int64_t large_ginv_form(const LargeState &S) { return S.pinv_active ? LARGE_SOLVE_PINV : LARGE_SOLVE_EXPLICIT; }
 
 // large_fused.cu: one cooperative kernel per chunk of projcg iterations (returns 1 when not eligible -> unfused path)
 int fused_projcg_chunk(LargeState &S, int iters, int first, double *xs, double *r, double *dc, double *Ad, double *rp, double *gp);
