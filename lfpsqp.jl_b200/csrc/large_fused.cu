@@ -34,18 +34,15 @@ namespace {
 
 constexpr int FT = 512;      // threads per CTA
 constexpr int TR = 16;       // rows per sweep of the triangular phases
-#ifndef FZ_CU
-#define FZ_CU 16
-#endif
-constexpr int CU = FZ_CU;   // 128-bit loads in flight per thread in the streaming phases
+constexpr int CU = 16;       // 128-bit loads in flight per thread in the streaming phases
 constexpr int RCH = 2048;    // column pairs per shared-memory chunk of rp in the row phase (2 buffers x 32 KB)
+constexpr size_t SMEM_MAX = 220 * 1024;   // dynamic shared memory opted in for every fused kernel (larger m: not eligible)
 
 struct FusedArgs {
   int64_t n, ldj, ldm;       // local columns (even), leading dimensions
   int m;
   const double *J, *Ginv, *hd, *Linv, *XT;
   double *xs, *dc, *r, *Ad, *rp, *gp, *tm, *tu, *ty;
-  int solve_mode;            // 0: explicit G^-1 (one phase; sharded over the ranks when column-sharded), 1: two triangular phases
   int *abort_flag;           // column-sharded: raised by a CTA whose peer-memory exchange timed out (see GridBar)
   double *part;              // 3 x gridDim partials: d.Ad | rp.gp | gp.gp
   const double *lp_rg;       // first chunk: partials of r.r from cg_init (loop slot 3)
@@ -179,6 +176,9 @@ __device__ __forceinline__ void cta_sum_multi(double (&v)[NV], double *shm /* (F
 // over the whole phase and all CTAs finish together); v goes through double-buffered shared-memory chunks (one L2
 // read per CTA instead of one per row); CU x 128-bit loads in flight per lane.  Single GPU: t -> a.tm.  Column-sharded:
 // {partial t_i, exchange number e} is pushed into every rank's mailbox row [my rank] with one 128-bit store per peer.
+// The main loop runs over whole blocks of CU x 32 pairs and keeps its loads free of bounds tests: with a predicate on each
+// load ptxas interleaves the loads with their uses (runs of 1-5 in flight instead of CU).  A partial block goes through the
+// tail loop, in the same per-lane summation order.
 template <bool SKIP = false>
 __device__ __forceinline__ void fz_rows(const FusedArgs &a, const double *v, double2 *vch, bool multi, unsigned long long e) {
   const int G = gridDim.x, c = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, m = a.m;
@@ -205,13 +205,17 @@ __device__ __forceinline__ void fz_rows(const FusedArgs &a, const double *v, dou
       }
       if (act) {
         const double *rb = row + 2 * base;
-        for (int p = lane; p < len; p += 32 * CU) {
+        int p = lane;
+        for (; p + (CU - 1) * 32 < len; p += 32 * CU) {
           double2 q[CU];
 #pragma unroll
-          for (int k = 0; k < CU; k++) { const int pp = p + k * 32; q[k] = (pp < len && (!SKIP || nzr[(base + pp) >> 3])) ? ld_stream2(rb + 2 * pp) : make_double2(0.0, 0.0); }
-          asm volatile("" ::: "memory");   // all CU loads are issued before the first shared-memory operand is fetched (bytes in flight)
+          for (int k = 0; k < CU; k++) { const int pp = p + k * 32; q[k] = (!SKIP || nzr[(base + pp) >> 3]) ? ld_stream2(rb + 2 * pp) : make_double2(0.0, 0.0); }
 #pragma unroll
-          for (int k = 0; k < CU; k++) { const int pp = p + k * 32; if (pp < len) { const double2 w = cur[pp]; acc += q[k].x * w.x + q[k].y * w.y; } }
+          for (int k = 0; k < CU; k++) { const double2 w = cur[p + k * 32]; acc += q[k].x * w.x + q[k].y * w.y; }
+        }
+        for (; p < len; p += 32) {
+          const double2 q = (!SKIP || nzr[(base + p) >> 3]) ? ld_stream2(rb + 2 * p) : make_double2(0.0, 0.0);
+          const double2 w = cur[p]; acc += q.x * w.x + q.y * w.y;
         }
       }
       __syncthreads();
@@ -348,9 +352,9 @@ __device__ __noinline__ bool fz_solve_sharded(const double *Ginv, int64_t ldm, i
   return ok;
 }
 
-// MULTI = column-sharded (world > 1): compiled separately so that the single-GPU kernel carries none of the mailbox code
-// (its registers go to the loads in flight of the streaming phases).
-template <bool MULTI>
+// MULTI = column-sharded (world > 1); TRI = the two triangular solve phases (large.cu::factorize's explicit-inverse guard)
+// instead of one phase with the explicit G^-1.  Each instantiation carries only its own solve and exchange code.
+template <bool MULTI, bool TRI>
 __global__ void __launch_bounds__(FT, 1) fused_projcg_kernel(FusedArgs a) {
   __shared__ int s_abort;
   GridBar grid{a.bar, 0u, gridDim.x, MULTI ? a.abort_flag : nullptr, &s_abort};
@@ -442,23 +446,23 @@ __global__ void __launch_bounds__(FT, 1) fused_projcg_kernel(FusedArgs a) {
     tick(2);
     // ---- u = G^-1 t.  Well-conditioned factor: the explicit symmetric inverse G^-1 = L^-T L^-1 (formed once per
     // factorisation by a DMMA GEMM) makes this ONE grid phase -- sharded over the ranks when column-sharded (each rank
-    // solves m / world rows and pushes its slice of u).  Otherwise (a.solve_mode == 1, large.cu::factorize's pivot-ratio
-    // guard): two dependent triangular phases y = L^-1 t, u = L^-T y with the accuracy of a triangular solve.
-    if (a.solve_mode == 0 && multi) {
-      if (!fz_solve_sharded(a.Ginv, a.ldm, m, a.rank, a.world, s_peer, ep, ep + 1, fsm)) grid.raise();
-      ++ep;
-    } else if (a.solve_mode == 0) {
-      fz_matvec(a.Ginv, a.ldm, m, a.tm, nullptr, 1, 0ULL, a.tu, red_d);
-    } else {
+    // solves m / world rows and pushes its slice of u).  Otherwise (TRI, large.cu::factorize's explicit-inverse guard):
+    // two dependent triangular phases y = L^-1 t, u = L^-T y with the accuracy of a triangular solve.
+    if constexpr (TRI) {
       if (!fz_matvec(a.Linv, a.ldm, m, a.tm, multi ? s_peer[a.rank] : nullptr, a.world, ep, a.ty, red_d)) grid.raise();
       if (grid.sync()) { status = 5; break; }
       fz_matvec(a.XT, a.ldm, m, a.ty, nullptr, 1, 0ULL, a.tu, red_d);
+    } else if constexpr (MULTI) {
+      if (!fz_solve_sharded(a.Ginv, a.ldm, m, a.rank, a.world, s_peer, ep, ep + 1, fsm)) grid.raise();
+      ++ep;
+    } else {
+      fz_matvec(a.Ginv, a.ldm, m, a.tm, nullptr, 1, 0ULL, a.tu, red_d);
     }
     if (grid.sync()) { status = 5; break; }
     tick(3);
     // ---- cols: gp = rp - J' u on the owned columns ; partials rp.gp, gp.gp
     {
-      if (a.solve_mode == 0 && multi) {
+      if constexpr (MULTI && !TRI) {
         bool ok = true;
         const LLEntry *ub = ll_u(a.peer[a.rank]);
         for (int i0 = tid; i0 < m; i0 += 4 * FT) {       // 4 independent polls in flight per thread
@@ -631,18 +635,16 @@ __global__ void __launch_bounds__(FT, 1) fused_pcg_kernel(FusedArgs a) {
 }  // namespace
 
 // Returns 0 when the chunk was enqueued, 1 when this configuration is not eligible (the caller uses the unfused path).
-int fused_projcg_chunk_single(LargeState &S, int iters, int first, double *xs, double *r, double *dc, double *Ad, double *rp, double *gp);   // large_fused_single.cu
 int fused_projcg_chunk(LargeState &S, int iters, int first, double *xs, double *r, double *dc, double *Ad, double *rp, double *gp) {
   if (S.ineq || S.family != LFPSQP_FAM_DIAGQUAD || (S.n_loc & 1) || S.m < 1 || !S.fused_ok || !S.Ginv) return 1;
-  if (S.world <= 1 && S.explicit_inverse_ok) return fused_projcg_chunk_single(S, iters, first, xs, r, dc, Ad, rp, gp);
   if (S.world > 1 && !(S.comm && S.comm->peer_ready && S.m <= PC_MAX && S.world <= PC_RANKS)) return 1;
+  const bool multi = S.world > 1, tri = !S.explicit_inverse_ok;
   FusedArgs a;
   for (int r = 0; r < PC_RANKS; r++) a.peer[r] = (S.world > 1) ? S.comm->peer_map[r] : nullptr;
   a.rank = S.rank; a.world = S.world; a.epoch = (S.world > 1) ? reinterpret_cast<unsigned long long *>(S.comm->peer_local + FZ_FLAG + PC_RANKS) : nullptr;   // lives with the region
   a.n = S.n_loc; a.ldj = S.ldj; a.ldm = S.ldm; a.m = S.m;
   a.J = S.J; a.Ginv = S.Ginv; a.hd = S.hdiag; a.Linv = S.Linv; a.XT = S.XT;
   a.xs = xs; a.dc = dc; a.r = r; a.Ad = Ad; a.rp = rp; a.gp = gp; a.tm = S.tm; a.tu = S.tu; a.ty = S.ty;
-  a.solve_mode = S.explicit_inverse_ok ? 0 : 1;
   a.abort_flag = reinterpret_cast<int *>(S.fused_part + 3 * (size_t)S.fused_grid + 14);
   a.part = S.fused_part; a.lp_rg = S.lp + 3 * (size_t)MAXP; a.np_rg = S.np_loop; a.first = first; a.max_iters = iters;
   a.ctrl = S.ctrl;
@@ -652,11 +654,13 @@ int fused_projcg_chunk(LargeState &S, int iters, int first, double *xs, double *
   a.prof = want_prof ? S.fused_part + 3 * (size_t)S.fused_grid : nullptr;
   const size_t smem = ((size_t)((S.m + 1) & ~1) + 2 * FT + 4 * RCH) * sizeof(double);
   void *args[] = {&a};
-  cudaError_t e = cudaLaunchCooperativeKernel(S.world > 1 ? (void *)fused_projcg_kernel<true> : (void *)fused_projcg_kernel<false>, dim3(S.fused_grid),
-                                              dim3(FT), args, smem, S.stream);
+  void *kern = multi ? (tri ? (void *)fused_projcg_kernel<true, true> : (void *)fused_projcg_kernel<true, false>)
+                     : (tri ? (void *)fused_projcg_kernel<false, true> : (void *)fused_projcg_kernel<false, false>);
+  cudaError_t e = cudaLaunchCooperativeKernel(kern, dim3(S.fused_grid), dim3(FT), args, smem, S.stream);
   if (e != cudaSuccess) { cudaGetLastError(); S.fused_ok = false; return 1; }
   S.launches++;
-  S.disp[LARGE_DISP_FUSED_GENERAL]++; S.disp[LARGE_DISP_SOLVE] |= a.solve_mode == 0 ? large_ginv_form(S) : (int64_t)LARGE_SOLVE_TRIANGULAR;
+  S.disp[multi || tri ? LARGE_DISP_FUSED_GENERAL : LARGE_DISP_FUSED_SINGLE]++;
+  S.disp[LARGE_DISP_SOLVE] |= tri ? (int64_t)LARGE_SOLVE_TRIANGULAR : large_ginv_form(S);
   if (want_prof) {
     double h[8];
     cudaMemcpyAsync(h, a.prof, sizeof(h), cudaMemcpyDeviceToHost, S.stream);
@@ -679,7 +683,6 @@ int fused_pcg(LargeState &S, double *dx, double *r, double *pv, double *z) {
   a.n = S.n_loc; a.ldj = S.ldj; a.ldm = S.ldm; a.m = S.m;
   a.J = S.J; a.Ginv = nullptr; a.hd = nullptr; a.Linv = nullptr; a.XT = nullptr;
   a.xs = dx; a.dc = pv; a.r = r; a.Ad = z; a.rp = nullptr; a.gp = nullptr; a.tm = S.tm; a.tu = S.tu; a.ty = S.ty;
-  a.solve_mode = 0;
   a.abort_flag = reinterpret_cast<int *>(S.fused_part + 3 * (size_t)S.fused_grid + 14);
   a.part = S.fused_part; a.lp_rg = S.lp + 5 * (size_t)MAXP; a.np_rg = S.np_loop_raw; a.first = 1; a.max_iters = 0;
   a.ctrl = S.ctrl; a.prof = nullptr;
@@ -704,14 +707,16 @@ void fused_projcg_init(LargeState &S, int device) {
   int coop = 0;
   if (cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, device) != cudaSuccess || !coop) { cudaGetLastError(); return; }
   const size_t smem = ((size_t)((S.m + 1) & ~1) + 2 * FT + 4 * RCH) * sizeof(double);
-  if (smem > 220 * 1024) return;
-  if (cudaFuncSetAttribute(fused_projcg_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess ||
-      cudaFuncSetAttribute(fused_projcg_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess ||
-      cudaFuncSetAttribute(fused_pcg_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess ||
-      cudaFuncSetAttribute(fused_pcg_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess ||
-      cudaFuncSetAttribute(fused_pcg_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) { cudaGetLastError(); return; }
+  if (smem > SMEM_MAX) return;
+  // the attribute is per kernel and process-wide: opting in to the eligibility limit (not this context's size) keeps a
+  // context with a larger m launchable after a smaller one was set up
+  const void *kernels[] = {(const void *)fused_projcg_kernel<false, false>, (const void *)fused_projcg_kernel<false, true>,
+                           (const void *)fused_projcg_kernel<true, false>, (const void *)fused_projcg_kernel<true, true>,
+                           (const void *)fused_pcg_kernel<false>, (const void *)fused_pcg_kernel<false, true>, (const void *)fused_pcg_kernel<true>};
+  for (const void *k : kernels)
+    if (cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_MAX) != cudaSuccess) { cudaGetLastError(); return; }
   int per_sm = 0;
-  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fused_projcg_kernel<true>, FT, smem) != cudaSuccess || per_sm < 1) { cudaGetLastError(); return; }
+  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fused_projcg_kernel<true, false>, FT, smem) != cudaSuccess || per_sm < 1) { cudaGetLastError(); return; }
   S.fused_grid = S.sm_count;
   void *p = nullptr;
   if (cudaMalloc(&p, (3 * (size_t)S.fused_grid + 16) * sizeof(double)) != cudaSuccess) { cudaGetLastError(); return; }   // partials | 9 prof | barrier | abort

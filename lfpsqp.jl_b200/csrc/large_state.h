@@ -102,8 +102,8 @@ enum {
   LARGE_DISP_KSPLIT_GRID = 1,   // largest split-K factor of a product with too few tiles for the GPU (0: none)
   LARGE_DISP_KSPLIT_WAVE = 2,   // largest wave-quantisation split-K factor of a SYRK (0: none)
   LARGE_DISP_ROWS_DOT = 3,      // mask of rows_dot_kernel instantiations
-  LARGE_DISP_FUSED_SINGLE = 4,  // launches of the single-GPU explicit-inverse fused projcg kernel (large_fused_single.cu)
-  LARGE_DISP_FUSED_GENERAL = 5, // launches of the general fused projcg kernel (large_fused.cu)
+  LARGE_DISP_FUSED_SINGLE = 4,  // launches of the single-GPU explicit-inverse fused projcg kernel (fused_projcg_kernel<false, false>)
+  LARGE_DISP_FUSED_GENERAL = 5, // launches of the other fused projcg instantiations (column-sharded or triangular solve)
   LARGE_DISP_FUSED_PCG = 6,     // launches of the fused pcg! kernel
   LARGE_DISP_SOLVE = 7,         // mask of the forms u = G^-1 t was applied in
 };
