@@ -114,6 +114,26 @@ typedef struct {
 #define LFPSQP_FAM_QCQP 101   /* fam_params = (const double*)(const lfpsqp_qcqp*), fam_stride must be 0 */
 
 /*
+ * Sparse QCQP (large-n mode only, one GPU; lfpsqp_solve_batched* return LFPSQP_ERR_FAMILY for it):
+ *   f(x)   = 1/2 x'P x + q.x + r
+ *   c_i(x) = 1/2 x'Qc_i x + Ac_i.x - bc_i = 0      i < m
+ * Matrices are coordinate lists with 0-based indices; all arrays are host memory (params_on_device = 1 is LFPSQP_ERR_ARG).
+ * P and every Qc_i are n x n and exactly symmetric (both triangles given); Qc stacks the m matrices: entry k belongs to
+ * Qc_{mat[k]}.  Ac is m x n: row = constraint, col = variable.  mat is NULL for P and Ac.  q and bc may be NULL (= 0).
+ * Setup rejects (LFPSQP_ERR_ARG) an index out of range, a duplicate entry, a matrix that is not exactly symmetric, a
+ * non-finite value, and nnz > 0 with a NULL array.  Limits: n < 2^31 and every nnz, as well as the union pattern of
+ * P + sum_i Qc_i and its source count, < 2^31 (32-bit indices on the device).  d(x) <= 0 and dl <= d(x) <= du are
+ * written as data with slack variables: see INTEGRATION.md.
+ */
+typedef struct { int64_t nnz; const int64_t *mat, *row, *col; const double *val; } lfpsqp_coo;
+typedef struct {
+  lfpsqp_coo P;  const double *q;  double r;
+  lfpsqp_coo Qc;
+  lfpsqp_coo Ac;  const double *bc;
+} lfpsqp_sparse_qcqp;
+#define LFPSQP_FAM_SPARSE_QCQP 102   /* fam_params = (const double*)(const lfpsqp_sparse_qcqp*) */
+
+/*
  * Host callbacks of the explicit-derivative core optimize(f, grad!, c!, jac!, hess_lag_vec!, x0, xl, xu, m, param)
  * (src/optimize.jl:119-143).  Conventions are the reference's (src/autodiff_generators.jl:7-9, :40-42, :80-104):
  * x is the first n entries of the working vector (optimize.jl:259 passes view(x, 1:n)); jac! fills Jc (m x n,
@@ -191,7 +211,8 @@ int lfpsqp_solve_batched_dev(lfpsqp_ctx *ctx, int family, int64_t n, int64_t m, 
  * Large-n mode: ONE instance with a dense m x n constraint Jacobian, host-orchestrated whole-GPU kernels
  * (FP64 DMMA Gram + blocked Cholesky replace ksvd!, src/la_helper.jl:8-34 / optimize.jl:291-293; streaming passes over
  * J replace kgemv!, la_helper.jl:36-44).  Families: LFPSQP_FAM_DIAGQUAD, LFPSQP_FAM_THOMSON,
- * LFPSQP_FAM_HOST (params = const lfpsqp_host_callbacks*); LFPSQP_FAM_QCQP is LFPSQP_ERR_FAMILY here.  Finite bounds xl <= x <= xu run the reference's 2n-variable
+ * LFPSQP_FAM_HOST (params = const lfpsqp_host_callbacks*), LFPSQP_FAM_SPARSE_QCQP (params = const lfpsqp_sparse_qcqp*; one GPU);
+ * LFPSQP_FAM_QCQP is LFPSQP_ERR_FAMILY here.  Finite bounds xl <= x <= xu run the reference's 2n-variable
  * embedding (src/inequality_helper.jl): lfpsqp_large_set_bounds after lfpsqp_large_setup, or the xl/xu arguments of
  * lfpsqp_solve_large / lfpsqp_solve_host.  projcg! on diagonal Lagrangian Hessians and pcg! run as persistent cooperative
  * kernels (large_fused.cu); LFPSQP_FUSED_PROJCG=0 in the environment selects the launch-per-phase loops.

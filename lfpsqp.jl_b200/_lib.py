@@ -27,6 +27,14 @@ class CQcqp(C.Structure):  # lfpsqp_qcqp: nine {const double*, int64 batch strid
     _fields_ = [f for name in QCQP_FIELDS for f in ((name, C.c_void_p), (name + "_stride", C.c_int64))]
 
 
+class CCoo(C.Structure):  # lfpsqp_coo: 0-based coordinate list; mat = constraint index of each entry (Qc) or NULL
+    _fields_ = [("nnz", C.c_int64), ("mat", C.c_void_p), ("row", C.c_void_p), ("col", C.c_void_p), ("val", C.c_void_p)]
+
+
+class CSparseQcqp(C.Structure):  # lfpsqp_sparse_qcqp
+    _fields_ = [("P", CCoo), ("q", C.c_void_p), ("r", C.c_double), ("Qc", CCoo), ("Ac", CCoo), ("bc", C.c_void_p)]
+
+
 TERM_DTYPE = np.dtype([("condition", "<i4"), ("status", "<i4"), ("f_diff", "<f8"), ("step_diff", "<f8"),
                        ("kkt_diff", "<f8"), ("iter", "<i8")])
 STATS_FIELDS = ("projcg_iters", "projcg_negcurv", "armijo_trials", "retract_outer", "retract_pcg", "pp_backtracks",

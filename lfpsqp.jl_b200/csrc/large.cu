@@ -214,6 +214,16 @@ static void host_x(LargeState &S, const double *x) {
 __global__ void set_partials_kernel(double *part, int np, double v) {
   for (int i = threadIdx.x; i < np; i += blockDim.x) part[i] = (i == 0) ? v : 0.0;
 }
+// SPARSE_QCQP CSR passes (spq_csr_kernel): mode 0 f partials, 1 grad, 2 Hessian action; G lanes per row from setup
+static void spq_csr(LargeState &S, int mode, const int *rp, const int *ci, const double *v, int lanes, const double *x, double *y,
+                    double *part, int pred) {
+  const lfpsqp::SpqDev &D = S.spq;
+  const int64_t n = D.n;
+#define SPQ_CSR(G, M) spq_csr_kernel<G, M><<<S.vgrid, 256, 0, S.stream>>>(n, rp, ci, v, x, D.q, D.r, y, part, S.ctrl, pred)
+  if (lanes == 32) { if (mode == 0) SPQ_CSR(32, 0); else if (mode == 1) SPQ_CSR(32, 1); else SPQ_CSR(32, 2); }
+  else { if (mode == 0) SPQ_CSR(4, 0); else if (mode == 1) SPQ_CSR(4, 1); else SPQ_CSR(4, 2); }
+#undef SPQ_CSR
+}
 static void fam_f(LargeState &S, const double *x) {  // -> gpart slot 0 (sum); caller finalizes s[0]
   if (S.family == LFPSQP_FAM_HOST) {
     host_x(S, x);
@@ -223,6 +233,8 @@ static void fam_f(LargeState &S, const double *x) {  // -> gpart slot 0 (sum); c
   } else if (S.family == LFPSQP_FAM_DIAGQUAD) {
     const double *xt = S.p_xt, *w = S.p_w;
     vec(S, S.n_loc, [=] __device__(int64_t j, double *acc) { double t = x[j] - xt[j]; acc[0] += 0.5 * w[j] * t * t; }, 0, 1);
+  } else if (S.family == LFPSQP_FAM_SPARSE_QCQP) {
+    spq_csr(S, 0, S.spq.prow, S.spq.pcol, S.spq.pval, S.spq.gp, x, nullptr, S.gpart, 0);
   } else {
     const int np = (int)(S.n / 3), npl = (int)(S.n_loc / 3), i0 = (int)(S.col0 / 3);
     const double *xf = thomson_gather(S, x, S.xfull);
@@ -241,6 +253,8 @@ static void fam_grad(LargeState &S, double *g, const double *x) {
   } else if (S.family == LFPSQP_FAM_DIAGQUAD) {
     const double *xt = S.p_xt, *w = S.p_w;
     vec(S, S.n_loc, [=] __device__(int64_t j, double *) { g[j] = w[j] * (x[j] - xt[j]); });
+  } else if (S.family == LFPSQP_FAM_SPARSE_QCQP) {
+    spq_csr(S, 1, S.spq.prow, S.spq.pcol, S.spq.pval, S.spq.gp, x, g, nullptr, 0);
   } else {
     const int np = (int)(S.n / 3), npl = (int)(S.n_loc / 3), i0 = (int)(S.col0 / 3);
     const double *xf = thomson_gather(S, x, S.xfull);
@@ -274,6 +288,12 @@ static void fam_c_jac(LargeState &S, double *Jout, double *cval, const double *x
     const double *b = S.p_b;
     vec(S, m, [=] __device__(int64_t i, double *) { cval[i] -= b[i]; });
     S.launches += 2;
+  } else if (S.family == LFPSQP_FAM_SPARSE_QCQP) {
+    if (m <= 0) return;
+    const lfpsqp::SpqDev &D = S.spq;
+    if (Jout) spq_cjac_kernel<true><<<m, 256, 0, S.stream>>>(D.con_ptr, D.seg_row, D.seg_a, D.seg_ptr, D.seg_col, D.seg_val, D.bc, x, Jout, S.ldj, cval);
+    else spq_cjac_kernel<false><<<m, 256, 0, S.stream>>>(D.con_ptr, D.seg_row, D.seg_a, D.seg_ptr, D.seg_col, D.seg_val, D.bc, x, nullptr, S.ldj, cval);
+    S.launches++;
   } else {
     if (Jout) cudaMemsetAsync(Jout, 0, (size_t)m * S.ldj * sizeof(double), S.stream);  // dense-treated, as the reference
     const int npl = (int)(S.n_loc / 3), i0 = (int)(S.col0 / 3);
@@ -302,6 +322,12 @@ static void fam_hess_prepare(LargeState &S, const double *x, const double *lam) 
       hd[j] = s;
     });
     S.launches++;
+  } else if (S.family == LFPSQP_FAM_SPARSE_QCQP) {  // values of H = P + sum_i lam_i Qc_i on the union pattern (fixed source order)
+    const lfpsqp::SpqDev &D = S.spq;
+    if (D.nh <= 0) return;
+    const int grid = (int)std::min<int64_t>((D.nh + 255) / 256, 8 * (int64_t)S.sm_count);
+    spq_hess_assemble_kernel<<<grid, 256, 0, S.stream>>>(D.nh, D.hsrc_ptr, D.hsrc_con, D.hsrc_val, lam, D.hval);
+    S.launches++;
   }
 }
 // dest = H src, partial src.dest -> loop-partial slot 0 ; returns the number of partials written
@@ -318,6 +344,10 @@ static int fam_hess(LargeState &S, double *dest, const double *src, const double
     const double *hd = S.hdiag; const LargeCtrl *ctrl = S.ctrl; double *lp = S.lp;
     // predicated elementwise kernel with the d.Ad partial (hdiag carries the bound terms: nv entries)
     hess_diag_kernel<<<S.vgrid, 256, 0, S.stream>>>(S.nv, hd, src, dest, lp, ctrl, pred);
+    S.launches++;
+    return S.vgrid;
+  } else if (S.family == LFPSQP_FAM_SPARSE_QCQP) {   // CSR pass over the assembled H; with bounds ineq_hess_aug_kernel writes the partial
+    spq_csr(S, 2, S.spq.hrow, S.spq.hcol, S.spq.hval, S.spq.gh, src, dest, S.ineq ? nullptr : S.lp, pred);
     S.launches++;
     return S.vgrid;
   } else {
@@ -1154,10 +1184,12 @@ extern "C" int lfpsqp_large_setup(lfpsqp_ctx *c, int family, int64_t n_global, i
                                   const double *params, int params_on_device) {
   if (!c) return LFPSQP_ERR_ARG;
   cudaSetDevice(c->device);
-  if (family != LFPSQP_FAM_DIAGQUAD && family != LFPSQP_FAM_THOMSON && family != LFPSQP_FAM_HOST)
-    return c->fail(LFPSQP_ERR_FAMILY, "large-n mode supports the DIAGQUAD, THOMSON and HOST (callback) families");
+  if (family != LFPSQP_FAM_DIAGQUAD && family != LFPSQP_FAM_THOMSON && family != LFPSQP_FAM_HOST && family != LFPSQP_FAM_SPARSE_QCQP)
+    return c->fail(LFPSQP_ERR_FAMILY, "large-n mode supports the DIAGQUAD, THOMSON, HOST (callback) and SPARSE_QCQP families");
   if (n_global < 1 || m < 0 || n_loc < 1 || col0 < 0 || col0 + n_loc > n_global || m > n_global)
     return c->fail(LFPSQP_ERR_ARG, "bad sizes for large-n setup");
+  if (family == LFPSQP_FAM_SPARSE_QCQP && (n_loc != n_global || c->comm.world > 1))
+    return c->fail(LFPSQP_ERR_FAMILY, "the SPARSE_QCQP family runs on one GPU (x'Qx couples column shards)");
   if (c->comm.world <= 1 && n_loc != n_global) return c->fail(LFPSQP_ERR_ARG, "a column shard needs a communicator (lfpsqp_comm_init)");
   if (family == LFPSQP_FAM_THOMSON && (n_global % 3 || m != n_global / 3 || n_loc % 3 || col0 % 3))
     return c->fail(LFPSQP_ERR_FAMILY, "THOMSON needs n = 3 m and column shards of whole points (col0 and n_loc multiples of 3)");
@@ -1167,6 +1199,13 @@ extern "C" int lfpsqp_large_setup(lfpsqp_ctx *c, int family, int64_t n_global, i
     if (!cb || !cb->f || !cb->grad || !cb->hess_lag_vec || (m > 0 && (!cb->c || !cb->jac)))
       return c->fail(LFPSQP_ERR_ARG, "HOST family: f, grad, hess_lag_vec (and c, jac when m > 0) callbacks are required");
     if (n_loc != n_global || c->comm.world > 1) return c->fail(LFPSQP_ERR_FAMILY, "the HOST (callback) family runs on one GPU");
+  }
+  SpqHost spq_host;   // validated and canonicalised before any previous state is released
+  if (family == LFPSQP_FAM_SPARSE_QCQP) {
+    if (!params) return c->fail(LFPSQP_ERR_ARG, "SPARSE_QCQP: params must point to a lfpsqp_sparse_qcqp descriptor");
+    if (params_on_device) return c->fail(LFPSQP_ERR_ARG, "SPARSE_QCQP: the descriptor and its arrays are host memory (params_on_device must be 0)");
+    int rc = spq_build(c, (const lfpsqp_sparse_qcqp *)params, n_global, m, spq_host);
+    if (rc) return rc;
   }
   lfpsqp_large_release(c);
   LargeState *Sp = new LargeState(); LargeState &S = *Sp;
@@ -1238,6 +1277,10 @@ extern "C" int lfpsqp_large_setup(lfpsqp_ctx *c, int family, int64_t n_global, i
     }
     S.p_Q = blob; S.p_A = blob + (size_t)m * nl; S.p_b = S.p_A + (size_t)m * nl; S.p_xt = S.p_b + m; S.p_w = S.p_xt + nl;
     if ((((uintptr_t)S.p_A) & 15) || (((uintptr_t)S.p_Q) & 15)) { lfpsqp_large_release(c); return c->fail(LFPSQP_ERR_ARG, "parameter blob must be 16-byte aligned"); }
+  }
+  if (family == LFPSQP_FAM_SPARSE_QCQP && !spq_upload(S, spq_host)) {
+    lfpsqp_large_release(c);
+    return c->fail(LFPSQP_ERR_NOMEM, "SPARSE_QCQP: device allocation or upload of the structures failed");
   }
   cudaFuncSetAttribute(dgemm_nt_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dgemm_smem_bytes<128>());
   cudaFuncSetAttribute(dgemm_nt_kernel<128, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dgemm_smem_bytes<128>());

@@ -42,4 +42,21 @@ struct IneqDev {
   int64_t nx = 0;
 };
 
+// LFPSQP_FAM_SPARSE_QCQP (kernels in large_families.cuh, built by large_spq.cu): device copies of the canonical structures.
+// P and the Lagrangian Hessian H = P + sum_i lam_i Qc_i are CSR matrices (32-bit indices); every entry of H lists its sources
+// (con -1 = the P entry, else the constraint), P first and then constraints in index order.  The constraints are segments
+// (i, r), sorted by i then r: row r of Qc_i merged with Ac[i, r], so that J[i, r] has exactly one owner.
+struct SpqDev {
+  int64_t n = 0, nh = 0;
+  int m = 0, gp = 4, gh = 4;                    // gp / gh: lanes per row of the P / H passes
+  const int *prow = nullptr, *pcol = nullptr;
+  const double *pval = nullptr, *q = nullptr;
+  double r = 0.0;
+  const int *hrow = nullptr, *hcol = nullptr, *hsrc_ptr = nullptr, *hsrc_con = nullptr;
+  const double *hsrc_val = nullptr;
+  double *hval = nullptr;
+  const int *con_ptr = nullptr, *seg_row = nullptr, *seg_ptr = nullptr, *seg_col = nullptr;
+  const double *seg_a = nullptr, *seg_val = nullptr, *bc = nullptr;
+};
+
 }  // namespace lfpsqp

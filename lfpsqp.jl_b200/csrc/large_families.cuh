@@ -147,4 +147,78 @@ __global__ void thomson_c_kernel(int npl, int i0, const double *__restrict__ x, 
   if (J) { double *r = J + (int64_t)(i0 + i) * ld + 3 * i; r[0] = 2.0 * a; r[1] = 2.0 * b; r[2] = 2.0 * c; }
 }
 
+// ================================================================== SPARSE_QCQP (LFPSQP_FAM_SPARSE_QCQP, one GPU)
+// f = 1/2 x'P x + q.x + r ; c_i = 1/2 x'Qc_i x + Ac_i.x - bc_i.  Structures: SpqDev (large_ctrl.h).  Every sum has a fixed
+// order (no atomics): two solves of one problem are bit-identical.
+
+// CSR pass y = A x with G lanes per row (rows handed out warp-uniformly, so every lane of a warp takes the shuffles)
+//   MODE 0: f partial sum_r x_r (1/2 (Ax)_r + q_r) -> part[blockIdx.x] (block 0 adds r0)
+//   MODE 1: y = A x + q (grad)
+//   MODE 2: y = A x (Hessian action), partial x.y -> part[blockIdx.x] unless part is NULL; predicated on ctrl->status
+template <int G, int MODE>
+__global__ void __launch_bounds__(256) spq_csr_kernel(int64_t n, const int *__restrict__ rp, const int *__restrict__ ci,
+                                                      const double *__restrict__ v, const double *__restrict__ x,
+                                                      const double *__restrict__ q, double r0, double *__restrict__ y,
+                                                      double *part, const LargeCtrl *ctrl, int pred) {
+  if (MODE == 2 && pred == 1 && ctrl->status != 0) return;
+  __shared__ double sh[33];
+  constexpr int RPW = 32 / G;   // rows per warp and step
+  const int lane = threadIdx.x & 31, sub = lane % G;
+  const int64_t warp = ((int64_t)blockIdx.x * 256 + threadIdx.x) >> 5, nwarp = (int64_t)gridDim.x * 8;
+  double acc = 0.0;
+  for (int64_t row0 = warp * RPW; row0 < n; row0 += nwarp * RPW) {
+    const int64_t row = row0 + lane / G;
+    double s = 0.0;
+    if (row < n) {
+      const int k1 = rp[row + 1];
+      for (int k = rp[row] + sub; k < k1; k += G) s += v[k] * x[ci[k]];
+    }
+#pragma unroll
+    for (int o = G / 2; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+    if (sub == 0 && row < n) {
+      if (MODE == 0) acc += x[row] * (0.5 * s + q[row]);
+      else if (MODE == 1) y[row] = s + q[row];
+      else { y[row] = s; acc += x[row] * s; }
+    }
+  }
+  if (MODE == 0 || (MODE == 2 && part)) {
+    const double t = block_sum(acc, sh);
+    if (threadIdx.x == 0) part[blockIdx.x] = (MODE == 0 && blockIdx.x == 0) ? t + r0 : t;
+  }
+}
+
+// values of H on its union pattern: hval[e] = sum over the sources of e, in their stored order, of (P entry | lam_i Qc_i entry)
+__global__ void __launch_bounds__(256) spq_hess_assemble_kernel(int64_t nh, const int *__restrict__ sp, const int *__restrict__ con,
+                                                                const double *__restrict__ val, const double *__restrict__ lam,
+                                                                double *__restrict__ hval) {
+  for (int64_t e = (int64_t)blockIdx.x * 256 + threadIdx.x; e < nh; e += (int64_t)gridDim.x * 256) {
+    double s = 0.0;
+    for (int k = sp[e]; k < sp[e + 1]; k++) { const int i = con[k]; s += (i < 0) ? val[k] : lam[i] * val[k]; }
+    hval[e] = s;
+  }
+}
+
+// one CTA per constraint i: cval[i] = sum over the segments (i, r) of x_r (1/2 (Qc_i x)_r + Ac[i, r]) - bc[i], and with
+// WRITE_J the structural entries J[i, r] = (Qc_i x)_r + Ac[i, r] (every other entry of J stays zero)
+template <bool WRITE_J>
+__global__ void __launch_bounds__(256) spq_cjac_kernel(const int *__restrict__ con_ptr, const int *__restrict__ seg_row,
+                                                       const double *__restrict__ seg_a, const int *__restrict__ seg_ptr,
+                                                       const int *__restrict__ seg_col, const double *__restrict__ seg_val,
+                                                       const double *__restrict__ bc, const double *__restrict__ x,
+                                                       double *__restrict__ J, int64_t ld, double *__restrict__ cval) {
+  __shared__ double sh[33];
+  const int i = blockIdx.x;
+  double acc = 0.0;
+  for (int s = con_ptr[i] + threadIdx.x; s < con_ptr[i + 1]; s += 256) {
+    double qx = 0.0;
+    for (int k = seg_ptr[s]; k < seg_ptr[s + 1]; k++) qx += seg_val[k] * x[seg_col[k]];
+    const int r = seg_row[s];
+    const double a = seg_a[s];
+    acc += x[r] * (0.5 * qx + a);
+    if (WRITE_J) J[(int64_t)i * ld + r] = qx + a;
+  }
+  const double t = block_sum(acc, sh);
+  if (threadIdx.x == 0) cval[i] = t - bc[i];
+}
+
 }  // namespace lfpsqp

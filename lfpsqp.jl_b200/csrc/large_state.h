@@ -17,6 +17,7 @@ struct LargeState {
   double *bq = nullptr, *br = nullptr, *bs = nullptr, *bt = nullptr;   // InequalityData (owned copies behind I.q .. I.t)
   double *cvh = nullptr, *cvc = nullptr;   // cvalaug = [h ; c] of ProjPenalty (retractions.jl:29), persistent across calls
   double *pb = nullptr, *Jw = nullptr;     // x-half operand of PJct' v ; J diag(Dy) for the weighted Gram
+  lfpsqp::SpqDev spq;                      // LFPSQP_FAM_SPARSE_QCQP: uploaded structures (large_spq.cu)
   // host-callback family (LFPSQP_FAM_HOST): the callbacks, pinned staging buffers, device staging of Jc (n x m)
   lfpsqp_host_callbacks cb = {};
   double *hx = nullptr, *hv = nullptr, *hw = nullptr, *hlam = nullptr, *hc = nullptr, *hJ = nullptr, *Jstage = nullptr;
@@ -115,6 +116,18 @@ inline int64_t large_ginv_form(const LargeState &S) { return S.pinv_active ? LAR
 int fused_projcg_chunk(LargeState &S, int iters, int first, double *xs, double *r, double *dc, double *Ad, double *rp, double *gp);
 int fused_pcg(LargeState &S, double *dx, double *r, double *pv, double *z);   // the whole pcg! call as one launch
 void fused_projcg_init(LargeState &S, int device);
+
+// large_spq.cu: LFPSQP_FAM_SPARSE_QCQP.  spq_build validates the descriptor (LFPSQP_ERR_ARG with a message) and builds the
+// canonical host form; spq_upload copies it into S.spq (false: allocation or copy failed)
+struct SpqHost {
+  int64_t n = 0;
+  int m = 0;
+  double r = 0.0;
+  std::vector<double> q, bc, pval, hsrc_val, seg_a, seg_val;
+  std::vector<int> prow, pcol, hrow, hcol, hsrc_ptr, hsrc_con, con_ptr, seg_row, seg_ptr, seg_col;
+};
+int spq_build(lfpsqp_ctx *c, const lfpsqp_sparse_qcqp *D, int64_t n, int64_t m, SpqHost &H);
+bool spq_upload(LargeState &S, const SpqHost &H);
 
 // large_eig.cu: eigen-decomposition of the Gram (one-sided Jacobi) -> scaled eigenvectors for the pseudo-inverse
 int large_eig_pinv_factors(LargeState &S, double *G, double *Vt, double *lam, int lower_only, int *sweeps_dev, unsigned long long *conv_dev,

@@ -15,6 +15,7 @@ from . import _lib
 
 ROSENBROCK, README_EQ, README_INEQ, THOMSON, DIAGQUAD, SIN, BOXQUAD = range(7)
 QCQP = 101
+SPARSE_QCQP = 102
 
 
 class DeviceCallback:
@@ -173,3 +174,207 @@ def qcqp(P=None, q=None, r=None, Qc=None, Ac=None, bc=None, Qd=None, Ad=None, bd
     for name in [k for k in arrays if _QCQP_SHAPES[k][:1] in ("m", "p") and dims[_QCQP_SHAPES[k][0]] == 0]:
         del arrays[name]      # empty constraint blocks: nothing to pass
     return QCQPFamily(arrays, n, m, p, B)
+
+
+def _coo_of(M, name):
+    """(row, col, val) of a matrix given as anything with .tocoo() (scipy.sparse) or as a dense 2-D array, and its shape"""
+    if hasattr(M, "tocoo"):
+        c = M.tocoo()
+        r, k, v, shape = c.row, c.col, c.data, tuple(c.shape)
+    else:
+        a = np.asarray(M, dtype=np.float64)
+        if a.ndim != 2:
+            raise _lib.LFPSQPError("sparse_qcqp: %s must be a matrix (2-D array or scipy.sparse), got shape %s" % (name, a.shape))
+        r, k = np.nonzero(a)
+        v, shape = a[r, k], a.shape
+    return np.asarray(r, np.int64), np.asarray(k, np.int64), np.asarray(v, np.float64), shape
+
+
+def _summed(r, k, v, ncols):
+    """duplicates summed (in input order), entries sorted by (row, col), exact zeros dropped"""
+    key, inv = np.unique(r * ncols + k, return_inverse=True)
+    s = np.bincount(inv.ravel(), weights=v, minlength=key.size)
+    nz = s != 0.0
+    return key[nz] // ncols, key[nz] % ncols, s[nz]
+
+
+def _symmetrised(r, k, v, n):
+    """(M + M')/2: each entry becomes 1/2 (M[r, c] + M[c, r]), a sum of two terms, so the result is exactly symmetric"""
+    r, k, v = _summed(r, k, v, n)
+    return _summed(np.concatenate([r, k]), np.concatenate([k, r]), 0.5 * np.concatenate([v, v]), n)
+
+
+def _coo_matvec(r, k, v, x, nrows):
+    return np.bincount(r, weights=v * x[k], minlength=nrows)
+
+
+class SparseQCQPFamily(Family):
+    """Sparse QCQP given by data (lfpsqp_sparse_qcqp, large-n mode); see sparse_qcqp().  Holds the canonical coordinate
+    lists: P, Ac, Ad as (row, col, val); Qc, Qd as (mat, row, col, val), sorted, duplicates summed, symmetric."""
+
+    def __init__(self, n, m, p, P, q, r, Qc, Ac, bc, Qd, Ad, bd):
+        super().__init__(SPARSE_QCQP, "sparse_qcqp", n, m, p)
+        self.P, self.q, self.r, self.Qc, self.Ac, self.bc = P, q, float(r), Qc, Ac, bc
+        self.Qd, self.Ad, self.bd = Qd, Ad, bd
+
+    def large_args(self):
+        """(descriptor pointer for lfpsqp_large_setup, object to keep alive during the call) of the equalities c = 0"""
+        def coo(t, stacked):
+            c = _lib.CCoo()
+            c.nnz = t[-1].size
+            if stacked:
+                c.mat = t[0].ctypes.data
+            c.row, c.col, c.val = (a.ctypes.data for a in t[-3:])
+            return c
+        desc = _lib.CSparseQcqp()
+        desc.P, desc.Qc, desc.Ac = coo(self.P, False), coo(self.Qc, True), coo(self.Ac, False)
+        desc.q, desc.r, desc.bc = self.q.ctypes.data, self.r, self.bc.ctypes.data
+        keep = (desc, self.P, self.Qc, self.Ac, self.q, self.bc)
+        return C.cast(C.pointer(desc), C.c_void_p), keep
+
+    def slack_embedding(self, x0, xl=None, xu=None, dl=None, du=None):
+        """The slack wrapper of src/optimize.jl:13-71 written as data: variables [x ; s] with s0 = d(x0), equalities
+        [c(x) ; d(x) - s] (Ad_k gains -1 in column n + k), bounds [xl ; dl] <= [x ; s] <= [xu ; du] (dl = -Inf, du = 0
+        by default, optimize.jl:83-85).  -> (family with p = 0, x0_aug, xl_aug, xu_aug)"""
+        n, m, p = self.n, self.m, self.p
+        dl = -np.inf * np.ones(p) if dl is None else np.asarray(dl, dtype=np.float64).ravel()
+        du = np.zeros(p) if du is None else np.asarray(du, dtype=np.float64).ravel()
+        if not (len(dl) == len(du) == p):
+            raise _lib.LFPSQPError("Bound vectors dl and du must be of size p")                 # optimize.jl:19-21
+        x0 = np.asarray(x0, dtype=np.float64)
+        xl = -np.inf * np.ones(n) if xl is None else np.asarray(xl, dtype=np.float64)
+        xu = np.inf * np.ones(n) if xu is None else np.asarray(xu, dtype=np.float64)
+        cat = np.concatenate
+        Qc = tuple(cat([a, b]) for a, b in zip(self.Qc, (self.Qd[0] + m,) + self.Qd[1:]))
+        k = np.arange(p, dtype=np.int64)
+        Ad = (self.Ad[0] + m, self.Ad[1], self.Ad[2])
+        Ac = tuple(cat(t) for t in zip(self.Ac, Ad, (k + m, k + n, -np.ones(p))))
+        order = np.lexsort((Ac[1], Ac[0]))
+        Ac = tuple(np.ascontiguousarray(a[order]) for a in Ac)
+        aug = SparseQCQPFamily(n + p, m + p, 0, self.P, cat([self.q, np.zeros(p)]), self.r, Qc, Ac, cat([self.bc, self.bd]),
+                               _EMPTY4, _EMPTY3, np.zeros(0))
+        return aug, cat([x0, self.d_values(x0)]), cat([xl, dl]), cat([xu, du])
+
+    def equalities(self):
+        """the same objective and equalities without d(x)"""
+        return SparseQCQPFamily(self.n, self.m, 0, self.P, self.q, self.r, self.Qc, self.Ac, self.bc, _EMPTY4, _EMPTY3, np.zeros(0))
+
+    def d_values(self, x):
+        """d(x) = 1/2 x'Qd_k x + Ad_k.x - bd_k (numpy)"""
+        x = np.asarray(x, dtype=np.float64)
+        mat, r, k, v = self.Qd
+        return (0.5 * np.bincount(mat, weights=v * x[r] * x[k], minlength=self.p)
+                + _coo_matvec(self.Ad[0], self.Ad[1], self.Ad[2], x, self.p) - self.bd)
+
+    def callbacks(self):
+        """numpy callbacks in the conventions of host.optimize_slack: dict(f, grad, hess_vec, c, jac, chess_vec, d, djac,
+        dhess_vec).  A reference for tests and the route of a problem through host callbacks; the device path does not use them."""
+        n = self.n
+
+        def quad(Qs, Ad, b, cnt):
+            mat, r, k, v = Qs
+
+            def val(out, x):
+                out[:] = 0.5 * np.bincount(mat, weights=v * x[r] * x[k], minlength=cnt) + _coo_matvec(Ad[0], Ad[1], Ad[2], x, cnt) - b
+
+            def jac(Jc, out, x):
+                val(out, x)
+                Jc[:, :] = 0.0
+                np.add.at(Jc, (mat, r), v * x[k])
+                np.add.at(Jc, (Ad[0], Ad[1]), Ad[2])
+
+            def hess(dest, src, x, lam):
+                dest[:] = np.bincount(r, weights=lam[mat] * v * src[k], minlength=n)
+            return val, jac, hess
+
+        P = self.P
+
+        def f(x):
+            return 0.5 * x @ _coo_matvec(P[0], P[1], P[2], x, n) + self.q @ x + self.r
+
+        def grad(g, x):
+            g[:] = _coo_matvec(P[0], P[1], P[2], x, n) + self.q
+
+        def hess_vec(dest, src, x):
+            dest[:] = _coo_matvec(P[0], P[1], P[2], src, n)
+
+        c, jac, chess = quad(self.Qc, self.Ac, self.bc, self.m)
+        d, djac, dhess = quad(self.Qd, self.Ad, self.bd, self.p)
+        return dict(f=f, grad=grad, hess_vec=hess_vec, c=c, jac=jac, chess_vec=chess, d=d, djac=djac, dhess_vec=dhess)
+
+
+_EMPTY3 = (np.zeros(0, np.int64), np.zeros(0, np.int64), np.zeros(0))
+_EMPTY4 = (np.zeros(0, np.int64),) + _EMPTY3
+
+
+def _stack(Ms, name, dims, dn):
+    """a sequence of symmetric n x n matrices -> (mat, row, col, val), sorted by (mat, row, col)"""
+    parts = []
+    for i, M in enumerate(Ms):
+        r, k, v, shape = _coo_of(M, "%s[%d]" % (name, i))
+        if shape[0] != shape[1]:
+            raise _lib.LFPSQPError("sparse_qcqp: %s[%d] must be square, got %s" % (name, i, shape))
+        if dims.setdefault("n", shape[0]) != shape[0]:
+            raise _lib.LFPSQPError("sparse_qcqp: %s[%d] gives n = %d, another array gives %d" % (name, i, shape[0], dims["n"]))
+        r, k, v = _symmetrised(r, k, v, shape[0])
+        parts.append((np.full(r.size, i, np.int64), r, k, v))
+    if dims.setdefault(dn, len(parts)) != len(parts):
+        raise _lib.LFPSQPError("sparse_qcqp: %s has %d matrices, another array gives %s = %d" % (name, len(parts), dn, dims[dn]))
+    return tuple(np.concatenate([p[j] for p in parts]) if parts else _EMPTY4[j] for j in range(4))
+
+
+def sparse_qcqp(P=None, q=None, r=None, Qc=None, Ac=None, bc=None, Qd=None, Ad=None, bd=None):
+    """Sparse quadratically constrained quadratic program (large-n mode, one GPU):
+
+        f(x)   = 1/2 x'P x + q.x + r
+        c_i(x) = 1/2 x'Qc[i] x + Ac[i].x - bc[i] = 0      i < m
+        d_k(x) = 1/2 x'Qd[k] x + Ad[k].x - bd[k] <= 0     k < p   (or dl <= d(x) <= du through optimize_large)
+
+    Matrices are scipy.sparse matrices (anything with .tocoo()) or dense arrays: P (n, n), Ac (m, n), Ad (p, n); Qc and Qd
+    are sequences of m and p (n, n) matrices.  None is all zero.  n, m and p are inferred.  Duplicate entries are summed and
+    square matrices symmetrised as (M + M')/2, which leaves the quadratic forms unchanged.
+
+        fam = families.sparse_qcqp(P=laplacian, Qd=[ball_k ...], bd=radii2 / 2)
+        x, obj, lam, info = optimize_large(fam.f, fam.c, fam.d, dl, du, x0, xl, xu, fam.m, fam.p)
+    """
+    dims = {}
+    Pc = _EMPTY3
+    if P is not None:
+        pr, pk, pv, shape = _coo_of(P, "P")
+        if shape[0] != shape[1]:
+            raise _lib.LFPSQPError("sparse_qcqp: P must be square, got %s" % (shape,))
+        dims["n"] = shape[0]
+        Pc = _symmetrised(pr, pk, pv, shape[0])
+    Qcc = _stack(Qc, "Qc", dims, "m") if Qc is not None else None
+    Qdc = _stack(Qd, "Qd", dims, "p") if Qd is not None else None
+    lin = {}
+    for name, M, dn in (("Ac", Ac, "m"), ("Ad", Ad, "p")):
+        if M is None:
+            continue
+        ar, ak, av, shape = _coo_of(M, name)
+        for d, size in ((dn, shape[0]), ("n", shape[1])):
+            if dims.setdefault(d, size) != size:
+                raise _lib.LFPSQPError("sparse_qcqp: %s gives %s = %d, another array gives %d" % (name, d, size, dims[d]))
+        lin[name] = _summed(ar, ak, av, shape[1])
+    vecs = {}
+    for name, v, dn in (("q", q, "n"), ("bc", bc, "m"), ("bd", bd, "p")):
+        if v is None:
+            continue
+        v = np.asarray(v, dtype=np.float64)
+        if v.ndim != 1:
+            raise _lib.LFPSQPError("sparse_qcqp: %s must be a vector, got shape %s" % (name, v.shape))
+        if dims.setdefault(dn, v.size) != v.size:
+            raise _lib.LFPSQPError("sparse_qcqp: %s gives %s = %d, another array gives %d" % (name, dn, v.size, dims[dn]))
+        vecs[name] = np.ascontiguousarray(v)
+    if "n" not in dims:
+        raise _lib.LFPSQPError("sparse_qcqp: n is unknown (give P, q, Qc, Ac, Qd or Ad)")
+    n, m, p = dims["n"], dims.get("m", 0), dims.get("p", 0)
+    if n < 1:
+        raise _lib.LFPSQPError("sparse_qcqp: n must be at least 1")
+    if m > 0 and Qc is None and Ac is None:
+        raise _lib.LFPSQPError("sparse_qcqp: m = %d equalities need Qc or Ac" % m)
+    if p > 0 and Qd is None and Ad is None:
+        raise _lib.LFPSQPError("sparse_qcqp: p = %d inequalities need Qd or Ad" % p)
+    return SparseQCQPFamily(n, m, p, Pc, vecs.get("q", np.zeros(n)), 0.0 if r is None else float(r),
+                            Qcc if Qcc is not None else _EMPTY4, lin.get("Ac", _EMPTY3), vecs.get("bc", np.zeros(m)),
+                            Qdc if Qdc is not None else _EMPTY4, lin.get("Ad", _EMPTY3), vecs.get("bd", np.zeros(p)))

@@ -4,8 +4,8 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from .api import LFPSQPParams, TerminationCondition, TerminationInfo
-from .families import DIAGQUAD, THOMSON
+from .api import LFPSQPParams, TerminationCondition, TerminationInfo, _family_of, _parse
+from .families import DIAGQUAD, SPARSE_QCQP, THOMSON
 
 
 class LargeProblem:
@@ -17,7 +17,12 @@ class LargeProblem:
         self.m = fam.m
         self.n_loc = fam.n if n_loc is None else n_loc
         self.n = fam.n if n_global is None else n_global
-        if params_dev_ptr is not None:
+        if fam.id == SPARSE_QCQP and fam.p > 0:
+            raise _lib.LFPSQPError("a sparse_qcqp with d(x) is solved by optimize_large, which adds the slack variables")
+        if fam.id == SPARSE_QCQP and params_dev_ptr is None:
+            pp, _keep = fam.large_args()
+            on_dev = 0
+        elif params_dev_ptr is not None:
             pp, on_dev = C.c_void_p(params_dev_ptr), 1
         else:
             pp, on_dev = _lib.ptr(fam.params), 0
@@ -176,3 +181,47 @@ def make_diagquad(n, m, seed=0, cond=1e4, dtype=np.float64):
     w = np.exp(rng.uniform(0.0, np.log(cond), n))
     b = 0.5 * Q @ (x0 * x0) + A @ x0
     return Q, A, b, xt, w, x0
+
+
+def optimize_large(*args, ctx=None, history=None, return_stats=False, noise=None):
+    """optimize(...) for ONE large instance of a large-n device family (diagquad, thomson, sparse_qcqp) on one GPU, with the
+    reference's method shapes (optimize.jl:13, :83, :88, :107, :112) -> (x, obj_values, λ_kkt, term_info).
+
+    With d(x) (sparse_qcqp only) the slack wrapper of optimize.jl:13-71 is built as data (SparseQCQPFamily.slack_embedding):
+    variables [x ; s], equalities [c(x) ; d(x) - s], bounds [xl ; dl] <= [x ; s] <= [xu ; du]; λ then has m + p entries
+    (optimize.jl:67-70).  noise (beta > 0): (T, N_working) rows of the caller's randn! sequence, N_working = 2 (n + p) with
+    bounds, else n."""
+    f, c, d, dl, du, x0, xl, xu, m, p, param = _parse(args)
+    fam = _family_of(f, c, d)
+    if fam.id not in (DIAGQUAD, THOMSON, SPARSE_QCQP):
+        raise _lib.LFPSQPError("optimize_large takes a large-n device family (diagquad, thomson, sparse_qcqp); %r is not one"
+                               % fam)
+    if d is None or p == 0:                                                              # optimize.jl:15-17
+        p = 0
+    if c is None and m != 0:
+        raise _lib.LFPSQPError("c! is nothing but m > 0")
+    x0 = np.ascontiguousarray(x0, dtype=np.float64)
+    if x0.ndim != 1 or (x0.size, m, p) != (fam.n, fam.m, fam.p if p > 0 else 0):
+        raise _lib.LFPSQPError("sizes (n=%d, m=%d, p=%d) do not match the family %r" % (x0.size, m, p, fam))
+    if (xl is None) != (xu is None):
+        raise _lib.LFPSQPError("xl and xu must both be given or both be nothing")
+    if xl is not None and not (len(xl) == len(xu) == x0.size):
+        raise _lib.LFPSQPError("xl, xu, and x0 must all be the same length")             # optimize.jl:144-148
+    param = param or LFPSQPParams()
+    if history is None:   # every iterate's objective, as the reference returns (optimize.jl:250, :426)
+        history = int(param.maxiter) + 1
+    if p > 0:
+        if fam.id != SPARSE_QCQP:
+            raise _lib.LFPSQPError("d(x) in large-n mode needs a sparse_qcqp family (its slack variables are data)")
+        prob_fam, x0w, xl, xu = fam.slack_embedding(x0, xl, xu, dl, du)
+    else:
+        prob_fam, x0w = fam, x0
+        if fam.id == SPARSE_QCQP and fam.p > 0:   # d! not passed (or p = 0): the equalities alone
+            prob_fam = fam.equalities()
+    prob = LargeProblem(prob_fam, ctx=ctx)
+    prob.set_bounds(xl, xu)
+    out = prob.solve(x0w, param, history=history, return_stats=return_stats, noise=noise)
+    if out[3].iter == param.maxiter:
+        import warnings
+        warnings.warn("Maximum # of outer iterations reached")                           # optimize.jl:438-440
+    return (out[0][:fam.n],) + tuple(out[1:])                                            # :67-70 (lambda untruncated)
