@@ -132,6 +132,11 @@ typedef struct {
   lfpsqp_coo Ac;  const double *bc;
 } lfpsqp_sparse_qcqp;
 #define LFPSQP_FAM_SPARSE_QCQP 102   /* fam_params = (const double*)(const lfpsqp_sparse_qcqp*) */
+/* The same problem class and descriptor, with J kept sparse on the device: one value array in CSR and one in CSC order
+ * (nnz(J) doubles each) instead of the dense m x n J (and its weighted copy with bounds).  The passes J v and J'u and the Gram
+ * J W J' run over the pattern (the Gram's work is sum_j nnz(column j)^2); G stays a dense m x m factor.  projcg! and pcg! run
+ * the launch-per-phase loops.  Same validation and the same refusals as LFPSQP_FAM_SPARSE_QCQP. */
+#define LFPSQP_FAM_SPARSE_QCQP_CSR 103
 
 /*
  * Host callbacks of the explicit-derivative core optimize(f, grad!, c!, jac!, hess_lag_vec!, x0, xl, xu, m, param)
@@ -211,7 +216,8 @@ int lfpsqp_solve_batched_dev(lfpsqp_ctx *ctx, int family, int64_t n, int64_t m, 
  * Large-n mode: ONE instance with a dense m x n constraint Jacobian, host-orchestrated whole-GPU kernels
  * (FP64 DMMA Gram + blocked Cholesky replace ksvd!, src/la_helper.jl:8-34 / optimize.jl:291-293; streaming passes over
  * J replace kgemv!, la_helper.jl:36-44).  Families: LFPSQP_FAM_DIAGQUAD, LFPSQP_FAM_THOMSON,
- * LFPSQP_FAM_HOST (params = const lfpsqp_host_callbacks*), LFPSQP_FAM_SPARSE_QCQP (params = const lfpsqp_sparse_qcqp*; one GPU);
+ * LFPSQP_FAM_HOST (params = const lfpsqp_host_callbacks*), LFPSQP_FAM_SPARSE_QCQP and LFPSQP_FAM_SPARSE_QCQP_CSR
+ * (params = const lfpsqp_sparse_qcqp*; one GPU);
  * LFPSQP_FAM_QCQP is LFPSQP_ERR_FAMILY here.  Finite bounds xl <= x <= xu run the reference's 2n-variable
  * embedding (src/inequality_helper.jl): lfpsqp_large_set_bounds after lfpsqp_large_setup, or the xl/xu arguments of
  * lfpsqp_solve_large / lfpsqp_solve_host.  projcg! on diagonal Lagrangian Hessians and pcg! run as persistent cooperative
@@ -276,10 +282,12 @@ int lfpsqp_large_phase_ms(lfpsqp_ctx *ctx, double *out4);
 /* what the last large-n call (factor, project, projcg, projcg_general, retract, pcg, solve) enqueued, recorded on the host
  * (read-only; no kernel changes).  out8 =
  *   [0] mask of dgemm_nt instantiations: 1 <128> lean, 2 <128> with extras (block-structure flags, batches), 4 <64> (N <= 64),
- *       8 <128, SKIP> (zero-slab skipping); bits 0-3 for the Gram's SYRK, bits 4-7 for every other product
+ *       8 <128, SKIP> (zero-slab skipping); bits 0-3 for the Gram's SYRK, bits 4-7 for every other product;
+ *       bit 8: sparse Gram (LFPSQP_FAM_SPARSE_QCQP_CSR)
  *   [1] largest split-K factor of a product with fewer than SMs / 2 tiles (0: none)
  *   [2] largest wave-quantisation split-K factor of a lower SYRK (0: none)
- *   [3] mask of rows_dot kernels: bits 0-2 R = 1, 2, 4 rows per CTA; bits 3-5 the same with zero-slab skipping
+ *   [3] mask of rows_dot kernels: bits 0-2 R = 1, 2, 4 rows per CTA; bits 3-5 the same with zero-slab skipping;
+ *       bit 6 CSR row pass J v, bit 7 CSC column pass J'u (LFPSQP_FAM_SPARSE_QCQP_CSR)
  *   [4] launches of the single-GPU explicit-inverse fused projcg kernel, [5] of the general fused projcg kernel,
  *   [6] launches of the fused pcg! kernel
  *   [7] mask of the forms the Gram solves took: 1 explicit inverse, 2 triangular solves, 4 truncated pseudo-inverse

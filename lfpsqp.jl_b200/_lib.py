@@ -170,9 +170,10 @@ class Context:
     @property
     def large_dispatch(self):
         """What the last large-n call enqueued (lfpsqp_large_last_dispatch): gemm = mask of dgemm_nt instantiations (1 <128>
-        lean, 2 <128> with extras, 4 <64>, 8 <128, SKIP>; bits 0-3 the Gram's SYRK, 4-7 other products), ksplit_grid /
-        ksplit_wave = largest split-K factors (0 none), rows_dot = mask (bits 0-2 R = 1, 2, 4; bits 3-5 with zero-slab
-        skipping), fused_single / fused_general / fused_pcg = fused kernel launches, solve = mask (1 explicit inverse,
+        lean, 2 <128> with extras, 4 <64>, 8 <128, SKIP>; bits 0-3 the Gram's SYRK, 4-7 other products; bit 8 the sparse
+        Gram of a jacobian="csr" sparse_qcqp), ksplit_grid / ksplit_wave = largest split-K factors (0 none), rows_dot = mask
+        (bits 0-2 R = 1, 2, 4; bits 3-5 with zero-slab skipping; bit 6 the CSR row pass J v, bit 7 the CSC column pass J'u),
+        fused_single / fused_general / fused_pcg = fused kernel launches, solve = mask (1 explicit inverse,
         2 triangular, 4 pseudo-inverse)"""
         out = (C.c_int64 * 8)()
         self.check(self.lib.lfpsqp_large_last_dispatch(self.h, out))

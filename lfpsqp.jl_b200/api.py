@@ -6,7 +6,7 @@ from typing import NamedTuple
 import numpy as np
 
 from . import _lib
-from .families import QCQP, SPARSE_QCQP, DeviceCallback
+from .families import QCQP, SPARSE_QCQP, SPARSE_QCQP_CSR, DeviceCallback
 
 # LinesearchOption / DisplayOption (src/LFPSQP.jl:27-35)
 armijo, exact = 0, 1
@@ -115,7 +115,7 @@ def optimize_batched(*args, ctx=None, history=64, return_stats=False, noise=None
     obj_len (B,), lambda (B,m+p), term (B,) structured array[, stats])."""
     f, c, d, dl, du, x0, xl, xu, m, p, param = _parse(args)
     fam = _family_of(f, c, d)
-    if fam.id == SPARSE_QCQP:
+    if fam.id in (SPARSE_QCQP, SPARSE_QCQP_CSR):
         raise _lib.LFPSQPError("sparse_qcqp is a large-n family (one large instance on one GPU): call optimize_large")
     if d is None or p == 0:   # optimize.jl:15-17
         p = 0

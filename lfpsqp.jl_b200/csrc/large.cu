@@ -21,6 +21,7 @@
 #include "large_kernels.cuh"
 #include "large_families.cuh"
 #include "large_ineq.cuh"
+#include "large_spj.cuh"
 #include "large_state.h"
 
 using namespace lfpsqp;
@@ -174,6 +175,54 @@ static void cols_dot(LargeState &S, const double *Jm, int64_t ld, int m, int64_t
     cols_dot_kernel<false><<<grid, 256, S.rows_per_split * sizeof(double), S.stream>>>(Jm, ld, m, ncols, u, S.cpart, S.rows_per_split, S.ctrl, pred);
   S.launches++;
 }
+
+// ---- the passes over the constraint Jacobian: dense S.J (rows_dot / cols_dot) or, for LFPSQP_FAM_SPARSE_QCQP_CSR, its CSR /
+// CSC value arrays (large_spj.cuh).  jcols leaves S.jsplit row splits in S.cpart.
+static int spj_items_grid(const LargeState &S) { return (int)(((int64_t)S.m + S.spj.nslot + 7) / 8); }   // one warp per item
+static void jrows(LargeState &S, const double *v, double *t, int pred) {   // t = J v (first n_loc entries of v)
+  if (!S.csr) { rows_dot(S, S.J, S.ldj, S.m, S.n_loc, v, t, pred); return; }
+  if (S.m <= 0) return;
+  spj_rows_kernel<<<spj_items_grid(S), 256, 0, S.stream>>>(S.spj, S.spq.con_ptr, S.spq.seg_row, v, t, S.spj_part, S.ctrl, pred);
+  S.launches++;
+  if (S.spj.nlong > 0) {
+    spj_combine_kernel<<<(S.spj.nlong + 255) / 256, 256, 0, S.stream>>>(S.spj, S.spj_part, nullptr, t, S.ctrl, pred);
+    S.launches++;
+  }
+  S.disp[LARGE_DISP_ROWS_DOT] |= 64;
+}
+static void jcols(LargeState &S, const double *u, int pred) {   // S.cpart = J'u
+  if (!S.csr) { cols_dot(S, S.J, S.ldj, S.m, S.n_loc, u, pred); return; }
+  if (S.m <= 0) return;
+  spj_cols_kernel<<<S.vgrid, 256, 0, S.stream>>>(S.spj, S.n_loc, u, S.cpart, S.ctrl, pred);
+  S.launches++;
+  S.disp[LARGE_DISP_ROWS_DOT] |= 128;
+}
+// jac! of the CSR form: cval = c(x), with jac also both value arrays of J
+static void spj_cjac(LargeState &S, bool jac, double *cval, const double *x) {
+  const lfpsqp::SpqDev &D = S.spq;
+  if (jac) spj_cjac_kernel<true><<<spj_items_grid(S), 256, 0, S.stream>>>(S.spj, D.con_ptr, D.seg_row, D.seg_a, D.seg_ptr, D.seg_col, D.seg_val, D.bc, x, cval, S.spj_part);
+  else spj_cjac_kernel<false><<<spj_items_grid(S), 256, 0, S.stream>>>(S.spj, D.con_ptr, D.seg_row, D.seg_a, D.seg_ptr, D.seg_col, D.seg_val, D.bc, x, cval, S.spj_part);
+  S.launches++;
+  if (S.spj.nlong > 0) {
+    spj_combine_kernel<<<(S.spj.nlong + 255) / 256, 256, 0, S.stream>>>(S.spj, S.spj_part, D.bc, cval, S.ctrl, 0);
+    S.launches++;
+  }
+}
+// S.G (lower triangle, every entry written) = J J', or J diag(Dy^2) J' with bounds, over the sparsity pattern
+static void spj_gram(LargeState &S) {
+  const int m = S.m;
+  const size_t smem = (size_t)m * sizeof(double);
+  const unsigned grid = (unsigned)(m + S.spj.nslot);
+  const lfpsqp::SpqDev &D = S.spq;
+  if (S.ineq) spj_gram_kernel<true><<<grid, 32, smem, S.stream>>>(S.spj, D.con_ptr, D.seg_row, S.I.Dy, S.G, S.ldm, S.spj_gpart);
+  else spj_gram_kernel<false><<<grid, 32, smem, S.stream>>>(S.spj, D.con_ptr, D.seg_row, nullptr, S.G, S.ldm, S.spj_gpart);
+  S.launches++;
+  if (S.spj.nlong > 0) {
+    spj_gram_combine_kernel<<<dim3((unsigned)((m + 255) / 256), (unsigned)S.spj.nlong), 256, 0, S.stream>>>(S.spj, S.spj_gpart, S.G, S.ldm);
+    S.launches++;
+  }
+  S.disp[LARGE_DISP_GEMM] |= 256;
+}
 // u = (J J')^-1 t through the cached factor: y = L^-1 t ; u = L^-T y
 static void gram_solve(LargeState &S, const double *t, double *u, double *u_copy, int pred) {
   const int m = S.m;
@@ -265,11 +314,12 @@ static void fam_grad(LargeState &S, double *g, const double *x) {
   }
   S.launches++;
 }
-// cval = c(x); with Jout also the Jacobian (jac! writes both, autodiff_generators.jl:40-42)
-static void fam_c_jac(LargeState &S, double *Jout, double *cval, const double *x) {
+// cval = c(x); with jac also the Jacobian (jac! writes both, autodiff_generators.jl:40-42)
+static void fam_c_jac(LargeState &S, bool jac, double *cval, const double *x) {
+  double *Jout = jac ? S.J : nullptr;
   // J is rewritten: its zero-slab map is stale until the next Gram scans it -- except for THOMSON, whose jac! kernel writes the
   // same three structural entries of every row whatever x is (a map entry can then only be conservatively non-zero)
-  if (Jout == S.J && S.family != LFPSQP_FAM_THOMSON) S.jmap_valid = false;
+  if (jac && S.family != LFPSQP_FAM_THOMSON) S.jmap_valid = false;
   const int m = S.m;
   if (S.family == LFPSQP_FAM_HOST) {
     host_x(S, x);
@@ -291,6 +341,7 @@ static void fam_c_jac(LargeState &S, double *Jout, double *cval, const double *x
   } else if (S.family == LFPSQP_FAM_SPARSE_QCQP) {
     if (m <= 0) return;
     const lfpsqp::SpqDev &D = S.spq;
+    if (S.csr) { spj_cjac(S, jac, cval, x); return; }
     if (Jout) spq_cjac_kernel<true><<<m, 256, 0, S.stream>>>(D.con_ptr, D.seg_row, D.seg_a, D.seg_ptr, D.seg_col, D.seg_val, D.bc, x, Jout, S.ldj, cval);
     else spq_cjac_kernel<false><<<m, 256, 0, S.stream>>>(D.con_ptr, D.seg_row, D.seg_a, D.seg_ptr, D.seg_col, D.seg_val, D.bc, x, nullptr, S.ldj, cval);
     S.launches++;
@@ -416,6 +467,7 @@ static void gram_syrk(LargeState &S, const double *Jg) {
 }
 static void gram_only(LargeState &S) {   // S.G (lower tiles) = J W J', all-reduced
   const int m = S.m;
+  if (S.csr) { spj_gram(S); return; }
   const double *Jg = S.ineq ? S.Jw : S.J;    // Jw = J diag(Dy) was formed by the factorize() call that precedes
   gram_syrk(S, Jg);
   if (S.world > 1) comm_allreduce(S, S.G, (size_t)m * S.ldm);
@@ -448,14 +500,15 @@ static int factorize(lfpsqp_ctx *c, LargeState &S) {
   const int m = S.m; const int64_t ldm = S.ldm;
   const double *Jg = S.J;
   S.invflag_valid = false;
-  if (S.ineq) {
+  if (S.ineq && !S.csr) {
     dim3 sg((unsigned)std::min<int64_t>(std::max<int64_t>(((S.n_loc >> 1) + 255) / 256, 1), 32), (unsigned)std::min(m, 65535));
     ineq_scale_cols_kernel<<<sg, 256, 0, S.stream>>>(S.J, S.ldj, m, S.n_loc, S.I.Dy, S.Jw);
     S.launches++;
     Jg = S.Jw;
   }
   cudaEventRecord(S.ev_g0, S.stream);
-  gram_syrk(S, Jg);   // SYRK, lower tiles
+  if (S.csr) spj_gram(S);   // weighted by Dy^2 with bounds
+  else gram_syrk(S, Jg);    // SYRK, lower tiles
   cudaEventRecord(S.ev_g1, S.stream);
   if (S.world > 1) comm_allreduce(S, S.G, (size_t)m * ldm);
   if (S.prefer_pinv) return factorize_pinv(c, S, false);   // this problem lost rank before: go straight to the eigen-decomposition
@@ -591,14 +644,14 @@ static void proj_passes(LargeState &S, const double *v, double *lam_out, int pre
     operand = S.pb;
   }
   if (S.m <= 0) return;
-  rows_dot(S, S.J, S.ldj, S.m, S.n_loc, operand, S.tm, pred);
+  jrows(S, operand, S.tm, pred);
   if (S.world > 1) comm_allreduce(S, S.tm, S.m);
   gram_solve(S, S.tm, S.tu, lam_out, pred);
-  cols_dot(S, S.J, S.ldj, S.m, S.n_loc, S.tu, pred);
+  jcols(S, S.tu, pred);
 }
 static void project(LargeState &S, double *v, double *lam_out, int pred, int want_norms, int want_mult = 0) {
   proj_passes(S, v, lam_out, pred);
-  const double *cp = S.cpart; int ns = S.m > 0 ? S.nsplit : 0; int64_t n = S.n_loc;
+  const double *cp = S.cpart; int ns = S.m > 0 ? S.jsplit : 0; int64_t n = S.n_loc;
   if (!S.ineq) {
     vec(S, n, [=] __device__(int64_t j, double *acc) {
       double s = 0.0;
@@ -627,14 +680,14 @@ static void project(LargeState &S, double *v, double *lam_out, int pred, int wan
 static int projcg(lfpsqp_ctx *c, LargeState &S, double tol, int64_t maxit, int chunk, const double *cvec = nullptr,
                   double *lam_out = nullptr) {
   const int64_t n = S.nv;   // working length: n_loc, or 2 n_loc with bounds
-  const int ns = S.m > 0 ? S.nsplit : 0;
+  const int ns = S.m > 0 ? S.jsplit : 0;
   double *xs = S.nd, *r = S.w0, *dc = S.w1, *Ad = S.w2, *rp = S.w3, *gp = S.w4;
   const double *b = S.d;
   if (S.family == LFPSQP_FAM_HOST) chunk = 1;   // the Hessian callback runs on the host: one status check per iteration
   if (cvec && S.m > 0 && !S.ineq) {
     const int m = S.m;
     tri_gemv_kernel<<<(m + 7) / 8, 256, m * sizeof(double), S.stream>>>(S.XT, S.ldm, m, cvec, S.tu, 1, nullptr, S.ctrl, 0, S.invflag_valid ? S.invflag : nullptr, S.nz_rows);   // L^-T c
-    cols_dot(S, S.J, S.ldj, m, S.n_loc, S.tu, 0);
+    jcols(S, S.tu, 0);
     const double *cp = S.cpart; const int64_t nl = S.n_loc;
     vec(S, n, [=] __device__(int64_t j, double *) { double s = 0.0; for (int k = 0; k < ns; k++) s += cp[(int64_t)k * nl + j]; xs[j] = s; });
     hess_apply(S, r, xs, 0);
@@ -697,7 +750,7 @@ static int projcg(lfpsqp_ctx *c, LargeState &S, double tol, int64_t maxit, int c
       const int st_keep = S.hctrl->status;
       hess_apply(S, Ad, xs, 0);
       vec(S, n, [=] __device__(int64_t i, double *) { Ad[i] = b[i] - Ad[i]; });
-      rows_dot(S, S.J, S.ldj, S.m, S.n_loc, Ad, S.tm, 0);
+      jrows(S, Ad, S.tm, 0);
       if (S.world > 1) comm_allreduce(S, S.tm, S.m);
       tri_gemv_kernel<<<(S.m + 7) / 8, 256, S.m * sizeof(double), S.stream>>>(S.Linv, S.ldm, S.m, S.tm, lam_out, 0, nullptr, S.ctrl, 0, S.invflag_valid ? S.invflag : nullptr, S.nz_rows);
       S.launches += 2;
@@ -723,11 +776,11 @@ static int run_pcg(lfpsqp_ctx *c, LargeState &S, double mu, double tol, int64_t 
       const int par = (int)(k & 1);
       if (S.world > 1) comm_allreduce_loop_slot(S, 5 + par, S.np_loop_raw);
       pcg_a_kernel<<<S.vgrid, 256, 0, S.stream>>>(n, pv, r, S.lp, S.np_loop, par, k == 0, S.ctrl);
-      rows_dot(S, S.J, S.ldj, m, nx, pv, S.tm, 2);     // J p_x (bigA' p = [S (Dx p_x + Dy p_y) ; J p_x] with bounds)
+      jrows(S, pv, S.tm, 2);                          // J p_x (bigA' p = [S (Dx p_x + Dy p_y) ; J p_x] with bounds)
       if (S.world > 1) comm_allreduce(S, S.tm, m);
-      cols_dot(S, S.J, S.ldj, m, nx, S.tm, 2);
-      if (S.ineq) ineq_pcg_z_kernel<<<S.vgrid, 256, 0, S.stream>>>(S.I, z, pv, S.cpart, S.nsplit, S.lp, S.ctrl);
-      else pcg_z_kernel<<<S.vgrid, 256, 0, S.stream>>>(n, z, pv, S.cpart, S.nsplit, S.lp, S.ctrl);
+      jcols(S, S.tm, 2);
+      if (S.ineq) ineq_pcg_z_kernel<<<S.vgrid, 256, 0, S.stream>>>(S.I, z, pv, S.cpart, S.jsplit, S.lp, S.ctrl);
+      else pcg_z_kernel<<<S.vgrid, 256, 0, S.stream>>>(n, z, pv, S.cpart, S.jsplit, S.lp, S.ctrl);
       if (S.world > 1) comm_allreduce_loop_slot(S, 4, S.np_loop_raw);
       pcg_x_kernel<<<S.vgrid, 256, 0, S.stream>>>(n, dx, r, pv, z, S.lp, S.np_loop, par, S.ctrl);
       S.launches += 3;
@@ -752,7 +805,7 @@ static int retract_pp(lfpsqp_ctx *c, LargeState &S, int *flag_out, int *it1, int
   double mu = prm.mu0;
   int i = 0, pcg_total = 0;
   while (i < prm.maxiter_retract) {
-    fam_c_jac(S, S.J, cval, xnew);                                                       // :340
+    fam_c_jac(S, true, cval, xnew);                                                       // :340
     // curtol = |c|_inf (slot 3 max), c.c (slot 0) ; with bounds also |h|_inf (slot 4), h.h (slot 1) and the stale tail
     if (!ineq) {
       vec(S, m, [=] __device__(int64_t a, double *acc) { double v = cval[a]; acc[0] += v * v; acc[3] = nanmax(acc[3], fabs(v)); }, 0, 1, 1);
@@ -784,9 +837,9 @@ static int retract_pp(lfpsqp_ctx *c, LargeState &S, int *flag_out, int *it1, int
     if (curtol < prm.eps_c) break;                                                       // :359-361
     const double prev_obj = (hh + cc) + mu * gg;                                         // :366
     // g = J' c + mu g, or bigA [h ; c] + mu g (:369) ; dx = 0 ; r = g ; r.r partials -> loop slot 5 (rho_0)
-    cols_dot(S, S.J, S.ldj, m, n, cval, 0);
-    if (ineq) ineq_pp_rhs_kernel<<<S.vgrid, 256, 0, S.stream>>>(I, gv, dx, r, pv, S.cpart, S.nsplit, mu, cvh, S.lp);
-    else pp_rhs_kernel<<<S.vgrid, 256, 0, S.stream>>>(n, gv, dx, r, pv, S.cpart, S.nsplit, mu, S.lp);
+    jcols(S, cval, 0);
+    if (ineq) ineq_pp_rhs_kernel<<<S.vgrid, 256, 0, S.stream>>>(I, gv, dx, r, pv, S.cpart, S.jsplit, mu, cvh, S.lp);
+    else pp_rhs_kernel<<<S.vgrid, 256, 0, S.stream>>>(n, gv, dx, r, pv, S.cpart, S.jsplit, mu, S.lp);
     S.launches++;
     if (run_pcg(c, S, mu, prm.eps_c, prm.maxiter_pcg)) return -1;                       // :375
     int pcg_i = S.hctrl->pcg_iter;
@@ -799,7 +852,7 @@ static int retract_pp(lfpsqp_ctx *c, LargeState &S, int *flag_out, int *it1, int
       xk -= dx[q]; xnew[q] = xk;
       double t = xk - xtil[q]; gv[q] = t; acc[1] += t * t;
     }, 0, 2);
-    fam_c_jac(S, nullptr, cval, xnew);                                                    // :392
+    fam_c_jac(S, false, cval, xnew);                                                    // :392
     vec(S, m, [=] __device__(int64_t a, double *acc) { double v = cval[a]; if (ineq) cvc[a] = v; acc[0] += v * v; }, 2, 1);   // slot 2 only
     if (ineq) {                                                                           // h -> cvalaug[1:n] (:395-397), slot 4
       vec(S, n, [=] __device__(int64_t j, double *acc) {
@@ -852,7 +905,7 @@ static int retract_nr(lfpsqp_ctx *c, LargeState &S, int *flag_out, int *it1) {
   const bool ineq = S.ineq; const lfpsqp::IneqDev I = S.I; const double *xb = S.x;
   cudaMemcpyAsync(xnew, S.xtil, S.nv * sizeof(double), cudaMemcpyDeviceToDevice, S.stream);
   if (ineq) y_retract(S, xnew, xb);                                                      // :118-123
-  fam_c_jac(S, nullptr, cval, xnew);
+  fam_c_jac(S, false, cval, xnew);
   cudaMemcpyAsync(D, S.Linv, (size_t)m * ldm * sizeof(double), cudaMemcpyDeviceToDevice, S.stream);   // D0 = L^-1
   int i = 0;
   while (i < S.prm.maxiter_retract) {
@@ -864,8 +917,8 @@ static int retract_nr(lfpsqp_ctx *c, LargeState &S, int *flag_out, int *it1) {
     vec(S, m, [=] __device__(int64_t a, double *) { t1[a] = -t1[a]; });                   // :140 delta = -D c
     // xnew += Q delta, Q = J' L^-T (:141)
     tri_gemv_kernel<<<(m + 7) / 8, 256, m * sizeof(double), S.stream>>>(S.XT, ldm, m, t1, S.tu, 1, nullptr, S.ctrl, 0, S.invflag_valid ? S.invflag : nullptr, S.nz_rows);
-    cols_dot(S, S.J, S.ldj, m, n, S.tu, 0);
-    { const double *cp = S.cpart; int ns = S.nsplit;
+    jcols(S, S.tu, 0);
+    { const double *cp = S.cpart; int ns = S.jsplit;
       // with bounds the basis is Q = PJct L^-T: x += Dy^2 w, y -= Dx Dy w, then y_retract! (:141-143)
       vec(S, n, [=] __device__(int64_t j, double *) {
         double s = 0.0; for (int k = 0; k < ns; k++) s += cp[(int64_t)k * n + j];
@@ -875,7 +928,7 @@ static int retract_nr(lfpsqp_ctx *c, LargeState &S, int *flag_out, int *it1) {
         ineq_yretract(I.q[j], I.r[j], I.s[j], I.t[j], xb[j], xb[n + j], xn, yn);
         xnew[j] = xn; xnew[n + j] = yn;
       }); }
-    fam_c_jac(S, nullptr, t2, xnew);                                                     // :144-149
+    fam_c_jac(S, false, t2, xnew);                                                     // :144-149
     vec(S, m, [=] __device__(int64_t a, double *) { dcv[a] = t2[a] - cval[a]; cval[a] = t2[a]; });
     // Good Broyden (:156-160): t2 = D' delta ; t1 = delta - D dc ; D += t1 t2' / (t2.dc)
     {
@@ -1015,7 +1068,7 @@ static int solve(lfpsqp_ctx *c, LargeState &S, const double *x0_host, double *x_
   int64_t it = 0, nobj = 0;
   double f_diff = INFINITY, step_diff = INFINITY, kkt_diff = INFINITY, prev_grad_norm = 0.0;
   fam_f(S, x); finalize(S, 1u, 0);
-  if (m > 0) fam_c_jac(S, nullptr, S.cval, x);                                          // :252
+  if (m > 0) fam_c_jac(S, false, S.cval, x);                                          // :252
   if (read_ctrl(c, S)) return LFPSQP_ERR_CUDA;
   if (S.cb_err) return LFPSQP_ERR_CALLBACK;
   double fval = S.hctrl->s[0];
@@ -1043,7 +1096,7 @@ static int solve(lfpsqp_ctx *c, LargeState &S, const double *x0_host, double *x_
     if (m > 0 || ineq) {
       const double tf0 = now_ms();
       if (m > 0) {
-        fam_c_jac(S, S.J, S.cval, x);                                                   // :283
+        fam_c_jac(S, true, S.cval, x);                                                   // :283
         if (factorize(c, S)) return LFPSQP_ERR_CUDA;
         cudaMemcpyAsync(xtil, d, nv * sizeof(double), cudaMemcpyDeviceToDevice, S.stream);   // d before the projection (rank-loss redo)
       }
@@ -1184,6 +1237,8 @@ extern "C" int lfpsqp_large_setup(lfpsqp_ctx *c, int family, int64_t n_global, i
                                   const double *params, int params_on_device) {
   if (!c) return LFPSQP_ERR_ARG;
   cudaSetDevice(c->device);
+  const bool csr = family == LFPSQP_FAM_SPARSE_QCQP_CSR;   // the same family with J kept sparse: S.family = SPARSE_QCQP, S.csr
+  if (csr) family = LFPSQP_FAM_SPARSE_QCQP;
   if (family != LFPSQP_FAM_DIAGQUAD && family != LFPSQP_FAM_THOMSON && family != LFPSQP_FAM_HOST && family != LFPSQP_FAM_SPARSE_QCQP)
     return c->fail(LFPSQP_ERR_FAMILY, "large-n mode supports the DIAGQUAD, THOMSON, HOST (callback) and SPARSE_QCQP families");
   if (n_global < 1 || m < 0 || n_loc < 1 || col0 < 0 || col0 + n_loc > n_global || m > n_global)
@@ -1211,7 +1266,7 @@ extern "C" int lfpsqp_large_setup(lfpsqp_ctx *c, int family, int64_t n_global, i
   LargeState *Sp = new LargeState(); LargeState &S = *Sp;
   c->large = Sp;
   S.comm = &c->comm; S.world = c->comm.world > 1 ? c->comm.world : 1; S.rank = c->comm.rank;
-  S.family = family; S.n = n_global; S.n_loc = n_loc; S.nv = n_loc; S.col0 = col0; S.m = (int)m; S.stream = c->stream;
+  S.family = family; S.csr = csr; S.n = n_global; S.n_loc = n_loc; S.nv = n_loc; S.col0 = col0; S.m = (int)m; S.stream = c->stream;
   S.sm_count = c->sm_count; S.ldj = up2(n_loc); S.ldm = up2(std::max<int64_t>(m, 1));
   S.vgrid = (int)std::min<int64_t>(std::max<int64_t>((n_loc + 255) / 256, 1), std::min<int64_t>(MAXP, 4 * (int64_t)c->sm_count));
   S.np_loop_raw = S.vgrid; S.np_loop = (S.world > 1) ? 1 : S.vgrid;
@@ -1224,14 +1279,15 @@ extern "C" int lfpsqp_large_setup(lfpsqp_ctx *c, int family, int64_t n_global, i
     S.rows_per_split = m > 0 ? (int)((m + S.nsplit - 1) / S.nsplit) : 1;
     S.nsplit = m > 0 ? (int)((m + S.rows_per_split - 1) / S.rows_per_split) : 1;
   }
+  S.jsplit = csr ? 1 : S.nsplit;
   S.cg_chunk = 2; S.pcg_chunk = 2;
   const size_t nl = (size_t)n_loc, mm = (size_t)std::max<int64_t>(m, 1);
   bool ok = true;
-  ok &= dalloc(S, &S.J, mm * S.ldj);
+  if (!csr) ok &= dalloc(S, &S.J, mm * S.ldj);
   ok &= dalloc(S, &S.G, mm * S.ldm); ok &= dalloc(S, &S.XT, mm * S.ldm); ok &= dalloc(S, &S.Linv, mm * S.ldm);
   ok &= dalloc(S, &S.Dblk, ((mm + 63) / 64) * 64 * 64); ok &= dalloc(S, &S.tmp64, mm * 64); ok &= dalloc(S, &S.thresh, 8);
   S.nz_rows = (int)((mm + 63) / 64); S.nz_ld = (int64_t)((S.ldj + GM_BK - 1) / GM_BK + 64) / 64 * 64; S.gram_mode = 0; S.nz_pending = false; S.g_blockdiag = 0; S.gdep_pending = false;
-  ok &= dalloc(S, &S.nzmap, (size_t)S.nz_rows * S.nz_ld);
+  if (!csr) ok &= dalloc(S, &S.nzmap, (size_t)S.nz_rows * S.nz_ld);
   ok &= dalloc(S, &S.blkflag, (size_t)S.nz_rows * S.nz_rows + S.nz_rows + 1);   // + done[nblk]
   ok &= dalloc(S, &S.invflag, (size_t)S.nz_rows * S.nz_rows + 1);
   { int dev = 0, v = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&v, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev); if (v > 2048) S.max_dyn_smem = v - 1024; }
@@ -1262,7 +1318,7 @@ extern "C" int lfpsqp_large_setup(lfpsqp_ctx *c, int family, int64_t n_global, i
   cudaEventCreate(&S.ev_g0); cudaEventCreate(&S.ev_g1);
   cudaMemsetAsync(S.lp, 0, (size_t)NSLOT * MAXP * 8, S.stream); cudaMemsetAsync(S.gpart, 0, (size_t)NSLOT * MAXP * 8, S.stream);
   cudaMemsetAsync(S.ctrl, 0, sizeof(LargeCtrl), S.stream);
-  cudaMemsetAsync(S.J, 0, mm * S.ldj * sizeof(double), S.stream);   // the pad column of an odd n_loc must stay zero (16-byte K chunks)
+  if (S.J) cudaMemsetAsync(S.J, 0, mm * S.ldj * sizeof(double), S.stream);   // the pad column of an odd n_loc must stay zero (16-byte K chunks)
   // parameters
   if (family == LFPSQP_FAM_DIAGQUAD) {
     const size_t cnt = 2 * mm * nl * (m > 0 ? 1 : 0) + (size_t)m + 2 * nl;
@@ -1278,7 +1334,7 @@ extern "C" int lfpsqp_large_setup(lfpsqp_ctx *c, int family, int64_t n_global, i
     S.p_Q = blob; S.p_A = blob + (size_t)m * nl; S.p_b = S.p_A + (size_t)m * nl; S.p_xt = S.p_b + m; S.p_w = S.p_xt + nl;
     if ((((uintptr_t)S.p_A) & 15) || (((uintptr_t)S.p_Q) & 15)) { lfpsqp_large_release(c); return c->fail(LFPSQP_ERR_ARG, "parameter blob must be 16-byte aligned"); }
   }
-  if (family == LFPSQP_FAM_SPARSE_QCQP && !spq_upload(S, spq_host)) {
+  if (family == LFPSQP_FAM_SPARSE_QCQP && (!spq_upload(S, spq_host) || (csr && !spj_upload(S, spq_host)))) {
     lfpsqp_large_release(c);
     return c->fail(LFPSQP_ERR_NOMEM, "SPARSE_QCQP: device allocation or upload of the structures failed");
   }
@@ -1293,10 +1349,15 @@ extern "C" int lfpsqp_large_setup(lfpsqp_ctx *c, int family, int64_t n_global, i
   CK(cudaFuncSetAttribute(tri_gemv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max<size_t>(mm * sizeof(double), 1024)));
   CK(cudaFuncSetAttribute(cols_dot_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max<size_t>(mm * sizeof(double), 1024)));
   CK(cudaFuncSetAttribute(cols_dot_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max<size_t>(mm * sizeof(double), 1024)));
+  if (csr) {   // the shared m-vector of the sparse Gram (128 KB at m = 16384)
+    CK(cudaFuncSetAttribute(spj_gram_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max<size_t>(mm * sizeof(double), 1024)));
+    CK(cudaFuncSetAttribute(spj_gram_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max<size_t>(mm * sizeof(double), 1024)));
+  }
   CK(cudaStreamSynchronize(S.stream));
   {
     const char *env = getenv("LFPSQP_FUSED_PROJCG");   // "0" selects the multi-kernel projcg loop (A/B measurements, tests)
-    if (m > 0 && !(env && env[0] == '0')) fused_projcg_init(S, c->device);   // pcg! is fused for every family, projcg for diagonal Hessians
+    // pcg! is fused for every family with a dense J, projcg for diagonal Hessians; the CSR form runs the launch-per-phase loops
+    if (m > 0 && !csr && !(env && env[0] == '0')) fused_projcg_init(S, c->device);
   }
   if (S.world > 1) {
     // every rank must take the same path (a rank in the launch-per-phase loop would deadlock against peers inside the fused
@@ -1385,7 +1446,7 @@ extern "C" int lfpsqp_large_set_bounds(lfpsqp_ctx *c, const double *xl_loc, cons
     bool ok = true;
     double **nvv[] = {&S.bq, &S.br, &S.bs, &S.bt, &S.I.Dx, &S.I.Dy, &S.I.S, &S.I.lamy, &S.cvh, &S.pb};
     for (double **v : nvv) ok &= dalloc(S, v, (size_t)nl + 2);
-    if (S.m > 0) { ok &= dalloc(S, &S.Jw, (size_t)S.m * S.ldj); if (ok) cudaMemsetAsync(S.Jw, 0, (size_t)S.m * S.ldj * 8, S.stream); }
+    if (S.m > 0 && !S.csr) { ok &= dalloc(S, &S.Jw, (size_t)S.m * S.ldj); if (ok) cudaMemsetAsync(S.Jw, 0, (size_t)S.m * S.ldj * 8, S.stream); }
     if (!ok) return c->fail(LFPSQP_ERR_NOMEM, "bound-embedding workspace allocation failed");
   }
   // bnd layout (abi.cu build_bounds): [kind | q | r | s | t], each nl doubles
@@ -1436,11 +1497,14 @@ extern "C" int lfpsqp_large_factor(lfpsqp_ctx *c, const double *x_loc, double *G
   const int m = S.m; const size_t ldm = S.ldm;
   CK(cudaMemcpyAsync(S.x, x_loc, S.n_loc * 8, cudaMemcpyHostToDevice, S.stream));
   memset(S.hctrl, 0, sizeof(LargeCtrl)); write_ctrl_fields(S);
-  fam_c_jac(S, S.J, S.cval, S.x);
+  fam_c_jac(S, true, S.cval, S.x);
   if (G_out) {  // G before it is overwritten by L
-    S.disp_syrk = true;
-    gemm_nt(S, m, m, (int)S.n_loc, S.J, S.ldj, S.J, S.ldj, S.G, ldm, GEMM_ASSIGN, 1);
-    S.disp_syrk = false;
+    if (S.csr) spj_gram(S);
+    else {
+      S.disp_syrk = true;
+      gemm_nt(S, m, m, (int)S.n_loc, S.J, S.ldj, S.J, S.ldj, S.G, ldm, GEMM_ASSIGN, 1);
+      S.disp_syrk = false;
+    }
     if (S.world > 1) comm_allreduce(S, S.G, (size_t)m * ldm);
     CK(cudaMemcpy2DAsync(G_out, m * 8, S.G, ldm * 8, m * 8, m, cudaMemcpyDeviceToHost, S.stream));
   }
@@ -1555,7 +1619,7 @@ extern "C" int lfpsqp_large_retract(lfpsqp_ctx *c, int method, const double *x_b
   CK(cudaMemcpyAsync(S.xtil, xtilde_loc, n * 8, cudaMemcpyHostToDevice, S.stream));
   memset(S.hctrl, 0, sizeof(LargeCtrl)); write_ctrl_fields(S);
   S.reset_counters();
-  fam_c_jac(S, S.J, S.cval, S.x);
+  fam_c_jac(S, true, S.cval, S.x);
   if (factorize(c, S)) return LFPSQP_ERR_CUDA;
   int fl = 0, i1 = 0, i2 = 0;
   if (method == 0) { if (retract_nr(c, S, &fl, &i1)) return LFPSQP_ERR_CUDA; }
@@ -1582,7 +1646,7 @@ extern "C" int lfpsqp_large_pcg(lfpsqp_ctx *c, const double *x_point_loc, double
   CK(cudaMemcpyAsync(r, b_loc, n * 8, cudaMemcpyHostToDevice, S.stream));
   memset(S.hctrl, 0, sizeof(LargeCtrl)); write_ctrl_fields(S);
   S.reset_counters();
-  fam_c_jac(S, S.J, S.cval, S.x);
+  fam_c_jac(S, true, S.cval, S.x);
   pcg_start_kernel<<<S.vgrid, 256, 0, S.stream>>>(n, r, dx, pv, lp);
   cudaEventRecord(c->ev0, S.stream);
   if (run_pcg(c, S, mu, tol, maxiter)) return LFPSQP_ERR_CUDA;

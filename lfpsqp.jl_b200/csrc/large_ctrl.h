@@ -59,4 +59,17 @@ struct SpqDev {
   const double *seg_a = nullptr, *seg_val = nullptr, *bc = nullptr;
 };
 
+// LFPSQP_FAM_SPARSE_QCQP_CSR (kernels in large_spj.cuh, built by large_spq.cu): J kept sparse.  CSR = (SpqDev::con_ptr,
+// SpqDev::seg_row, jr); CSC = (cptr, crow, jc), csc_of[s] = CSC slot of segment s.  A row with more than SPJ_CHUNK entries is
+// "long": it is cut into chunks of SPJ_CHUNK segments (slots), numbered in row order; row_slot[i] = first slot of row i
+// (row_slot[i + 1] == row_slot[i] for a short row), slot_row / slot_beg / slot_end describe slot s, long_row lists the long rows.
+constexpr int SPJ_CHUNK = 4096;
+struct SpjDev {
+  int m = 0, nslot = 0, nlong = 0;
+  int64_t nnz = 0;
+  const int *cptr = nullptr, *crow = nullptr, *csc_of = nullptr;
+  const int *row_slot = nullptr, *slot_row = nullptr, *slot_beg = nullptr, *slot_end = nullptr, *long_row = nullptr;
+  double *jr = nullptr, *jc = nullptr;
+};
+
 }  // namespace lfpsqp

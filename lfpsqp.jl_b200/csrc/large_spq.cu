@@ -160,3 +160,46 @@ bool spq_upload(LargeState &S, const SpqHost &H) {
   // the host vectors are the caller's: the copies must have landed before it returns
   return ok && cudaStreamSynchronize(S.stream) == cudaSuccess;
 }
+
+bool spj_upload(LargeState &S, const SpqHost &H) {
+  const int m = H.m;
+  const int64_t n = H.n, nnz = (int64_t)H.seg_row.size();   // < 2^31: spq_build refuses more segments
+  // CSC by a counting sort over the CSR order: the rows of every column come out increasing
+  std::vector<int> cptr((size_t)n + 1, 0), crow((size_t)nnz), csc_of((size_t)nnz);
+  for (int64_t s = 0; s < nnz; s++) cptr[(size_t)H.seg_row[(size_t)s] + 1]++;
+  for (int64_t j = 0; j < n; j++) cptr[(size_t)j + 1] += cptr[(size_t)j];
+  {
+    std::vector<int> next(cptr.begin(), cptr.end() - 1);
+    for (int i = 0; i < m; i++)
+      for (int s = H.con_ptr[(size_t)i]; s < H.con_ptr[(size_t)i + 1]; s++) {
+        const int p = next[(size_t)H.seg_row[(size_t)s]]++;
+        crow[(size_t)p] = i; csc_of[(size_t)s] = p;
+      }
+  }
+  // chunks of the rows longer than SPJ_CHUNK segments: a function of the pattern alone
+  std::vector<int> row_slot((size_t)m + 1, 0), slot_row, slot_beg, slot_end, long_row;
+  for (int i = 0; i < m; i++) {
+    const int b = H.con_ptr[(size_t)i], e = H.con_ptr[(size_t)i + 1];
+    if (e - b > lfpsqp::SPJ_CHUNK) {
+      long_row.push_back(i);
+      for (int s = b; s < e; s += lfpsqp::SPJ_CHUNK) {
+        slot_row.push_back(i); slot_beg.push_back(s); slot_end.push_back((int)std::min<int64_t>((int64_t)s + lfpsqp::SPJ_CHUNK, e));
+      }
+    }
+    row_slot[(size_t)i + 1] = (int)slot_row.size();
+  }
+  lfpsqp::SpjDev &P = S.spj;
+  P.m = m; P.nnz = nnz; P.nslot = (int)slot_row.size(); P.nlong = (int)long_row.size();
+  bool ok = upload(S, &P.cptr, cptr) && upload(S, &P.crow, crow) && upload(S, &P.csc_of, csc_of) && upload(S, &P.row_slot, row_slot) &&
+            upload(S, &P.slot_row, slot_row) && upload(S, &P.slot_beg, slot_beg) && upload(S, &P.slot_end, slot_end) &&
+            upload(S, &P.long_row, long_row);
+  double **bufs[] = {&P.jr, &P.jc, &S.spj_part, &S.spj_gpart};
+  const size_t cnt[] = {(size_t)nnz, (size_t)nnz, (size_t)P.nslot, (size_t)P.nslot * (size_t)m};
+  for (int k = 0; ok && k < 4; k++) {
+    void *p = nullptr;
+    ok = cudaMalloc(&p, std::max<size_t>(cnt[k], 1) * sizeof(double)) == cudaSuccess;
+    if (ok) { S.owned.push_back(p); *bufs[k] = (double *)p; }
+  }
+  if (!ok) { cudaGetLastError(); return false; }
+  return cudaStreamSynchronize(S.stream) == cudaSuccess;
+}

@@ -18,6 +18,12 @@ struct LargeState {
   double *cvh = nullptr, *cvc = nullptr;   // cvalaug = [h ; c] of ProjPenalty (retractions.jl:29), persistent across calls
   double *pb = nullptr, *Jw = nullptr;     // x-half operand of PJct' v ; J diag(Dy) for the weighted Gram
   lfpsqp::SpqDev spq;                      // LFPSQP_FAM_SPARSE_QCQP: uploaded structures (large_spq.cu)
+  // LFPSQP_FAM_SPARSE_QCQP_CSR (family stays LFPSQP_FAM_SPARSE_QCQP, csr set): J in CSR / CSC form instead of S.J
+  // (large_spj.cuh); spj_part: chunk partials of the row pass and of jac!'s c, spj_gpart: chunk partial rows of the Gram
+  bool csr = false;
+  lfpsqp::SpjDev spj;
+  double *spj_part = nullptr, *spj_gpart = nullptr;
+  int jsplit = 1;                          // row splits a J column pass leaves in cpart: 1 (CSC pass) or nsplit (cols_dot)
   // host-callback family (LFPSQP_FAM_HOST): the callbacks, pinned staging buffers, device staging of Jc (n x m)
   lfpsqp_host_callbacks cb = {};
   double *hx = nullptr, *hv = nullptr, *hw = nullptr, *hlam = nullptr, *hc = nullptr, *hJ = nullptr, *Jstage = nullptr;
@@ -128,6 +134,9 @@ struct SpqHost {
 };
 int spq_build(lfpsqp_ctx *c, const lfpsqp_sparse_qcqp *D, int64_t n, int64_t m, SpqHost &H);
 bool spq_upload(LargeState &S, const SpqHost &H);
+// LFPSQP_FAM_SPARSE_QCQP_CSR: the CSC pattern of J and the chunk partition of long rows (host, fixed order), the two value
+// arrays and the chunk partial buffers -> S.spj, S.spj_part, S.spj_gpart (false: allocation or copy failed)
+bool spj_upload(LargeState &S, const SpqHost &H);
 
 // large_eig.cu: eigen-decomposition of the Gram (one-sided Jacobi) -> scaled eigenvectors for the pseudo-inverse
 int large_eig_pinv_factors(LargeState &S, double *G, double *Vt, double *lam, int lower_only, int *sweeps_dev, unsigned long long *conv_dev,

@@ -16,6 +16,8 @@ from . import _lib
 ROSENBROCK, README_EQ, README_INEQ, THOMSON, DIAGQUAD, SIN, BOXQUAD = range(7)
 QCQP = 101
 SPARSE_QCQP = 102
+SPARSE_QCQP_CSR = 103   # the same problem with its Jacobian kept sparse on the device (jacobian="csr")
+_JACOBIAN_IDS = {"dense": SPARSE_QCQP, "csr": SPARSE_QCQP_CSR}
 
 
 class DeviceCallback:
@@ -210,10 +212,14 @@ def _coo_matvec(r, k, v, x, nrows):
 
 class SparseQCQPFamily(Family):
     """Sparse QCQP given by data (lfpsqp_sparse_qcqp, large-n mode); see sparse_qcqp().  Holds the canonical coordinate
-    lists: P, Ac, Ad as (row, col, val); Qc, Qd as (mat, row, col, val), sorted, duplicates summed, symmetric."""
+    lists: P, Ac, Ad as (row, col, val); Qc, Qd as (mat, row, col, val), sorted, duplicates summed, symmetric.
+    jacobian: the storage of J on the device, "dense" (family SPARSE_QCQP) or "csr" (SPARSE_QCQP_CSR)."""
 
-    def __init__(self, n, m, p, P, q, r, Qc, Ac, bc, Qd, Ad, bd):
-        super().__init__(SPARSE_QCQP, "sparse_qcqp", n, m, p)
+    def __init__(self, n, m, p, P, q, r, Qc, Ac, bc, Qd, Ad, bd, jacobian="dense"):
+        if jacobian not in _JACOBIAN_IDS:
+            raise _lib.LFPSQPError('sparse_qcqp: jacobian must be "dense" or "csr", got %r' % (jacobian,))
+        super().__init__(_JACOBIAN_IDS[jacobian], "sparse_qcqp", n, m, p)
+        self.jacobian = jacobian
         self.P, self.q, self.r, self.Qc, self.Ac, self.bc = P, q, float(r), Qc, Ac, bc
         self.Qd, self.Ad, self.bd = Qd, Ad, bd
 
@@ -252,12 +258,13 @@ class SparseQCQPFamily(Family):
         order = np.lexsort((Ac[1], Ac[0]))
         Ac = tuple(np.ascontiguousarray(a[order]) for a in Ac)
         aug = SparseQCQPFamily(n + p, m + p, 0, self.P, cat([self.q, np.zeros(p)]), self.r, Qc, Ac, cat([self.bc, self.bd]),
-                               _EMPTY4, _EMPTY3, np.zeros(0))
+                               _EMPTY4, _EMPTY3, np.zeros(0), self.jacobian)
         return aug, cat([x0, self.d_values(x0)]), cat([xl, dl]), cat([xu, du])
 
     def equalities(self):
         """the same objective and equalities without d(x)"""
-        return SparseQCQPFamily(self.n, self.m, 0, self.P, self.q, self.r, self.Qc, self.Ac, self.bc, _EMPTY4, _EMPTY3, np.zeros(0))
+        return SparseQCQPFamily(self.n, self.m, 0, self.P, self.q, self.r, self.Qc, self.Ac, self.bc, _EMPTY4, _EMPTY3, np.zeros(0),
+                                self.jacobian)
 
     def d_values(self, x):
         """d(x) = 1/2 x'Qd_k x + Ad_k.x - bd_k (numpy)"""
@@ -323,7 +330,7 @@ def _stack(Ms, name, dims, dn):
     return tuple(np.concatenate([p[j] for p in parts]) if parts else _EMPTY4[j] for j in range(4))
 
 
-def sparse_qcqp(P=None, q=None, r=None, Qc=None, Ac=None, bc=None, Qd=None, Ad=None, bd=None):
+def sparse_qcqp(P=None, q=None, r=None, Qc=None, Ac=None, bc=None, Qd=None, Ad=None, bd=None, jacobian="dense"):
     """Sparse quadratically constrained quadratic program (large-n mode, one GPU):
 
         f(x)   = 1/2 x'P x + q.x + r
@@ -334,9 +341,16 @@ def sparse_qcqp(P=None, q=None, r=None, Qc=None, Ac=None, bc=None, Qd=None, Ad=N
     are sequences of m and p (n, n) matrices.  None is all zero.  n, m and p are inferred.  Duplicate entries are summed and
     square matrices symmetrised as (M + M')/2, which leaves the quadratic forms unchanged.
 
+    jacobian selects how the device stores the m x n constraint Jacobian.  "dense" (the default) keeps it as a dense array
+    (8 m n bytes, twice with bounds); its passes stream all of it and the Gram is a dense DMMA SYRK.  "csr" keeps only its
+    structural entries, in CSR and CSC order, and runs the passes and the Gram over that pattern: memory and work scale with
+    nnz(J), which lets n grow far beyond what a dense J allows.  Both give the same solution up to rounding.
+
         fam = families.sparse_qcqp(P=laplacian, Qd=[ball_k ...], bd=radii2 / 2)
         x, obj, lam, info = optimize_large(fam.f, fam.c, fam.d, dl, du, x0, xl, xu, fam.m, fam.p)
     """
+    if jacobian not in _JACOBIAN_IDS:
+        raise _lib.LFPSQPError('sparse_qcqp: jacobian must be "dense" or "csr", got %r' % (jacobian,))
     dims = {}
     Pc = _EMPTY3
     if P is not None:
@@ -377,4 +391,4 @@ def sparse_qcqp(P=None, q=None, r=None, Qc=None, Ac=None, bc=None, Qd=None, Ad=N
         raise _lib.LFPSQPError("sparse_qcqp: p = %d inequalities need Qd or Ad" % p)
     return SparseQCQPFamily(n, m, p, Pc, vecs.get("q", np.zeros(n)), 0.0 if r is None else float(r),
                             Qcc if Qcc is not None else _EMPTY4, lin.get("Ac", _EMPTY3), vecs.get("bc", np.zeros(m)),
-                            Qdc if Qdc is not None else _EMPTY4, lin.get("Ad", _EMPTY3), vecs.get("bd", np.zeros(p)))
+                            Qdc if Qdc is not None else _EMPTY4, lin.get("Ad", _EMPTY3), vecs.get("bd", np.zeros(p)), jacobian)

@@ -70,6 +70,10 @@ function optimize_batched(fam::DeviceFamily, X0::Matrix{Float64}, xl, xu, param:
     x, obj, len, λ, term
 end
 
+# large-n sparse QCQP (lfpsqp_sparse_qcqp descriptor, lfpsqp_large_setup): Jacobian stored dense or in CSR / CSC form
+const LFPSQP_FAM_SPARSE_QCQP = 102
+const LFPSQP_FAM_SPARSE_QCQP_CSR = 103
+
 # dense QCQP given by data (LFPSQP_FAM_QCQP = 101): lfpsqp_qcqp is nine {pointer, batch stride} pairs
 struct CQcqp
     P::Ptr{Float64}; P_stride::Int64; q::Ptr{Float64}; q_stride::Int64; r::Ptr{Float64}; r_stride::Int64

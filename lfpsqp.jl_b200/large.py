@@ -5,7 +5,9 @@ import numpy as np
 
 from . import _lib
 from .api import LFPSQPParams, TerminationCondition, TerminationInfo, _family_of, _parse
-from .families import DIAGQUAD, SPARSE_QCQP, THOMSON
+from .families import DIAGQUAD, SPARSE_QCQP, SPARSE_QCQP_CSR, THOMSON
+
+_SPARSE = (SPARSE_QCQP, SPARSE_QCQP_CSR)
 
 
 class LargeProblem:
@@ -17,9 +19,9 @@ class LargeProblem:
         self.m = fam.m
         self.n_loc = fam.n if n_loc is None else n_loc
         self.n = fam.n if n_global is None else n_global
-        if fam.id == SPARSE_QCQP and fam.p > 0:
+        if fam.id in _SPARSE and fam.p > 0:
             raise _lib.LFPSQPError("a sparse_qcqp with d(x) is solved by optimize_large, which adds the slack variables")
-        if fam.id == SPARSE_QCQP and params_dev_ptr is None:
+        if fam.id in _SPARSE and params_dev_ptr is None:
             pp, _keep = fam.large_args()
             on_dev = 0
         elif params_dev_ptr is not None:
@@ -193,7 +195,7 @@ def optimize_large(*args, ctx=None, history=None, return_stats=False, noise=None
     bounds, else n."""
     f, c, d, dl, du, x0, xl, xu, m, p, param = _parse(args)
     fam = _family_of(f, c, d)
-    if fam.id not in (DIAGQUAD, THOMSON, SPARSE_QCQP):
+    if fam.id not in (DIAGQUAD, THOMSON) + _SPARSE:
         raise _lib.LFPSQPError("optimize_large takes a large-n device family (diagquad, thomson, sparse_qcqp); %r is not one"
                                % fam)
     if d is None or p == 0:                                                              # optimize.jl:15-17
@@ -211,12 +213,12 @@ def optimize_large(*args, ctx=None, history=None, return_stats=False, noise=None
     if history is None:   # every iterate's objective, as the reference returns (optimize.jl:250, :426)
         history = int(param.maxiter) + 1
     if p > 0:
-        if fam.id != SPARSE_QCQP:
+        if fam.id not in _SPARSE:
             raise _lib.LFPSQPError("d(x) in large-n mode needs a sparse_qcqp family (its slack variables are data)")
         prob_fam, x0w, xl, xu = fam.slack_embedding(x0, xl, xu, dl, du)
     else:
         prob_fam, x0w = fam, x0
-        if fam.id == SPARSE_QCQP and fam.p > 0:   # d! not passed (or p = 0): the equalities alone
+        if fam.id in _SPARSE and fam.p > 0:   # d! not passed (or p = 0): the equalities alone
             prob_fam = fam.equalities()
     prob = LargeProblem(prob_fam, ctx=ctx)
     prob.set_bounds(xl, xu)
