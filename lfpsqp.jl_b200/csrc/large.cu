@@ -64,14 +64,16 @@ static int read_ctrl(lfpsqp_ctx *c, LargeState &S) {
     S.guard_pending = false;
     const double lo = S.hctrl->ldiag_min, hi = S.hctrl->ldiag_max;   // ~lambda_min(G) (from above), trace(G)
     S.pivot_ratio2 = (lo > 0.0) ? hi / lo : INFINITY;
-    S.explicit_inverse_ok = S.pivot_ratio2 <= S.inverse_guard;
-    const char *env = getenv("LFPSQP_EXPLICIT_INVERSE");
-    if (env && (env[0] == '0' || env[0] == '1')) S.explicit_inverse_ok = env[0] == '1';
+    S.explicit_inverse_ok = S.force_inverse >= 0 ? S.force_inverse == 1 : S.pivot_ratio2 <= S.inverse_guard;
   }
   return 0;
 }
 static void write_ctrl_fields(LargeState &S) {  // push the host copy (tolerances, limits, statuses) to the device
   cudaMemcpyAsync(S.ctrl, S.hctrl, sizeof(LargeCtrl), cudaMemcpyHostToDevice, S.stream);
+}
+static void reset_ctrl(LargeState &S) {   // a cleared control block on the host and the device
+  memset(S.hctrl, 0, sizeof(LargeCtrl));
+  write_ctrl_fields(S);
 }
 
 // lfpsqp_large_last_dispatch bits of a dgemm_nt instantiation: 1 <128> lean, 2 <128> with the extras' prologue, 4 <64>,
@@ -91,13 +93,7 @@ static void gemm_nt(LargeState &S, int M, int N, int K, const double *A, int64_t
   GemmExt X; if (ext) X = *ext;
   if (X.batch > 1) {   // independent products of one shape: blockIdx.z = product
     grid.z = X.batch;
-    if (narrow) dgemm_nt_kernel<64><<<grid, 256, dgemm_smem_bytes<64>(), S.stream>>>(M, N, K, A, lda, B, ldb, C, ldc, mode, lower, 1, 0, X);
-    else dgemm_nt_kernel<128><<<grid, 256, dgemm_smem_bytes<128>(), S.stream>>>(M, N, K, A, lda, B, ldb, C, ldc, mode, lower, 1, 0, X);
-    note_gemm(S, narrow ? 4 : 2);
-    S.launches++;
-    return;
-  }
-  if (mode != GEMM_SUB && tiles * 2 <= S.sm_count && K >= 1024 && !X.tri) {
+  } else if (mode != GEMM_SUB && tiles * 2 <= S.sm_count && K >= 1024 && !X.tri) {
     ksplit = std::min(std::min(16, S.sm_count / tiles), K / 256);
     while (ksplit > 1 && (size_t)ksplit * M * (N + 1) * 8 > S.gemm_ws_bytes) ksplit--;
     if (ksplit < 1) ksplit = 1;
@@ -118,23 +114,19 @@ static void gemm_nt(LargeState &S, int M, int N, int K, const double *A, int64_t
   // zero-slab skipping (SYRK of a block-sparse J): the chunk list of one K slice must fit behind the tiles in shared memory
   const int kchunks = (K + GM_BK - 1) / GM_BK, per = (kchunks + ksplit - 1) / ksplit;
   const size_t skip_smem = dgemm_smem_bytes<128>() + (size_t)per * sizeof(int);
-  const bool skip = X.nz && !narrow && skip_smem <= (size_t)S.max_dyn_smem;
+  const bool skip = X.nz && X.batch <= 1 && !narrow && skip_smem <= (size_t)S.max_dyn_smem;
   const bool lean = !ext;   // plain product: the instantiation without the extras' prologue
   note_gemm(S, skip ? 8 : narrow ? 4 : lean ? 1 : 2);
+  const auto kern = skip ? dgemm_nt_kernel<128, true> : narrow ? dgemm_nt_kernel<64> : lean ? dgemm_nt_kernel<128, false, false> : dgemm_nt_kernel<128>;
+  const size_t smem = skip ? skip_smem : narrow ? dgemm_smem_bytes<64>() : dgemm_smem_bytes<128>();
   if (ksplit == 1) {
-    if (skip) dgemm_nt_kernel<128, true><<<grid, 256, skip_smem, S.stream>>>(M, N, K, A, lda, B, ldb, C, ldc, mode, lower, 1, 0, X);
-    else if (narrow) dgemm_nt_kernel<64><<<grid, 256, dgemm_smem_bytes<64>(), S.stream>>>(M, N, K, A, lda, B, ldb, C, ldc, mode, lower, 1, 0, X);
-    else if (lean) dgemm_nt_kernel<128, false, false><<<grid, 256, dgemm_smem_bytes<128>(), S.stream>>>(M, N, K, A, lda, B, ldb, C, ldc, mode, lower, 1, 0, X);
-    else dgemm_nt_kernel<128><<<grid, 256, dgemm_smem_bytes<128>(), S.stream>>>(M, N, K, A, lda, B, ldb, C, ldc, mode, lower, 1, 0, X);
+    kern<<<grid, 256, smem, S.stream>>>(M, N, K, A, lda, B, ldb, C, ldc, mode, lower, 1, 0, X);
     S.launches++;
   } else {
     grid.z = ksplit;
     const int64_t ldw = (N + 1) & ~1;   // even row pitch: the epilogue stores 16-byte pairs
     const int64_t stride = (int64_t)M * ldw;
-    if (skip) dgemm_nt_kernel<128, true><<<grid, 256, skip_smem, S.stream>>>(M, N, K, A, lda, B, ldb, S.gemm_ws, ldw, GEMM_ASSIGN, lower, ksplit, stride, X);
-    else if (narrow) dgemm_nt_kernel<64><<<grid, 256, dgemm_smem_bytes<64>(), S.stream>>>(M, N, K, A, lda, B, ldb, S.gemm_ws, ldw, GEMM_ASSIGN, lower, ksplit, stride, X);
-    else if (lean) dgemm_nt_kernel<128, false, false><<<grid, 256, dgemm_smem_bytes<128>(), S.stream>>>(M, N, K, A, lda, B, ldb, S.gemm_ws, ldw, GEMM_ASSIGN, lower, ksplit, stride, X);
-    else dgemm_nt_kernel<128><<<grid, 256, dgemm_smem_bytes<128>(), S.stream>>>(M, N, K, A, lda, B, ldb, S.gemm_ws, ldw, GEMM_ASSIGN, lower, ksplit, stride, X);
+    kern<<<grid, 256, smem, S.stream>>>(M, N, K, A, lda, B, ldb, S.gemm_ws, ldw, GEMM_ASSIGN, lower, ksplit, stride, X);
     const double *ws = S.gemm_ws;
     const double sgn = (mode == GEMM_ASSIGN_NEG) ? -1.0 : 1.0;
     const int lo = lower;
@@ -152,18 +144,12 @@ static void gemm_nt(LargeState &S, int M, int N, int K, const double *A, int64_t
 
 static void rows_dot(LargeState &S, const double *Jm, int64_t ld, int m, int64_t ncols, const double *v, double *t, int pred) {
   if (m <= 0) return;
-  if (Jm == S.J && S.jmap_valid && S.gram_mode == 1) {   // block-sparse J: same pass, loads of all-zero slabs not issued
-    if (m >= 8 * S.sm_count) rows_dot_kernel<4, true><<<(m + 3) / 4, 256, 0, S.stream>>>(Jm, ld, m, ncols, v, t, S.ctrl, pred, S.nzmap, S.nz_ld);
-    else if (m >= 2 * S.sm_count) rows_dot_kernel<2, true><<<(m + 1) / 2, 256, 0, S.stream>>>(Jm, ld, m, ncols, v, t, S.ctrl, pred, S.nzmap, S.nz_ld);
-    else rows_dot_kernel<1, true><<<m, 256, 0, S.stream>>>(Jm, ld, m, ncols, v, t, S.ctrl, pred, S.nzmap, S.nz_ld);
-    S.disp[LARGE_DISP_ROWS_DOT] |= (m >= 8 * S.sm_count ? 4 : m >= 2 * S.sm_count ? 2 : 1) << 3;
-    S.launches++;
-    return;
-  }
-  if (m >= 8 * S.sm_count) rows_dot_kernel<4><<<(m + 3) / 4, 256, 0, S.stream>>>(Jm, ld, m, ncols, v, t, S.ctrl, pred);
-  else if (m >= 2 * S.sm_count) rows_dot_kernel<2><<<(m + 1) / 2, 256, 0, S.stream>>>(Jm, ld, m, ncols, v, t, S.ctrl, pred);
-  else rows_dot_kernel<1><<<m, 256, 0, S.stream>>>(Jm, ld, m, ncols, v, t, S.ctrl, pred);
-  S.disp[LARGE_DISP_ROWS_DOT] |= m >= 8 * S.sm_count ? 4 : m >= 2 * S.sm_count ? 2 : 1;   // bits 0-2: R = 1, 2, 4 ; 3-5: SKIP
+  const bool skip = Jm == S.J && S.jmap_valid && S.gram_mode == 1;   // block-sparse J: same pass, loads of all-zero slabs not issued
+  const int R = m >= 8 * S.sm_count ? 4 : m >= 2 * S.sm_count ? 2 : 1;
+  static decltype(&rows_dot_kernel<1>) const kern[2][3] = {{rows_dot_kernel<1>, rows_dot_kernel<2>, rows_dot_kernel<4>},
+                                                           {rows_dot_kernel<1, true>, rows_dot_kernel<2, true>, rows_dot_kernel<4, true>}};
+  kern[skip][R / 2]<<<(m + R - 1) / R, 256, 0, S.stream>>>(Jm, ld, m, ncols, v, t, S.ctrl, pred, skip ? S.nzmap : nullptr, skip ? S.nz_ld : 0);
+  S.disp[LARGE_DISP_ROWS_DOT] |= R << (skip ? 3 : 0);   // bits 0-2: R = 1, 2, 4 ; 3-5: SKIP
   S.launches++;
 }
 static void cols_dot(LargeState &S, const double *Jm, int64_t ld, int m, int64_t ncols, const double *u, int pred) {
@@ -223,6 +209,13 @@ static void spj_gram(LargeState &S) {
   }
   S.disp[LARGE_DISP_GEMM] |= 256;
 }
+// u = T t with T = L^-1 (lower) or T = L^-T (upper, S.XT) of the cached factor; u_copy (optional) receives u as well
+static void tri_gemv(LargeState &S, int upper, const double *t, double *u, double *u_copy, int pred) {
+  const int m = S.m;
+  tri_gemv_kernel<<<(m + 7) / 8, 256, m * sizeof(double), S.stream>>>(upper ? S.XT : S.Linv, S.ldm, m, t, u, upper, u_copy, S.ctrl, pred,
+                                                                      S.invflag_valid ? S.invflag : nullptr, S.nz_rows);
+  S.launches++;
+}
 // u = (J J')^-1 t through the cached factor: y = L^-1 t ; u = L^-T y
 static void gram_solve(LargeState &S, const double *t, double *u, double *u_copy, int pred) {
   const int m = S.m;
@@ -233,10 +226,9 @@ static void gram_solve(LargeState &S, const double *t, double *u, double *u_copy
     S.launches++;
     return;
   }
-  tri_gemv_kernel<<<(m + 7) / 8, 256, m * sizeof(double), S.stream>>>(S.Linv, S.ldm, m, t, S.ty, 0, nullptr, S.ctrl, pred, S.invflag_valid ? S.invflag : nullptr, S.nz_rows);
-  tri_gemv_kernel<<<(m + 7) / 8, 256, m * sizeof(double), S.stream>>>(S.XT, S.ldm, m, S.ty, u, 1, u_copy, S.ctrl, pred, S.invflag_valid ? S.invflag : nullptr, S.nz_rows);
+  tri_gemv(S, 0, t, S.ty, nullptr, pred);
+  tri_gemv(S, 1, S.ty, u, u_copy, pred);
   S.disp[LARGE_DISP_SOLVE] |= LARGE_SOLVE_TRIANGULAR;
-  S.launches += 2;
 }
 
 // ------------------------------------------------------------------ family dispatch (device callbacks, whole-GPU kernels)
@@ -367,8 +359,7 @@ static void fam_hess_prepare(LargeState &S, const double *x, const double *lam) 
     const lfpsqp::IneqDev I = S.I; const bool ineq = S.ineq;
     // with bounds the augmented terms of inequality_helper.jl:144-158 are diagonal too: fold them into hdiag (2n entries)
     vec(S, n, [=] __device__(int64_t j, double *) {
-      double s = w[j];
-      for (int k = 0; k < ns; k++) s += cp[(int64_t)k * n + j];
+      double s = split_sum(cp, ns, n, j, w[j]);
       if (ineq) { const double ly2 = 2.0 * I.lamy[j]; s += ly2 * I.q[j]; hd[n + j] = ly2 * I.s[j]; }
       hd[j] = s;
     });
@@ -451,8 +442,7 @@ template <class T> static bool dalloc(LargeState &S, T **p, size_t count);
 static void gram_syrk(LargeState &S, const double *Jg) {
   const int m = S.m;
   GemmExt X; const GemmExt *ext = nullptr;
-  const char *env = getenv("LFPSQP_GRAM_SKIP");   // "0": always the plain dense SYRK (tests compare the two bit for bit)
-  if (S.gram_mode != 2 && S.nzmap && m > 64 && !(env && env[0] == '0')) {
+  if (S.gram_skip && S.gram_mode != 2 && S.nzmap && m > 64) {
     cudaMemsetAsync(&S.ctrl->nz_count, 0, sizeof(unsigned long long), S.stream);
     dim3 sg((unsigned)((S.n_loc + 1023) / 1024), (unsigned)S.nz_rows);
     zero_slab_map_kernel<<<sg, 256, 0, S.stream>>>(Jg, S.ldj, m, S.n_loc, S.nzmap, S.nz_ld, &S.ctrl->nz_count);
@@ -465,11 +455,21 @@ static void gram_syrk(LargeState &S, const double *Jg) {
   gemm_nt(S, m, m, (int)S.n_loc, Jg, S.ldj, Jg, S.ldj, S.G, S.ldm, GEMM_ASSIGN, 1, ext);
   S.disp_syrk = false;
 }
-static void gram_only(LargeState &S) {   // S.G (lower tiles) = J W J', all-reduced
+// S.G (lower triangle) = J J', or with bounds J diag(Dy^2) J' = PJct' PJct (optimize.jl:288-289 / SURVEY App. B), summed over
+// the ranks.  timed: ev_g0 / ev_g1 bracket the product (the gram_ms of lfpsqp_large_factor).
+static void gram(LargeState &S, bool timed) {
   const int m = S.m;
-  if (S.csr) { spj_gram(S); return; }
-  const double *Jg = S.ineq ? S.Jw : S.J;    // Jw = J diag(Dy) was formed by the factorize() call that precedes
-  gram_syrk(S, Jg);
+  const double *Jg = S.J;
+  if (S.ineq && !S.csr) {   // SYRK operand Jw = J diag(Dy); the CSR Gram applies the weights itself
+    dim3 sg((unsigned)std::min<int64_t>(std::max<int64_t>(((S.n_loc >> 1) + 255) / 256, 1), 32), (unsigned)std::min(m, 65535));
+    ineq_scale_cols_kernel<<<sg, 256, 0, S.stream>>>(S.J, S.ldj, m, S.n_loc, S.I.Dy, S.Jw);
+    S.launches++;
+    Jg = S.Jw;
+  }
+  if (timed) cudaEventRecord(S.ev_g0, S.stream);
+  if (S.csr) spj_gram(S);
+  else gram_syrk(S, Jg);
+  if (timed) cudaEventRecord(S.ev_g1, S.stream);
   if (S.world > 1) comm_allreduce(S, S.G, (size_t)m * S.ldm);
 }
 // Truncated path of optimize.jl:297-302 in Gram form: G = V diag(lambda) V' (Jacobi, large_eig.cu), G^+ into S.Ginv.
@@ -482,7 +482,7 @@ static int factorize_pinv(lfpsqp_ctx *c, LargeState &S, bool regram) {
     if (ok && !S.Ginv) ok = dalloc(S, &S.Ginv, (size_t)m * ldm);
     if (!ok) return c->fail(LFPSQP_ERR_NOMEM, "rank-deficient path: workspace allocation failed");
   }
-  if (regram) gram_only(S);
+  if (regram) gram(S, false);
   unsigned long long *sc = S.eigScratch;
   if (large_eig_pinv_factors(S, S.G, S.eigV, S.eigLam, 1, reinterpret_cast<int *>(sc + 34), sc, reinterpret_cast<unsigned *>(sc + 32)))
     return c->fail(LFPSQP_ERR_CUDA, "rank-deficient path: cooperative launch of the Jacobi eigen-solver failed");
@@ -494,23 +494,10 @@ static int factorize_pinv(lfpsqp_ctx *c, LargeState &S, bool regram) {
   return 0;
 }
 
-// ------------------------------------------------------------------ factorisation: G = J J' = L L', XT = L^-T, Linv = L^-1
-// (with bounds G = J diag(Dy^2) J' = PJct' PJct, optimize.jl:288-289 / SURVEY App. B)
+// ------------------------------------------------------------------ factorisation of the Gram in S.G: G = L L', XT = L^-T, Linv = L^-1
 static int factorize(lfpsqp_ctx *c, LargeState &S) {
   const int m = S.m; const int64_t ldm = S.ldm;
-  const double *Jg = S.J;
   S.invflag_valid = false;
-  if (S.ineq && !S.csr) {
-    dim3 sg((unsigned)std::min<int64_t>(std::max<int64_t>(((S.n_loc >> 1) + 255) / 256, 1), 32), (unsigned)std::min(m, 65535));
-    ineq_scale_cols_kernel<<<sg, 256, 0, S.stream>>>(S.J, S.ldj, m, S.n_loc, S.I.Dy, S.Jw);
-    S.launches++;
-    Jg = S.Jw;
-  }
-  cudaEventRecord(S.ev_g0, S.stream);
-  if (S.csr) spj_gram(S);   // weighted by Dy^2 with bounds
-  else gram_syrk(S, Jg);    // SYRK, lower tiles
-  cudaEventRecord(S.ev_g1, S.stream);
-  if (S.world > 1) comm_allreduce(S, S.G, (size_t)m * ldm);
   if (S.prefer_pinv) return factorize_pinv(c, S, false);   // this problem lost rank before: go straight to the eigen-decomposition
   S.pinv_active = false; S.rank_cur = m;
   diag_thresh_kernel<<<1, 256, 0, S.stream>>>(S.G, ldm, m, S.prm.eps_rank, S.thresh);
@@ -523,26 +510,23 @@ static int factorize(lfpsqp_ctx *c, LargeState &S) {
   const GemmExt *f1 = nullptr, *f2 = nullptr;
   int *done = nullptr;
   bool chain = true;
-  {
-    const char *env = getenv("LFPSQP_GRAM_SKIP");
-    if (S.blkflag && nblk > 1 && !(env && env[0] == '0')) {
-      block_nz_kernel<<<dim3(nblk, nblk), 256, 0, S.stream>>>(S.G, ldm, m, S.blkflag, nblk);
-      S.launches++;
-      F1.bf = S.blkflag; F1.bf_ld = nblk; F1.bf_n = nblk; F1.bf_mode = 1;
-      F2 = F1; F2.bf_mode = 2; F3 = F1; F3.bf_mode = 3;
-      f1 = &F1; f2 = &F2;
-      done = S.blkflag + (size_t)nblk * nblk;
-      // diagonal blocks nothing will ever update: factorised now, in parallel; the chain below skips them
-      cudaMemsetAsync(&S.ctrl->g_dependent, 0, sizeof(int), S.stream);
-      potf2_inv_indep_kernel<NB><<<nblk, 256, psm, S.stream>>>(S.G, ldm, m, S.Dblk, S.thresh, &S.ctrl->rankflag, S.blkflag, nblk, done,
-                                                               &S.ctrl->g_dependent);
-      S.launches++;
-      if (S.g_blockdiag == 1) {   // block diagonal last time: look now (one short sync instead of ~5 launches per block)
-        cudaMemcpyAsync(&S.hctrl->g_dependent, &S.ctrl->g_dependent, sizeof(int), cudaMemcpyDeviceToHost, S.stream);
-        if (cudaStreamSynchronize(S.stream) == cudaSuccess && S.hctrl->g_dependent == 0) chain = false;
-        else S.g_blockdiag = 0;
-      } else S.gdep_pending = true;
-    }
+  if (S.blkflag && nblk > 1 && S.gram_skip) {
+    block_nz_kernel<<<dim3(nblk, nblk), 256, 0, S.stream>>>(S.G, ldm, m, S.blkflag, nblk);
+    S.launches++;
+    F1.bf = S.blkflag; F1.bf_ld = nblk; F1.bf_n = nblk; F1.bf_mode = 1;
+    F2 = F1; F2.bf_mode = 2; F3 = F1; F3.bf_mode = 3;
+    f1 = &F1; f2 = &F2;
+    done = S.blkflag + (size_t)nblk * nblk;
+    // diagonal blocks nothing will ever update: factorised now, in parallel; the chain below skips them
+    cudaMemsetAsync(&S.ctrl->g_dependent, 0, sizeof(int), S.stream);
+    potf2_inv_indep_kernel<NB><<<nblk, 256, psm, S.stream>>>(S.G, ldm, m, S.Dblk, S.thresh, &S.ctrl->rankflag, S.blkflag, nblk, done,
+                                                             &S.ctrl->g_dependent);
+    S.launches++;
+    if (S.g_blockdiag == 1) {   // block diagonal last time: look now (one short sync instead of ~5 launches per block)
+      cudaMemcpyAsync(&S.hctrl->g_dependent, &S.ctrl->g_dependent, sizeof(int), cudaMemcpyDeviceToHost, S.stream);
+      if (cudaStreamSynchronize(S.stream) == cudaSuccess && S.hctrl->g_dependent == 0) chain = false;
+      else S.g_blockdiag = 0;
+    } else S.gdep_pending = true;
   }
   // Right-looking blocked Cholesky with LOOK-AHEAD: the single-CTA factorisation of diagonal block b+1 (latency-bound, ~50 us)
   // runs on a second stream while the main stream applies the rank-NB update of block b to the rest of the trailing matrix.
@@ -654,8 +638,7 @@ static void project(LargeState &S, double *v, double *lam_out, int pred, int wan
   const double *cp = S.cpart; int ns = S.m > 0 ? S.jsplit : 0; int64_t n = S.n_loc;
   if (!S.ineq) {
     vec(S, n, [=] __device__(int64_t j, double *acc) {
-      double s = 0.0;
-      for (int k = 0; k < ns; k++) s += cp[(int64_t)k * n + j];
+      const double s = split_sum(cp, ns, n, j);
       double r = v[j] - s; v[j] = r;
       acc[0] += r * r; acc[3] = nanmax(acc[3], fabs(r));
     }, 0, want_norms ? 1 : 0, want_norms);
@@ -685,14 +668,13 @@ static int projcg(lfpsqp_ctx *c, LargeState &S, double tol, int64_t maxit, int c
   const double *b = S.d;
   if (S.family == LFPSQP_FAM_HOST) chunk = 1;   // the Hessian callback runs on the host: one status check per iteration
   if (cvec && S.m > 0 && !S.ineq) {
-    const int m = S.m;
-    tri_gemv_kernel<<<(m + 7) / 8, 256, m * sizeof(double), S.stream>>>(S.XT, S.ldm, m, cvec, S.tu, 1, nullptr, S.ctrl, 0, S.invflag_valid ? S.invflag : nullptr, S.nz_rows);   // L^-T c
+    tri_gemv(S, 1, cvec, S.tu, nullptr, 0);   // L^-T c
     jcols(S, S.tu, 0);
     const double *cp = S.cpart; const int64_t nl = S.n_loc;
-    vec(S, n, [=] __device__(int64_t j, double *) { double s = 0.0; for (int k = 0; k < ns; k++) s += cp[(int64_t)k * nl + j]; xs[j] = s; });
+    vec(S, n, [=] __device__(int64_t j, double *) { xs[j] = split_sum(cp, ns, nl, j); });
     hess_apply(S, r, xs, 0);
     vec(S, n, [=] __device__(int64_t i, double *) { r[i] -= b[i]; });
-    S.launches += 3;
+    S.launches += 2;
   } else
   vec(S, n, [=] __device__(int64_t i, double *) { xs[i] = 0.0; r[i] = -b[i]; });
   // g = r - U U' r (projcg.jl:59-60) ; r = g ; d = -g ; rg partials -> loop slot 3 (= 2 + (par^1) for k = 0)
@@ -752,8 +734,8 @@ static int projcg(lfpsqp_ctx *c, LargeState &S, double tol, int64_t maxit, int c
       vec(S, n, [=] __device__(int64_t i, double *) { Ad[i] = b[i] - Ad[i]; });
       jrows(S, Ad, S.tm, 0);
       if (S.world > 1) comm_allreduce(S, S.tm, S.m);
-      tri_gemv_kernel<<<(S.m + 7) / 8, 256, S.m * sizeof(double), S.stream>>>(S.Linv, S.ldm, S.m, S.tm, lam_out, 0, nullptr, S.ctrl, 0, S.invflag_valid ? S.invflag : nullptr, S.nz_rows);
-      S.launches += 2;
+      tri_gemv(S, 0, S.tm, lam_out, nullptr, 0);
+      S.launches++;
       (void)st_keep;
     }
   }
@@ -916,12 +898,12 @@ static int retract_nr(lfpsqp_ctx *c, LargeState &S, int *flag_out, int *it1) {
     rows_dot(S, D, ldm, m, m, cval, t1, 0);                                              // D c
     vec(S, m, [=] __device__(int64_t a, double *) { t1[a] = -t1[a]; });                   // :140 delta = -D c
     // xnew += Q delta, Q = J' L^-T (:141)
-    tri_gemv_kernel<<<(m + 7) / 8, 256, m * sizeof(double), S.stream>>>(S.XT, ldm, m, t1, S.tu, 1, nullptr, S.ctrl, 0, S.invflag_valid ? S.invflag : nullptr, S.nz_rows);
+    tri_gemv(S, 1, t1, S.tu, nullptr, 0);
     jcols(S, S.tu, 0);
     { const double *cp = S.cpart; int ns = S.jsplit;
       // with bounds the basis is Q = PJct L^-T: x += Dy^2 w, y -= Dx Dy w, then y_retract! (:141-143)
       vec(S, n, [=] __device__(int64_t j, double *) {
-        double s = 0.0; for (int k = 0; k < ns; k++) s += cp[(int64_t)k * n + j];
+        const double s = split_sum(cp, ns, n, j);
         if (!ineq) { xnew[j] += s; return; }
         const double dx = I.Dx[j], dy = I.Dy[j];
         double xn = xnew[j] + dy * dy * s, yn = xnew[n + j] - dx * dy * s;
@@ -936,7 +918,7 @@ static int retract_nr(lfpsqp_ctx *c, LargeState &S, int *flag_out, int *it1) {
       cols_dot_kernel<false><<<grid, 256, S.rows_per_split * sizeof(double), S.stream>>>(D, ldm, m, m, t1, S.cpart, S.rows_per_split, S.ctrl, 0);
       const double *cp = S.cpart; int ns = S.nsplit;
       vec(S, m, [=] __device__(int64_t a, double *acc) {
-        double s = 0.0; for (int k = 0; k < ns; k++) s += cp[(int64_t)k * m + a];
+        const double s = split_sum(cp, ns, m, a);
         t2[a] = s; acc[0] += s * dcv[a];
       }, 0, 1);
       finalize(S, 1u, 0, 1u);
@@ -949,11 +931,27 @@ static int retract_nr(lfpsqp_ctx *c, LargeState &S, int *flag_out, int *it1) {
         D[(int64_t)rr * ldm + cc2] += (1.0 / ctrl->s[0]) * t1[rr] * t2[cc2];
       });
     }
-    S.launches += 9;
+    S.launches += 8;
     i++;
   }
   *flag_out = (i == S.prm.maxiter_retract) ? 1 : 0; *it1 = i;
   return 0;
+}
+
+// one trial point of a line search: xtil = x + al d, retracted into xnew by kind 0 Euclidean (a copy), 1 YRetract, 2 NR or
+// 3 ProjPenalty; flag = the retraction's flag (0 for kinds 0 and 1)
+static int retract_trial(lfpsqp_ctx *c, LargeState &S, int kind, double al, int *flag) {
+  const double *x = S.x, *d = S.d; double *xtil = S.xtil;
+  vec(S, S.nv, [=] __device__(int64_t i, double *) { xtil[i] = x[i] + al * d[i]; });
+  int rc = 0, i1 = 0, i2 = 0;
+  *flag = 0;
+  if (kind <= 1) {
+    cudaMemcpyAsync(S.xnew, xtil, S.nv * sizeof(double), cudaMemcpyDeviceToDevice, S.stream);
+    if (kind == 1) y_retract(S, S.xnew, x);
+  } else if (kind == 2) rc = retract_nr(c, S, flag, &i1);
+  else rc = retract_pp(c, S, flag, &i1, &i2);
+  S.retract_outer += i1; S.retract_pcg += i2; S.armijo_trials++;
+  return rc;
 }
 
 // ------------------------------------------------------------------ exact_linesearch! (linesearch.jl:107-339), host control flow
@@ -964,17 +962,11 @@ static int exact_linesearch(lfpsqp_ctx *c, LargeState &S, int kind, double fval,
   const double phi1 = (3.0 - sqrt(5.0)) / 2.0, phi2 = (sqrt(5.0) - 1.0) / 2.0, phi3 = (sqrt(5.0) + 1.0) / 2.0;
   double Delta = prm.alpha, f_a = 0, f_b = 0, f_c = 0, f_d = 0, a_a = 0, a_b = 0, a_c = 0, a_d = 0;
   double *x_a = S.ex[0], *x_b = S.ex[1], *x_c = S.ex[2], *x_d = S.ex[3], *swp;
-  const double *x = S.x, *d = S.d; double *xtil = S.xtil, *xnew = S.xnew;
+  const double *x = S.x, *d = S.d; double *xnew = S.xnew;
   bool do_shrinking = true;
   int flag = 0, rc = 0;
   auto TRIAL = [&](double *pt, double al) {
-    vec(S, n, [=] __device__(int64_t i, double *) { xtil[i] = x[i] + al * d[i]; });
-    int i1 = 0, i2 = 0;
-    if (kind == 0) { cudaMemcpyAsync(xnew, xtil, n * 8, cudaMemcpyDeviceToDevice, S.stream); flag = 0; }
-    else if (kind == 1) { cudaMemcpyAsync(xnew, xtil, n * 8, cudaMemcpyDeviceToDevice, S.stream); y_retract(S, xnew, x); flag = 0; }
-    else if (kind == 2) rc |= retract_nr(c, S, &flag, &i1);
-    else rc |= retract_pp(c, S, &flag, &i1, &i2);
-    S.retract_outer += i1; S.retract_pcg += i2; S.armijo_trials++;
+    rc |= retract_trial(c, S, kind, al, &flag);
     cudaMemcpyAsync(pt, xnew, n * 8, cudaMemcpyDeviceToDevice, S.stream);
   };
   auto FVAL = [&](const double *pt) -> double {
@@ -1063,8 +1055,7 @@ static int solve(lfpsqp_ctx *c, LargeState &S, const double *x0_host, double *x_
     vec(S, n, [=] __device__(int64_t j, double *) { x[n + j] = ineq_y0(I.q[j], I.r[j], I.s[j], I.t[j], x[j]); });
     CK(cudaMemsetAsync(S.cvh, 0, n * sizeof(double), S.stream));
   }
-  memset(S.hctrl, 0, sizeof(LargeCtrl));
-  write_ctrl_fields(S);
+  reset_ctrl(S);
   int64_t it = 0, nobj = 0;
   double f_diff = INFINITY, step_diff = INFINITY, kkt_diff = INFINITY, prev_grad_norm = 0.0;
   fam_f(S, x); finalize(S, 1u, 0);
@@ -1097,6 +1088,7 @@ static int solve(lfpsqp_ctx *c, LargeState &S, const double *x0_host, double *x_
       const double tf0 = now_ms();
       if (m > 0) {
         fam_c_jac(S, true, S.cval, x);                                                   // :283
+        gram(S, true);
         if (factorize(c, S)) return LFPSQP_ERR_CUDA;
         cudaMemcpyAsync(xtil, d, nv * sizeof(double), cudaMemcpyDeviceToDevice, S.stream);   // d before the projection (rank-loss redo)
       }
@@ -1153,14 +1145,7 @@ static int solve(lfpsqp_ctx *c, LargeState &S, const double *x0_host, double *x_
     const bool exact = (prm.linesearch != 0 && !prm.disable_linesearch);                // :415-420
     if (exact) { if (exact_linesearch(c, S, kind, fval, &newf, &f_diff, &step_diff, &flag)) return S.cb_err ? LFPSQP_ERR_CALLBACK : LFPSQP_ERR_CUDA; }
     while (!exact && step_diff > prm.eps_x) {
-      double al = alpha;
-      vec(S, nv, [=] __device__(int64_t i, double *) { xtil[i] = x[i] + al * d[i]; });
-      int i1 = 0, i2 = 0;
-      if (kind == 0) cudaMemcpyAsync(xnew, xtil, nv * sizeof(double), cudaMemcpyDeviceToDevice, S.stream);
-      else if (kind == 1) { cudaMemcpyAsync(xnew, xtil, nv * sizeof(double), cudaMemcpyDeviceToDevice, S.stream); y_retract(S, xnew, x); }
-      else if (kind == 2) { if (retract_nr(c, S, &flag, &i1)) return S.cb_err ? LFPSQP_ERR_CALLBACK : LFPSQP_ERR_CUDA; }
-      else { if (retract_pp(c, S, &flag, &i1, &i2)) return S.cb_err ? LFPSQP_ERR_CALLBACK : LFPSQP_ERR_CUDA; }
-      S.retract_outer += i1; S.retract_pcg += i2; S.armijo_trials++;
+      if (retract_trial(c, S, kind, alpha, &flag)) return S.cb_err ? LFPSQP_ERR_CALLBACK : LFPSQP_ERR_CUDA;
       // linesearch.jl:57-60 has no lower bound on alpha in this branch: when the retraction fails at EVERY alpha the
       // reference spins forever once alpha has underflowed to 0.  Stop at the floor the other branch uses (:82-85):
         // flag 98, LFPSQP_ST_NONFINITE.
@@ -1231,6 +1216,16 @@ template <class T> static bool dalloc(LargeState &S, T **p, size_t count) {
   if (cudaMalloc(&q, std::max<size_t>(count, 1) * sizeof(T)) != cudaSuccess) { cudaGetLastError(); return false; }
   S.owned.push_back(q); *p = (T *)q;
   return true;
+}
+// count = the number of ranks on which flag is set (one all-reduce: also a barrier of all ranks)
+static int ranks_with(lfpsqp_ctx *c, LargeState &S, bool flag, int *count) {
+  double v = flag ? 1.0 : 0.0;
+  CK(cudaMemcpyAsync(S.commbuf, &v, 8, cudaMemcpyHostToDevice, S.stream));
+  comm_allreduce(S, S.commbuf, 1);
+  CK(cudaMemcpyAsync(&v, S.commbuf, 8, cudaMemcpyDeviceToHost, S.stream));
+  CK(cudaStreamSynchronize(S.stream));
+  *count = (int)lround(v);
+  return 0;
 }
 
 extern "C" int lfpsqp_large_setup(lfpsqp_ctx *c, int family, int64_t n_global, int64_t m, int64_t col0, int64_t n_loc,
@@ -1354,21 +1349,20 @@ extern "C" int lfpsqp_large_setup(lfpsqp_ctx *c, int family, int64_t n_global, i
     CK(cudaFuncSetAttribute(spj_gram_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max<size_t>(mm * sizeof(double), 1024)));
   }
   CK(cudaStreamSynchronize(S.stream));
-  {
-    const char *env = getenv("LFPSQP_FUSED_PROJCG");   // "0" selects the multi-kernel projcg loop (A/B measurements, tests)
-    // pcg! is fused for every family with a dense J, projcg for diagonal Hessians; the CSR form runs the launch-per-phase loops
-    if (m > 0 && !csr && !(env && env[0] == '0')) fused_projcg_init(S, c->device);
-  }
+  // the environment switches of the README (A/B measurements, tests), read once per problem
+  const char *fused_env = getenv("LFPSQP_FUSED_PROJCG"), *skip_env = getenv("LFPSQP_GRAM_SKIP"), *inv_env = getenv("LFPSQP_EXPLICIT_INVERSE");
+  S.gram_skip = !(skip_env && skip_env[0] == '0');
+  S.force_inverse = (inv_env && (inv_env[0] == '0' || inv_env[0] == '1')) ? inv_env[0] - '0' : -1;
+  // pcg! is fused for every family with a dense J, projcg for diagonal Hessians; the CSR form runs the launch-per-phase loops
+  if (m > 0 && !csr && !(fused_env && fused_env[0] == '0')) fused_projcg_init(S, c->device);
   if (S.world > 1) {
     // every rank must take the same path (a rank in the launch-per-phase loop would deadlock against peers inside the fused
     // mailbox protocol): fused only if ALL ranks are eligible.  The all-reduce is also the barrier that ends setup, so that
     // no rank starts exchanging while another one is still uploading its parameters.
-    double flag = S.fused_ok ? 1.0 : 0.0;
-    CK(cudaMemcpyAsync(S.commbuf, &flag, 8, cudaMemcpyHostToDevice, S.stream));
-    comm_allreduce(S, S.commbuf, 1);
-    CK(cudaMemcpyAsync(&flag, S.commbuf, 8, cudaMemcpyDeviceToHost, S.stream));
-    CK(cudaStreamSynchronize(S.stream));
-    if (flag < (double)S.world - 0.5) S.fused_ok = false;
+    int fused_ranks = 0;
+    int rc = ranks_with(c, S, S.fused_ok, &fused_ranks);
+    if (rc) return rc;
+    if (fused_ranks < S.world) S.fused_ok = false;
   }
   return LFPSQP_OK;
 }
@@ -1379,6 +1373,11 @@ static int need_large(lfpsqp_ctx *c) {
   cudaSetDevice(c->device);
   c->large->stream = c->stream;
   std::fill(c->large->disp, c->large->disp + 8, (int64_t)0);   // every entry call starts a new dispatch record
+  return 0;
+}
+static int need_unit(lfpsqp_ctx *c) {   // need_large for the unit-level ops, which work on the unbounded problem only
+  int rc = need_large(c); if (rc) return rc;
+  if (c->large->ineq) return c->fail(LFPSQP_ERR_UNSUPPORTED, "unit-level large-n ops work on the unbounded problem (lfpsqp_ineq_op covers the bound operators)");
   return 0;
 }
 static int prep_params(lfpsqp_ctx *c, LargeState &S, const lfpsqp_params *prm) {
@@ -1431,13 +1430,10 @@ extern "C" int lfpsqp_large_set_bounds(lfpsqp_ctx *c, const double *xl_loc, cons
   if (ineq == LFPSQP_ERR_BOUNDS) return c->fail(LFPSQP_ERR_BOUNDS, "Infeasible: lower bounds cannot be greater than upper bounds");
   if (ineq < 0) return c->fail(LFPSQP_ERR_ARG, "xl and xu must both be given or both be NULL");
   if (S.world > 1) {  // optimize.jl:151 looks at ALL of xl, xu: any rank with a finite bound switches every rank
-    double flag = ineq ? 1.0 : 0.0;
-    CK(cudaMemcpyAsync(S.commbuf, &flag, 8, cudaMemcpyHostToDevice, S.stream));
-    comm_allreduce(S, S.commbuf, 1);
-    CK(cudaMemcpyAsync(&flag, S.commbuf, 8, cudaMemcpyDeviceToHost, S.stream));
-    CK(cudaStreamSynchronize(S.stream));
-    if (flag > 0 && !ineq) bnd.assign(5 * nl, 0.0);   // this shard: all lines (q = r = s = t = 0)
-    ineq = flag > 0;
+    int bounded_ranks = 0;
+    if ((rc = ranks_with(c, S, ineq != 0, &bounded_ranks))) return rc;
+    if (bounded_ranks > 0 && !ineq) bnd.assign(5 * nl, 0.0);   // this shard: all lines (q = r = s = t = 0)
+    ineq = bounded_ranks > 0;
   }
   S.ineq = ineq != 0;
   S.nv = S.ineq ? 2 * nl : nl;
@@ -1490,24 +1486,15 @@ extern "C" int lfpsqp_solve_host(lfpsqp_ctx *c, const lfpsqp_host_callbacks *cb,
 // Unit-level: factorisation of the Jacobian at x (ksvd! replacement) -- G = J J' (lower), L, L^-1 returned to the host
 extern "C" int lfpsqp_large_factor(lfpsqp_ctx *c, const double *x_loc, double *G_out, double *L_out, double *Linv_out,
                                    int *rank_deficient, double *gram_ms) {
-  int rc = need_large(c); if (rc) return rc;
+  int rc = need_unit(c); if (rc) return rc;
   LargeState &S = *c->large;
-  if (S.ineq) return c->fail(LFPSQP_ERR_UNSUPPORTED, "unit-level large-n ops work on the unbounded problem (lfpsqp_ineq_op covers the bound operators)");
   lfpsqp_params p; lfpsqp_default_params(&p); S.prm = p;
   const int m = S.m; const size_t ldm = S.ldm;
   CK(cudaMemcpyAsync(S.x, x_loc, S.n_loc * 8, cudaMemcpyHostToDevice, S.stream));
-  memset(S.hctrl, 0, sizeof(LargeCtrl)); write_ctrl_fields(S);
+  reset_ctrl(S);
   fam_c_jac(S, true, S.cval, S.x);
-  if (G_out) {  // G before it is overwritten by L
-    if (S.csr) spj_gram(S);
-    else {
-      S.disp_syrk = true;
-      gemm_nt(S, m, m, (int)S.n_loc, S.J, S.ldj, S.J, S.ldj, S.G, ldm, GEMM_ASSIGN, 1);
-      S.disp_syrk = false;
-    }
-    if (S.world > 1) comm_allreduce(S, S.G, (size_t)m * ldm);
-    CK(cudaMemcpy2DAsync(G_out, m * 8, S.G, ldm * 8, m * 8, m, cudaMemcpyDeviceToHost, S.stream));
-  }
+  gram(S, true);
+  if (G_out) CK(cudaMemcpy2DAsync(G_out, m * 8, S.G, ldm * 8, m * 8, m, cudaMemcpyDeviceToHost, S.stream));   // before L overwrites it
   S.prefer_pinv = false;
   factorize(c, S);
   if (read_ctrl(c, S)) return LFPSQP_ERR_CUDA;
@@ -1530,9 +1517,8 @@ extern "C" int lfpsqp_large_factor(lfpsqp_ctx *c, const double *x_loc, double *G
 // Unit-level: tangent projection v - J'(J J')^-1 J v with the factor cached by lfpsqp_large_factor (kgemv! pair,
 // optimize.jl:306-307) and the multipliers (J J')^-1 J v (optimize.jl:333-343)
 extern "C" int lfpsqp_large_project(lfpsqp_ctx *c, const double *v_loc, double *v_out_loc, double *lambda_out) {
-  int rc = need_large(c); if (rc) return rc;
+  int rc = need_unit(c); if (rc) return rc;
   LargeState &S = *c->large;
-  if (S.ineq) return c->fail(LFPSQP_ERR_UNSUPPORTED, "unit-level large-n ops work on the unbounded problem (lfpsqp_ineq_op covers the bound operators)");
   CK(cudaMemcpyAsync(S.d, v_loc, S.n_loc * 8, cudaMemcpyHostToDevice, S.stream));
   project(S, S.d, S.lam, 0, 0);
   CK(cudaMemcpyAsync(v_out_loc, S.d, S.n_loc * 8, cudaMemcpyDeviceToHost, S.stream));
@@ -1546,14 +1532,13 @@ extern "C" int lfpsqp_large_project(lfpsqp_ctx *c, const double *v_loc, double *
 // "projcg iterations / s" metric).  Needs lfpsqp_large_factor at the same x first.  ms = device time of the loop.
 extern "C" int lfpsqp_large_projcg(lfpsqp_ctx *c, const double *x_loc, const double *lam, double tol, int64_t maxit,
                                    int chunk, double *sol_out_loc, int64_t *iters, double *nr, int *status, double *ms) {
-  int rc = need_large(c); if (rc) return rc;
+  int rc = need_unit(c); if (rc) return rc;
   LargeState &S = *c->large;
-  if (S.ineq) return c->fail(LFPSQP_ERR_UNSUPPORTED, "unit-level large-n ops work on the unbounded problem (lfpsqp_ineq_op covers the bound operators)");
   const int64_t n = S.n_loc;
   double *g = S.g, *d = S.d;
   CK(cudaMemcpyAsync(S.x, x_loc, n * 8, cudaMemcpyHostToDevice, S.stream));
   if (S.m > 0) { if (lam) CK(cudaMemcpyAsync(S.lam, lam, S.m * 8, cudaMemcpyHostToDevice, S.stream)); else cudaMemsetAsync(S.lam, 0, S.m * 8, S.stream); }
-  memset(S.hctrl, 0, sizeof(LargeCtrl)); write_ctrl_fields(S);
+  reset_ctrl(S);
   fam_grad(S, g, S.x);
   vec(S, n, [=] __device__(int64_t i, double *) { d[i] = -1.0 * g[i]; });
   if (S.m > 0) project(S, d, nullptr, 0, 0);
@@ -1579,16 +1564,15 @@ extern "C" int lfpsqp_large_projcg(lfpsqp_ctx *c, const double *x_loc, const dou
 extern "C" int lfpsqp_large_projcg_general(lfpsqp_ctx *c, const double *x_loc, const double *lam, const double *b_loc,
                                            const double *cvec, double tol, int64_t maxit, double *sol_out_loc,
                                            double *lambda_out, int64_t *iters, double *nr, int *status) {
-  int rc = need_large(c); if (rc) return rc;
+  int rc = need_unit(c); if (rc) return rc;
   LargeState &S = *c->large;
-  if (S.ineq) return c->fail(LFPSQP_ERR_UNSUPPORTED, "unit-level large-n ops work on the unbounded problem (lfpsqp_ineq_op covers the bound operators)");
   if (!x_loc || !b_loc) return c->fail(LFPSQP_ERR_ARG, "x and b are required");
   const int64_t n = S.n_loc;
   CK(cudaMemcpyAsync(S.x, x_loc, n * 8, cudaMemcpyHostToDevice, S.stream));
   CK(cudaMemcpyAsync(S.d, b_loc, n * 8, cudaMemcpyHostToDevice, S.stream));
   if (S.m > 0) { if (lam) CK(cudaMemcpyAsync(S.lam, lam, S.m * 8, cudaMemcpyHostToDevice, S.stream)); else cudaMemsetAsync(S.lam, 0, S.m * 8, S.stream); }
   if (S.m > 0 && cvec) CK(cudaMemcpyAsync(S.nr_t1, cvec, S.m * 8, cudaMemcpyHostToDevice, S.stream));
-  memset(S.hctrl, 0, sizeof(LargeCtrl)); write_ctrl_fields(S);
+  reset_ctrl(S);
   fam_hess_prepare(S, S.x, S.lam);
   S.reset_counters();
   if (projcg(c, S, tol, maxit, S.cg_chunk, (S.m > 0 && cvec) ? S.nr_t1 : nullptr, (S.m > 0 && lambda_out) ? S.nr_t2 : nullptr)) return LFPSQP_ERR_CUDA;
@@ -1608,18 +1592,18 @@ extern "C" int lfpsqp_large_projcg_general(lfpsqp_ctx *c, const double *x_loc, c
 extern "C" int lfpsqp_large_retract(lfpsqp_ctx *c, int method, const double *x_base_loc, const double *xtilde_loc,
                                     const lfpsqp_params *prm, double *xnew_out_loc, double *cval_out, int *flag,
                                     int64_t *iters, int64_t *pcg_iters) {
-  int rc = need_large(c); if (rc) return rc;
+  int rc = need_unit(c); if (rc) return rc;
   LargeState &S = *c->large;
-  if (S.ineq) return c->fail(LFPSQP_ERR_UNSUPPORTED, "unit-level large-n ops work on the unbounded problem (lfpsqp_ineq_op covers the bound operators)");
   lfpsqp_params p2 = *prm; p2.do_project_retract = (method == 0) ? 0 : 1;
   rc = prep_params(c, S, &p2); if (rc) return rc;
   if (S.m < 1) return c->fail(LFPSQP_ERR_ARG, "retraction needs m > 0");
   const int64_t n = S.n_loc;
   CK(cudaMemcpyAsync(S.x, x_base_loc, n * 8, cudaMemcpyHostToDevice, S.stream));
   CK(cudaMemcpyAsync(S.xtil, xtilde_loc, n * 8, cudaMemcpyHostToDevice, S.stream));
-  memset(S.hctrl, 0, sizeof(LargeCtrl)); write_ctrl_fields(S);
+  reset_ctrl(S);
   S.reset_counters();
   fam_c_jac(S, true, S.cval, S.x);
+  gram(S, true);
   if (factorize(c, S)) return LFPSQP_ERR_CUDA;
   int fl = 0, i1 = 0, i2 = 0;
   if (method == 0) { if (retract_nr(c, S, &fl, &i1)) return LFPSQP_ERR_CUDA; }
@@ -1636,15 +1620,14 @@ extern "C" int lfpsqp_large_retract(lfpsqp_ctx *c, int method, const double *x_b
 // x = 0, r = b.  Outputs the solution, the final residual, flag (1 iff iters == maxiter) and the iteration count.
 extern "C" int lfpsqp_large_pcg(lfpsqp_ctx *c, const double *x_point_loc, double mu, const double *b_loc, double tol,
                                 int64_t maxiter, double *x_out_loc, double *r_out_loc, int *flag, int64_t *iters) {
-  int rc = need_large(c); if (rc) return rc;
+  int rc = need_unit(c); if (rc) return rc;
   LargeState &S = *c->large;
-  if (S.ineq) return c->fail(LFPSQP_ERR_UNSUPPORTED, "unit-level large-n ops work on the unbounded problem (lfpsqp_ineq_op covers the bound operators)");
   if (S.m < 1) return c->fail(LFPSQP_ERR_ARG, "pcg needs m > 0");
   const int64_t n = S.n_loc;
   double *r = S.w0, *pv = S.w1, *dx = S.w3, *lp = S.lp;
   CK(cudaMemcpyAsync(S.x, x_point_loc, n * 8, cudaMemcpyHostToDevice, S.stream));
   CK(cudaMemcpyAsync(r, b_loc, n * 8, cudaMemcpyHostToDevice, S.stream));
-  memset(S.hctrl, 0, sizeof(LargeCtrl)); write_ctrl_fields(S);
+  reset_ctrl(S);
   S.reset_counters();
   fam_c_jac(S, true, S.cval, S.x);
   pcg_start_kernel<<<S.vgrid, 256, 0, S.stream>>>(n, r, dx, pv, lp);

@@ -69,8 +69,7 @@ __global__ void __launch_bounds__(256) ineq_proj_pre_kernel(IneqDev I, const dou
 // the elementwise tail of the projection: (ox, oy) = v - Q Q' v given w_j = sum_rs cpart[rs][j]
 __device__ __forceinline__ void ineq_proj_tail(const IneqDev &I, int64_t j, double vx, double vy, const double *cpart, int nsplit,
                                                double &ox, double &oy, double &aa, double &wj) {
-  double s = 0.0;
-  for (int k = 0; k < nsplit; k++) s += cpart[(int64_t)k * I.nx + j];
+  const double s = split_sum(cpart, nsplit, I.nx, j);
   const double dx = I.Dx[j], dy = I.Dy[j];
   aa = dx * vx + dy * vy; wj = s;
   ox = vx - (dx * aa + dy * dy * s);
@@ -137,8 +136,7 @@ __global__ void __launch_bounds__(256) ineq_pp_rhs_kernel(IneqDev I, double *__r
   const int64_t nx = I.nx;
   double a = 0.0;
   for (int64_t j = (int64_t)blockIdx.x * 256 + threadIdx.x; j < nx; j += (int64_t)gridDim.x * 256) {
-    double s = 0.0;
-    for (int k = 0; k < nsplit; k++) s += cpart[(int64_t)k * nx + j];
+    const double s = split_sum(cpart, nsplit, nx, j);
     const double sw = I.S[j] * cvh[j];
     const double gx = (s + I.Dx[j] * sw) + mu * g[j];
     const double gy = mu * g[nx + j] + I.Dy[j] * sw;
@@ -159,8 +157,7 @@ __global__ void __launch_bounds__(256) ineq_pcg_z_kernel(IneqDev I, double *__re
   const double mu = ctrl->mu;
   double a = 0.0;
   for (int64_t j = (int64_t)blockIdx.x * 256 + threadIdx.x; j < nx; j += (int64_t)gridDim.x * 256) {
-    double s = 0.0;
-    for (int k = 0; k < nsplit; k++) s += cpart[(int64_t)k * nx + j];
+    const double s = split_sum(cpart, nsplit, nx, j);
     const double px = p[j], py = p[nx + j], Sj = I.S[j], dxj = I.Dx[j], dyj = I.Dy[j];
     const double th = Sj * (dxj * px + dyj * py), sw = Sj * th;
     const double zx = (s + dxj * sw) + mu * px, zy = mu * py + dyj * sw;

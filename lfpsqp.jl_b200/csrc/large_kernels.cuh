@@ -115,6 +115,11 @@ __global__ void __launch_bounds__(256) cols_dot_kernel(const double *__restrict_
     cpart[(int64_t)rs * ncols + c] = a0;
   }
 }
+// entry j of J'u from the row splits a column pass left in cpart (row pitch ld): s + cpart[0][j] + cpart[1][j] + ..., in that order
+__device__ __forceinline__ double split_sum(const double *cpart, int nsplit, int64_t ld, int64_t j, double s = 0.0) {
+  for (int k = 0; k < nsplit; k++) s += cpart[(int64_t)k * ld + j];
+  return s;
+}
 
 // ------------------------------------------------------------------ triangular GEMVs: out[i] = sum_k T[i][k] in[k]
 // lower: k <= i ; upper: k >= i.  One warp per row; `in` staged in shared memory.
@@ -256,8 +261,7 @@ __global__ void __launch_bounds__(256) cg_update2_kernel(int64_t n, const double
   __shared__ double sh[33];
   double a = 0.0, b = 0.0;
   for (int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x; i < n; i += (int64_t)gridDim.x * 256) {
-    double s = 0.0;
-    for (int k = 0; k < nsplit; k++) s += cpart[(int64_t)k * n + i];
+    const double s = split_sum(cpart, nsplit, n, i);
     double rpi = rp[i], g = rpi - s;
     gp[i] = g; a += rpi * g; b += g * g;
   }
@@ -291,8 +295,7 @@ __global__ void __launch_bounds__(256) cg_init_kernel(int64_t n, double *__restr
   __shared__ double sh[33];
   double a = 0.0;
   for (int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x; i < n; i += (int64_t)gridDim.x * 256) {
-    double s = 0.0;
-    for (int k = 0; k < nsplit; k++) s += cpart[(int64_t)k * n + i];
+    const double s = split_sum(cpart, nsplit, n, i);
     double g = r[i] - s;
     r[i] = g; d[i] = -1.0 * g; a += g * g;
   }
@@ -320,9 +323,7 @@ __global__ void __launch_bounds__(256) pp_rhs_kernel(int64_t n, double *__restri
   __shared__ double sh[33];
   double a = 0.0;
   for (int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x; i < n; i += (int64_t)gridDim.x * 256) {
-    double s = 0.0;
-    for (int k = 0; k < nsplit; k++) s += cpart[(int64_t)k * n + i];
-    double gi = s + mu * g[i];
+    double gi = split_sum(cpart, nsplit, n, i) + mu * g[i];
     g[i] = gi; dx[i] = 0.0; r[i] = gi; p[i] = 0.0; a += gi * gi;
   }
   a = block_sum(a, sh);
@@ -368,8 +369,7 @@ __global__ void __launch_bounds__(256) pcg_z_kernel(int64_t n, double *__restric
   const double mu = ctrl->mu;
   double a = 0.0;
   for (int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x; i < n; i += (int64_t)gridDim.x * 256) {
-    double s = 0.0;
-    for (int k = 0; k < nsplit; k++) s += cpart[(int64_t)k * n + i];
+    const double s = split_sum(cpart, nsplit, n, i);
     double pi = p[i], zi = s + mu * pi;
     z[i] = zi; a += pi * zi;
   }

@@ -35,7 +35,8 @@ struct LargeState {
   double *Ginv = nullptr;                  // explicit G^-1 = L^-T L^-1 (m x m, symmetric) for the one-phase solve of the fused kernel
   // explicit-inverse guard: u = G^-1 t loses cond(G) eps, two triangular solves only cond(L) eps.  factorize() bounds cond(G)
   // from above by kappa = trace(G) * lambda_max(G^-1) (power iterations on the explicit inverse); above `inverse_guard` the
-  // fused kernel runs the two triangular phases instead (LFPSQP_EXPLICIT_INVERSE=0/1 forces either path: tests)
+  // fused kernel runs the two triangular phases instead.  force_inverse: LFPSQP_EXPLICIT_INVERSE=0/1 at setup forces either path
+  // (tests), -1 leaves the choice to the guard
   // rank-deficient Jacobians (large_eig.cu): after a failed Cholesky pivot test the solves use the truncated pseudo-inverse
   // G^+ (held in Ginv) of the eigen-decomposed Gram; rank_cur feeds projcg's iteration cap and the NR / ProjPenalty choice
   bool pinv_active = false, prefer_pinv = false;
@@ -44,6 +45,7 @@ struct LargeState {
   unsigned long long *eigScratch = nullptr;    // [32] convergence per sweep | barrier counter | sweeps done
   double *noise_dev = nullptr; size_t noise_cap = 0; int64_t noise_T = 0;   // caller-supplied noise rows (lfpsqp_ctx_set_noise), beta > 0
   bool explicit_inverse_ok = true, guard_pending = false;
+  int force_inverse = -1;
   double inverse_guard = 1e6, pivot_ratio2 = 1.0;   // pivot_ratio2: the last kappa
   int m = 0, sm_count = 148, world = 1, rank = 0;
   cudaStream_t stream = nullptr;
@@ -61,8 +63,10 @@ struct LargeState {
   // g_blockdiag: the previous factorisation found G block diagonal (every diagonal block independent) -> the next one reads the
   // count back right after the parallel diagonal factorisation and, if it is still 0, enqueues neither the Cholesky chain nor the
   // inverse's GEMM levels (hundreds of launches that would all return at once)
+  // gram_skip: structure detection (zero-slab map, block flags) is on; LFPSQP_GRAM_SKIP=0 at setup turns it off (tests compare
+  // against the plain dense path bit for bit)
   int g_blockdiag = 0;
-  bool gdep_pending = false;
+  bool gdep_pending = false, gram_skip = true;
   int *invflag = nullptr;      // [nblk][nblk] block structure of L^-1 (scanned after the inverse) for the triangular passes; null: off
   bool invflag_valid = false;
   int *blkflag = nullptr;      // [nblk][nblk] block structure of G / L for the factorisation (large_gemm.cuh::GemmExt::bf)
