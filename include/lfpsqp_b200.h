@@ -252,7 +252,13 @@ int lfpsqp_solve_host(lfpsqp_ctx *ctx, const lfpsqp_host_callbacks *cb, int64_t 
  *             following project / projcg calls use the truncated pseudo-inverse, optimize.jl:297-302)
  *   project : v - J'(J J')^-1 J v and lambda = (J J')^-1 J v with the cached factor                    [kgemv! x2, optimize.jl:306-307, :333-343]
  *   projcg  : projcg! (src/projcg.jl:40-121) at x with multipliers lam on b = P(-grad f(x)), c = 0; status:
- *             1 converged, 2 negative curvature, 3 rg<=0, 4 iteration limit; ms = device time of the loop */
+ *             1 converged, 2 negative curvature, 3 rg<=0, 4 iteration limit; ms = device time of the loop
+ * With bounds set (lfpsqp_large_set_bounds) these calls and lfpsqp_large_retract / lfpsqp_large_pcg work on the 2n embedding
+ * (src/inequality_helper.jl): x, v, b, x_base, xtilde and every vector output have the working length 2 n_loc, laid out
+ * [x-half | y-half]; factor returns the weighted Gram G_w = J diag(Dy^2) J' at x; project writes m + n_loc multipliers
+ * [lambda ; lambda_y]; projcg takes lam in that layout and applies the augmented Hessian (:144-158); pcg's operator is
+ * bigA bigA' + mu I at x_point.  projcg_general is LFPSQP_ERR_UNSUPPORTED with bounds, and so are all of these calls on
+ * a column-sharded problem with bounds.  lfpsqp_large_working_length gives the working length. */
 int lfpsqp_large_factor(lfpsqp_ctx *ctx, const double *x_loc, double *G_out, double *L_out, double *Linv_out,
                         int *rank_deficient, double *gram_ms);
 int lfpsqp_large_project(lfpsqp_ctx *ctx, const double *v_loc, double *v_out_loc, double *lambda_out);
@@ -293,6 +299,8 @@ int lfpsqp_large_phase_ms(lfpsqp_ctx *ctx, double *out4);
  *   [7] mask of the forms the Gram solves took: 1 explicit inverse, 2 triangular solves, 4 truncated pseudo-inverse
  * LFPSQP_ERR_ARG before lfpsqp_large_setup. */
 int lfpsqp_large_last_dispatch(lfpsqp_ctx *ctx, int64_t *out8);
+/* length of this rank's working vectors of the bound problem: n_loc, or 2 n_loc with the bound embedding switched on */
+int lfpsqp_large_working_length(lfpsqp_ctx *ctx, int64_t *nv);
 
 /* Unit-level bound embedding (src/inequality_helper.jl; y_retract! src/retractions.jl:451-500) on one instance; runs the
  * device code of the batched solver.  J: m x n row-major (== Jct column-major), may be NULL when m = 0.

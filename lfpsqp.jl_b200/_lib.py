@@ -51,7 +51,7 @@ EXPORTS = [
     "lfpsqp_ineq_op", "lfpsqp_large_phase_ms", "lfpsqp_comm_ipc_export", "lfpsqp_comm_ipc_import", "lfpsqp_comm_mode",
     "lfpsqp_large_set_bounds", "lfpsqp_solve_host", "lfpsqp_linesearch", "lfpsqp_aug_hess_vec", "lfpsqp_large_projcg_general",
     "lfpsqp_ctx_create_multi", "lfpsqp_ctx_device_count", "lfpsqp_ctx_set_noise", "lfpsqp_last_kernel",
-    "lfpsqp_large_last_dispatch",
+    "lfpsqp_large_last_dispatch", "lfpsqp_large_working_length",
 ]
 
 _lib = None
@@ -99,6 +99,7 @@ def load():
         lib.lfpsqp_ineq_op.argtypes = [P, C.c_int, I, I, P, P, P, P, I, P, I]
         lib.lfpsqp_large_phase_ms.argtypes = [P, P]
         lib.lfpsqp_large_last_dispatch.argtypes = [P, C.POINTER(C.c_int64)]
+        lib.lfpsqp_large_working_length.argtypes = [P, C.POINTER(C.c_int64)]
         lib.lfpsqp_comm_ipc_export.argtypes = [P, P]
         lib.lfpsqp_comm_ipc_import.argtypes = [P, P]
         lib.lfpsqp_comm_mode.argtypes = [P]

@@ -1375,9 +1375,11 @@ static int need_large(lfpsqp_ctx *c) {
   std::fill(c->large->disp, c->large->disp + 8, (int64_t)0);   // every entry call starts a new dispatch record
   return 0;
 }
-static int need_unit(lfpsqp_ctx *c) {   // need_large for the unit-level ops, which work on the unbounded problem only
+// need_large for the unit-level ops: with bounds they work on one GPU only (a column shard's embedding rows are not exchanged)
+static int need_unit(lfpsqp_ctx *c) {
   int rc = need_large(c); if (rc) return rc;
-  if (c->large->ineq) return c->fail(LFPSQP_ERR_UNSUPPORTED, "unit-level large-n ops work on the unbounded problem (lfpsqp_ineq_op covers the bound operators)");
+  if (c->large->ineq && c->large->world > 1)
+    return c->fail(LFPSQP_ERR_UNSUPPORTED, "unit-level large-n ops with bounds run on one GPU (this problem is column-sharded)");
   return 0;
 }
 static int prep_params(lfpsqp_ctx *c, LargeState &S, const lfpsqp_params *prm) {
@@ -1483,15 +1485,23 @@ extern "C" int lfpsqp_solve_host(lfpsqp_ctx *c, const lfpsqp_host_callbacks *cb,
                             term, stats);
 }
 
-// Unit-level: factorisation of the Jacobian at x (ksvd! replacement) -- G = J J' (lower), L, L^-1 returned to the host
+// Unit-level: factorisation of the Jacobian at x (ksvd! replacement) -- G = J J' (lower), L, L^-1 returned to the host.
+// With bounds x is the working point [x | y] (2 n_loc entries) and G is the weighted G_w = J diag(Dy^2) J' of that point.
 extern "C" int lfpsqp_large_factor(lfpsqp_ctx *c, const double *x_loc, double *G_out, double *L_out, double *Linv_out,
                                    int *rank_deficient, double *gram_ms) {
   int rc = need_unit(c); if (rc) return rc;
   LargeState &S = *c->large;
   lfpsqp_params p; lfpsqp_default_params(&p); S.prm = p;
   const int m = S.m; const size_t ldm = S.ldm;
-  CK(cudaMemcpyAsync(S.x, x_loc, S.n_loc * 8, cudaMemcpyHostToDevice, S.stream));
+  CK(cudaMemcpyAsync(S.x, x_loc, S.nv * 8, cudaMemcpyHostToDevice, S.stream));
   reset_ctrl(S);
+  if (S.ineq) ineq_gradient(S, S.x);   // Dx, Dy, S of the point: the weights of G_w and the bound part of the projector (:277)
+  if (m < 1) {   // nothing to factorise; with bounds the projector is the bound part alone
+    CK(cudaStreamSynchronize(S.stream));
+    if (rank_deficient) *rank_deficient = 0;
+    if (gram_ms) *gram_ms = 0.0;
+    return LFPSQP_OK;
+  }
   fam_c_jac(S, true, S.cval, S.x);
   gram(S, true);
   if (G_out) CK(cudaMemcpy2DAsync(G_out, m * 8, S.G, ldm * 8, m * 8, m, cudaMemcpyDeviceToHost, S.stream));   // before L overwrites it
@@ -1515,14 +1525,17 @@ extern "C" int lfpsqp_large_factor(lfpsqp_ctx *c, const double *x_loc, double *G
 }
 
 // Unit-level: tangent projection v - J'(J J')^-1 J v with the factor cached by lfpsqp_large_factor (kgemv! pair,
-// optimize.jl:306-307) and the multipliers (J J')^-1 J v (optimize.jl:333-343)
+// optimize.jl:306-307) and the multipliers (J J')^-1 J v (optimize.jl:333-343).  With bounds v is a working vector
+// (2 n_loc entries), the projector is the one of the 2n embedding at the factorised point and lambda_out receives
+// [lambda (m) ; lambda_y (n_loc)] (calculate_lambda_kkt!, inequality_helper.jl:286-308).
 extern "C" int lfpsqp_large_project(lfpsqp_ctx *c, const double *v_loc, double *v_out_loc, double *lambda_out) {
   int rc = need_unit(c); if (rc) return rc;
   LargeState &S = *c->large;
-  CK(cudaMemcpyAsync(S.d, v_loc, S.n_loc * 8, cudaMemcpyHostToDevice, S.stream));
-  project(S, S.d, S.lam, 0, 0);
-  CK(cudaMemcpyAsync(v_out_loc, S.d, S.n_loc * 8, cudaMemcpyDeviceToHost, S.stream));
+  CK(cudaMemcpyAsync(S.d, v_loc, S.nv * 8, cudaMemcpyHostToDevice, S.stream));
+  project(S, S.d, S.lam, 0, 0, /*want_mult=*/1);
+  CK(cudaMemcpyAsync(v_out_loc, S.d, S.nv * 8, cudaMemcpyDeviceToHost, S.stream));
   if (lambda_out && S.m > 0) CK(cudaMemcpyAsync(lambda_out, S.lam, S.m * 8, cudaMemcpyDeviceToHost, S.stream));
+  if (lambda_out && S.ineq) CK(cudaMemcpyAsync(lambda_out + S.m, S.I.lamy, S.n_loc * 8, cudaMemcpyDeviceToHost, S.stream));
   CK(cudaStreamSynchronize(S.stream));
   return LFPSQP_OK;
 }
@@ -1530,18 +1543,26 @@ extern "C" int lfpsqp_large_project(lfpsqp_ctx *c, const double *v_loc, double *
 // Unit-level + benchmark: projcg! (projcg.jl:40-121) at the point x with multipliers lam, right-hand side b = P(-grad f(x)),
 // tolerance tol, at most maxit iterations (tol = 0 with maxit = K times a fixed number of iterations: the
 // "projcg iterations / s" metric).  Needs lfpsqp_large_factor at the same x first.  ms = device time of the loop.
+// With bounds x and the solution are working vectors (2 n_loc entries), lam is [lambda (m) ; lambda_y (n_loc)] and the
+// Hessian is the augmented one of inequality_helper.jl:144-158.
 extern "C" int lfpsqp_large_projcg(lfpsqp_ctx *c, const double *x_loc, const double *lam, double tol, int64_t maxit,
                                    int chunk, double *sol_out_loc, int64_t *iters, double *nr, int *status, double *ms) {
   int rc = need_unit(c); if (rc) return rc;
   LargeState &S = *c->large;
-  const int64_t n = S.n_loc;
+  const int64_t n = S.nv;
   double *g = S.g, *d = S.d;
   CK(cudaMemcpyAsync(S.x, x_loc, n * 8, cudaMemcpyHostToDevice, S.stream));
   if (S.m > 0) { if (lam) CK(cudaMemcpyAsync(S.lam, lam, S.m * 8, cudaMemcpyHostToDevice, S.stream)); else cudaMemsetAsync(S.lam, 0, S.m * 8, S.stream); }
+  if (S.ineq) {   // lambda_y of the Hessian; g has a zero y-half (optimize.jl:191)
+    if (lam) CK(cudaMemcpyAsync(S.I.lamy, lam + S.m, S.n_loc * 8, cudaMemcpyHostToDevice, S.stream));
+    else CK(cudaMemsetAsync(S.I.lamy, 0, S.n_loc * 8, S.stream));
+    CK(cudaMemsetAsync(g + S.n_loc, 0, S.n_loc * 8, S.stream));
+  }
   reset_ctrl(S);
+  if (S.ineq) ineq_gradient(S, S.x);
   fam_grad(S, g, S.x);
   vec(S, n, [=] __device__(int64_t i, double *) { d[i] = -1.0 * g[i]; });
-  if (S.m > 0) project(S, d, nullptr, 0, 0);
+  if (S.m > 0 || S.ineq) project(S, d, nullptr, 0, 0);
   fam_hess_prepare(S, S.x, S.lam);
   S.reset_counters();
   cudaEventRecord(c->ev0, S.stream);
@@ -1566,6 +1587,7 @@ extern "C" int lfpsqp_large_projcg_general(lfpsqp_ctx *c, const double *x_loc, c
                                            double *lambda_out, int64_t *iters, double *nr, int *status) {
   int rc = need_unit(c); if (rc) return rc;
   LargeState &S = *c->large;
+  if (S.ineq) return c->fail(LFPSQP_ERR_UNSUPPORTED, "projcg_general works on the unbounded problem: its start x0 = U c and its multipliers U'(b - A x) have no bound-embedding form here");
   if (!x_loc || !b_loc) return c->fail(LFPSQP_ERR_ARG, "x and b are required");
   const int64_t n = S.n_loc;
   CK(cudaMemcpyAsync(S.x, x_loc, n * 8, cudaMemcpyHostToDevice, S.stream));
@@ -1588,7 +1610,9 @@ extern "C" int lfpsqp_large_projcg_general(lfpsqp_ctx *c, const double *x_loc, c
 }
 
 // Unit-level: retract!(cval, xnew, c!, xtilde, x, method) (src/retractions.jl:75-177 NR / :265-441 ProjPenalty) with the
-// factorisation taken at x_base (as armijo! calls it, linesearch.jl:52).  method: 0 = NR, 1 = ProjPenalty.
+// factorisation taken at x_base (as armijo! calls it, linesearch.jl:52).  method: 0 = NR, 1 = ProjPenalty.  With bounds
+// x_base, xtilde and xnew are working points [x | y] (2 n_loc entries), and the c-part of ProjPenalty's merit vector
+// starts at zero, as at the start of a solve.
 extern "C" int lfpsqp_large_retract(lfpsqp_ctx *c, int method, const double *x_base_loc, const double *xtilde_loc,
                                     const lfpsqp_params *prm, double *xnew_out_loc, double *cval_out, int *flag,
                                     int64_t *iters, int64_t *pcg_iters) {
@@ -1597,11 +1621,13 @@ extern "C" int lfpsqp_large_retract(lfpsqp_ctx *c, int method, const double *x_b
   lfpsqp_params p2 = *prm; p2.do_project_retract = (method == 0) ? 0 : 1;
   rc = prep_params(c, S, &p2); if (rc) return rc;
   if (S.m < 1) return c->fail(LFPSQP_ERR_ARG, "retraction needs m > 0");
-  const int64_t n = S.n_loc;
+  const int64_t n = S.nv;
   CK(cudaMemcpyAsync(S.x, x_base_loc, n * 8, cudaMemcpyHostToDevice, S.stream));
   CK(cudaMemcpyAsync(S.xtil, xtilde_loc, n * 8, cudaMemcpyHostToDevice, S.stream));
+  if (S.ineq) CK(cudaMemsetAsync(S.cvc, 0, S.m * 8, S.stream));
   reset_ctrl(S);
   S.reset_counters();
+  if (S.ineq) ineq_gradient(S, S.x);
   fam_c_jac(S, true, S.cval, S.x);
   gram(S, true);
   if (factorize(c, S)) return LFPSQP_ERR_CUDA;
@@ -1617,18 +1643,20 @@ extern "C" int lfpsqp_large_retract(lfpsqp_ctx *c, int method, const double *x_b
 }
 
 // Unit-level: pcg!(mu, J, no_precondition, x, r, p, z, tmp_m, tol, maxiter) (src/retractions.jl:179-246) with J = jac(x_point),
-// x = 0, r = b.  Outputs the solution, the final residual, flag (1 iff iters == maxiter) and the iteration count.
+// x = 0, r = b.  Outputs the solution, the final residual, flag (1 iff iters == maxiter) and the iteration count.  With
+// bounds x_point, b and the outputs are working vectors (2 n_loc entries) and the operator is bigA bigA' + mu I at x_point.
 extern "C" int lfpsqp_large_pcg(lfpsqp_ctx *c, const double *x_point_loc, double mu, const double *b_loc, double tol,
                                 int64_t maxiter, double *x_out_loc, double *r_out_loc, int *flag, int64_t *iters) {
   int rc = need_unit(c); if (rc) return rc;
   LargeState &S = *c->large;
   if (S.m < 1) return c->fail(LFPSQP_ERR_ARG, "pcg needs m > 0");
-  const int64_t n = S.n_loc;
+  const int64_t n = S.nv;
   double *r = S.w0, *pv = S.w1, *dx = S.w3, *lp = S.lp;
   CK(cudaMemcpyAsync(S.x, x_point_loc, n * 8, cudaMemcpyHostToDevice, S.stream));
   CK(cudaMemcpyAsync(r, b_loc, n * 8, cudaMemcpyHostToDevice, S.stream));
   reset_ctrl(S);
   S.reset_counters();
+  if (S.ineq) ineq_gradient(S, S.x);   // Dx, Dy, S of bigA at x_point
   fam_c_jac(S, true, S.cval, S.x);
   pcg_start_kernel<<<S.vgrid, 256, 0, S.stream>>>(n, r, dx, pv, lp);
   cudaEventRecord(c->ev0, S.stream);
@@ -1641,6 +1669,13 @@ extern "C" int lfpsqp_large_pcg(lfpsqp_ctx *c, const double *x_point_loc, double
   if (flag) *flag = (S.hctrl->pcg_iter == maxiter) ? 1 : 0;
   { float ms = 0; cudaEventElapsedTime(&ms, c->ev0, c->ev1); c->last_ms = ms; }   // device time of the pcg! loop (lfpsqp_last_kernel_ms)
   c->last_launches = S.launches;
+  return LFPSQP_OK;
+}
+
+// length of this rank's working vectors: n_loc, or 2 n_loc once lfpsqp_large_set_bounds has switched the embedding on
+extern "C" int lfpsqp_large_working_length(lfpsqp_ctx *c, int64_t *nv) {
+  if (!c || !c->large || !nv) return LFPSQP_ERR_ARG;
+  *nv = c->large->nv;
   return LFPSQP_OK;
 }
 

@@ -11,7 +11,12 @@ _SPARSE = (SPARSE_QCQP, SPARSE_QCQP_CSR)
 
 
 class LargeProblem:
-    """Binds one (sharded) problem to a Context: lfpsqp_large_setup, then solve / factor / project / projcg."""
+    """Binds one (sharded) problem to a Context: lfpsqp_large_setup, then solve / factor / project / projcg.
+
+    Without bounds the working vectors of the unit-level calls (factor, project, projcg, pcg, retract) are this rank's n_loc
+    entries of x.  With finite bounds (set_bounds) they are the 2 n_loc entries [x | y] of the embedding of
+    src/inequality_helper.jl: factor returns the weighted Gram G_w = J diag(Dy^2) J' at that point, project returns the
+    multipliers [lambda ; lambda_y] (m + n_loc entries), and projcg takes them in the same layout."""
 
     def __init__(self, fam, ctx=None, col0=0, n_loc=None, n_global=None, params_dev_ptr=None):
         self.ctx = ctx or _lib.default_context()
@@ -37,6 +42,22 @@ class LargeProblem:
         if xl is not None and xu is not None and not (len(xl) == len(xu) == self.n_loc):
             raise _lib.LFPSQPError("xl, xu, and x0 must all be the same length")     # optimize.jl:144-148
         self.ctx.check(self.ctx.lib.lfpsqp_large_set_bounds(self.ctx.h, _lib.ptr(xl), _lib.ptr(xu)))
+
+    @property
+    def nv(self):
+        """working length of the unit-level calls as the library holds it: n_loc, or 2 n_loc with the bound embedding
+        (the library decides, after optimize.jl:151, and on every rank of a sharded problem alike)"""
+        out = C.c_int64(0)
+        self.ctx.check(self.ctx.lib.lfpsqp_large_working_length(self.ctx.h, C.byref(out)))
+        return out.value
+
+    def _working(self, v, what):
+        v = np.ascontiguousarray(v, dtype=np.float64)
+        nv = self.nv
+        if v.shape != (nv,):
+            raise _lib.LFPSQPError("%s must have the working length %d (%s), not %s"
+                                   % (what, nv, "[x | y] with bounds" if nv != self.n_loc else "n_loc", v.shape))
+        return v
 
     def solve(self, x0, param=None, history=None, return_stats=False, noise=None):
         """noise (beta > 0): (T, N_working_local) rows of the caller's randn! sequence (optimize.jl:264-273)"""
@@ -71,7 +92,7 @@ class LargeProblem:
 
     def factor(self, x, want=("G", "L", "Linv")):
         m = self.m
-        x = np.ascontiguousarray(x, dtype=np.float64)
+        x = self._working(x, "x")
         G = np.zeros((m, m)) if "G" in want else None
         L = np.zeros((m, m)) if "L" in want else None
         Li = np.zeros((m, m)) if "Linv" in want else None
@@ -81,16 +102,18 @@ class LargeProblem:
         return dict(G=G, L=L, Linv=Li, rank_deficient=rd.value, gram_ms=ms.value)
 
     def project(self, v):
-        v = np.ascontiguousarray(v, dtype=np.float64)
-        out = np.empty_like(v); lam = np.zeros(max(self.m, 1))
+        """-> (projected v, multipliers): lambda (m), or [lambda ; lambda_y] (m + n_loc) with bounds"""
+        v = self._working(v, "v")
+        nlam = self.m + (v.size - self.n_loc)
+        out = np.empty_like(v); lam = np.zeros(max(nlam, 1))
         self.ctx.check(self.ctx.lib.lfpsqp_large_project(self.ctx.h, _lib.ptr(v), _lib.ptr(out), _lib.ptr(lam)))
-        return out, lam[:self.m]
+        return out, lam[:nlam]
 
     def retract(self, method, x_base, xtilde, param=None):
         """retract! with method "nr" | "pp" -> (flag, xnew, cval, iters, pcg_iters)"""
         cp = (param or LFPSQPParams()).to_c()
-        xb = np.ascontiguousarray(x_base, dtype=np.float64); xt = np.ascontiguousarray(xtilde, dtype=np.float64)
-        xnew = np.empty(self.n_loc); cval = np.zeros(max(self.m, 1))
+        xb = self._working(x_base, "x_base"); xt = self._working(xtilde, "xtilde")
+        xnew = np.empty_like(xb); cval = np.zeros(max(self.m, 1))
         fl = C.c_int(0); it = C.c_int64(0); pit = C.c_int64(0)
         self.ctx.check(self.ctx.lib.lfpsqp_large_retract(self.ctx.h, 0 if method == "nr" else 1, _lib.ptr(xb), _lib.ptr(xt),
                                                          C.cast(C.pointer(cp), C.c_void_p), _lib.ptr(xnew), _lib.ptr(cval),
@@ -99,9 +122,9 @@ class LargeProblem:
         return fl.value, xnew, cval[:self.m], it.value, pit.value
 
     def pcg(self, x_point, mu, b, tol=1e-6, maxiter=100):
-        """pcg! on (J'J + mu I) x = b with J = jac(x_point) -> (x, r, flag, iters)"""
-        xp = np.ascontiguousarray(x_point, dtype=np.float64); b = np.ascontiguousarray(b, dtype=np.float64)
-        x = np.empty(self.n_loc); r = np.empty(self.n_loc); fl = C.c_int(0); it = C.c_int64(0)
+        """pcg! on (J'J + mu I) x = b with J = jac(x_point), or with bounds on (bigA bigA' + mu I) x = b -> (x, r, flag, iters)"""
+        xp = self._working(x_point, "x_point"); b = self._working(b, "b")
+        x = np.empty_like(xp); r = np.empty_like(xp); fl = C.c_int(0); it = C.c_int64(0)
         self.ctx.check(self.ctx.lib.lfpsqp_large_pcg(self.ctx.h, _lib.ptr(xp), mu, _lib.ptr(b), tol, maxiter, _lib.ptr(x), _lib.ptr(r),
                                                      C.cast(C.pointer(fl), C.c_void_p), C.cast(C.pointer(it), C.c_void_p)))
         return x, r, fl.value, it.value
@@ -119,9 +142,12 @@ class LargeProblem:
         return dict(sol=sol, lam=lout[:self.m], iters=it.value, nr=nr.value, status=st.value)
 
     def projcg(self, x, lam=None, tol=0.0, maxit=10, chunk=0, want_solution=True):
-        x = np.ascontiguousarray(x, dtype=np.float64)
+        """projcg! at x with multipliers lam (m, or [lambda ; lambda_y] of m + n_loc entries with bounds); needs factor(x) first"""
+        x = self._working(x, "x")
         lam = None if lam is None else np.ascontiguousarray(lam, dtype=np.float64)
-        sol = np.empty(self.n_loc) if want_solution else None
+        if lam is not None and lam.shape != (self.m + x.size - self.n_loc,):
+            raise _lib.LFPSQPError("lam must have %d entries, not %s" % (self.m + x.size - self.n_loc, lam.shape))
+        sol = np.empty_like(x) if want_solution else None
         it = C.c_int64(0); nr = C.c_double(0); st = C.c_int(0); ms = C.c_double(0)
         self.ctx.check(self.ctx.lib.lfpsqp_large_projcg(self.ctx.h, _lib.ptr(x), _lib.ptr(lam), tol, maxit, chunk, _lib.ptr(sol),
                                                         C.cast(C.pointer(it), C.c_void_p), C.cast(C.pointer(nr), C.c_void_p),
