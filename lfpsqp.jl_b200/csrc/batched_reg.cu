@@ -8,10 +8,10 @@
 using namespace lfpsqp;
 
 namespace {
-template <class Fam, int LW, int NPL, int ME, bool INEQ, bool SPARSE, int MINB = 3>
+template <class Fam, int LW, int NPL, int ME, bool INEQ, bool SPARSE, int HEAD = 0, int MINB = 3>
 int launch(lfpsqp_ctx *c, BatchedArgs &A) {
-  using RS = RegSolver<Fam, LW, NPL, ME, INEQ, SPARSE>;
-  auto kern = batched_reg_kernel<Fam, LW, NPL, ME, INEQ, SPARSE, MINB>;
+  using RS = RegSolver<Fam, LW, NPL, ME, INEQ, SPARSE, HEAD>;
+  auto kern = batched_reg_kernel<Fam, LW, NPL, ME, INEQ, SPARSE, HEAD, MINB>;
   constexpr int GROUPS = REG_NT / LW;   // instances in flight per CTA
   const size_t smem = (size_t)((INEQ ? 5 * RS::NAP : 0) + GROUPS * RS::STASH_DOUBLES) * 8;
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -30,6 +30,13 @@ bool sparse_ok(const lfpsqp_ctx *c, int NA, int LW) {
   for (int j = 0; j < NA; j++) if (c->bnd_host[j] != 0.0 && ++cnt[j % LW] > 1) return false;
   return true;
 }
+
+// line head: do slots 0 .. HEAD-1 (elements j < HEAD LW) hold only line pairs (kind 0; padding past N_A is zero)?
+bool line_head_ok(const lfpsqp_ctx *c, int NA, int HEAD, int LW) {
+  if ((int)c->bnd_host.size() < NA) return false;
+  for (int j = 0; j < NA && j < HEAD * LW; j++) if (c->bnd_host[j] != 0.0) return false;
+  return true;
+}
 }  // namespace
 
 // returns LFPSQP_OK when launched, 1 when this problem shape has no register-resident instantiation (caller falls
@@ -44,7 +51,10 @@ int launch_batched_reg(lfpsqp_ctx *c, BatchedArgs &A) {
       if (ME != 1 || !A.ineq) return 1;
       if (NA <= 32) return launch<SepReadmeIneq, 16, 2, 1, true, false>(c, A);
       if (NA <= 64) {
-        if (NA <= 56 && sparse_ok(c, NA, 8)) return launch<SepReadmeIneq, 8, 7, 1, true, true, 2>(c, A);
+        if (NA <= 56 && sparse_ok(c, NA, 8)) {
+          if (line_head_ok(c, NA, 6, 8)) return launch<SepReadmeIneq, 8, 7, 1, true, true, 6, 2>(c, A);
+          return launch<SepReadmeIneq, 8, 7, 1, true, true, 0, 2>(c, A);
+        }
         return launch<SepReadmeIneq, 16, 4, 1, true, false>(c, A);
       }
       if (NA <= 128) return launch<SepReadmeIneq, 32, 4, 1, true, false>(c, A);

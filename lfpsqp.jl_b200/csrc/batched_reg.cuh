@@ -29,7 +29,10 @@
 // Alternatives measured against this kernel on a B200 (C2, LW = 8: 1.687 ms for 65,536 instances) and dropped: bit masks
 // for "slot holds a user variable / a slack" instead of index compares 1.82 ms; the line formula for every slot plus one
 // fix-up branch per lane 1.76 ms; pcg!'s dx accumulated in the stash 2.04 ms; family parameters re-read through the L1
-// instead of cached in registers 1.72 ms (profiles/r2_c2_ab_feature_switches.log).
+// instead of cached in registers 1.72 ms (profiles/r2_c2_ab_feature_switches.log).  With the line head (HEAD = NPL - 1,
+// 1.389 ms): user-variable and line-gradient facts made compile-time in the head slots as well 1.288 ms, but the
+// constants change how the compiler contracts those slots' expressions into FMAs (results differ in the last bits);
+// the head at 168 registers (MINB = 3) spills 1.4 KB and is slower, 1.76 ms (profiles/r3_c2_line_head_ab.log).
 
 namespace lfpsqp {
 
@@ -106,7 +109,12 @@ template <int LW> LFPSQP_DEV void gmax_sum2(unsigned mask, double &mx, double &a
   }
 }
 
-template <class Fam, int LW, int NPL, int ME, bool INEQ, bool SPARSE>
+// HEAD: slots 0 .. HEAD-1 of every lane hold only line pairs (bound kind 0, q = r = s = t = 0; checked by the
+// launcher).  There the bound kind and the bound table are compile-time, so calculate_h is x - y, inequality_gradient,
+// y_retract_elem and generate_initial_y take the line branch, and the parabola / circle code and the table reads are not
+// emitted.  The line gradients and the user / slack tests stay runtime values in every slot: that keeps every
+// expression compiled as with HEAD = 0 (same FMA contraction, bitwise-identical results).
+template <class Fam, int LW, int NPL, int ME, bool INEQ, bool SPARSE, int HEAD>
 struct RegSolver {
   static constexpr int KP = Fam::KP > 0 ? Fam::KP : 1;
   static constexpr int MEA = ME > 0 ? ME : 1;
@@ -115,6 +123,7 @@ struct RegSolver {
   static constexpr int NGR = SPARSE ? 1 : NPL;
   enum { SV_X = 0, SV_D, SV_XTIL, SV_XNEW, SV_GV, SV_COUNT };
   static constexpr int STASH_DOUBLES = SV_COUNT * VECD;      // per group
+  static constexpr int GPW = 32 / LW;                        // groups per warp
   struct Vec { double x[NPL]; double y[INEQ ? NPL : 1]; };
 
   const int lane;        // lane within the group
@@ -127,7 +136,7 @@ struct RegSolver {
   const double *bnd;
   unsigned kinds;        // 2 bits per slot: this lane's bound kinds (bkind without the shared-memory read)
   double pcg_rho_stop;   // largest rho with sqrt(rho) <= eps_c: pcg!'s test norm(r) > tol (retractions.jl:207) without the sqrt
-  double *stash;         // this group's parking area
+  double *stash;         // this lane's first element in its warp's parking area (see sx)
   double ep[NPL][KP];    // cached per-element family parameters
   // instance state
   Vec x;
@@ -168,19 +177,21 @@ struct RegSolver {
   LFPSQP_DEV void eload(int k, double *e) const {   // family parameters of user slot k
     LF_UNROLL for (int q = 0; q < KP; q++) e[q] = ep[k][q];
   }
-  LFPSQP_DEV int bkind(int k) const { return INEQ ? (int)((kinds >> (2 * k)) & 3u) : 0; }
-  LFPSQP_DEV double bq(int k) const { return INEQ ? bnd[NAP + idx(k)] : 0.0; }
-  LFPSQP_DEV double br(int k) const { return INEQ ? bnd[2 * NAP + idx(k)] : 0.0; }
-  LFPSQP_DEV double bs(int k) const { return INEQ ? bnd[3 * NAP + idx(k)] : 0.0; }
-  LFPSQP_DEV double bt(int k) const { return INEQ ? bnd[4 * NAP + idx(k)] : 0.0; }
+  LFPSQP_DEV int bkind(int k) const { return (INEQ && k >= HEAD) ? (int)((kinds >> (2 * k)) & 3u) : 0; }
+  LFPSQP_DEV double bq(int k) const { return (INEQ && k >= HEAD) ? bnd[NAP + idx(k)] : 0.0; }
+  LFPSQP_DEV double br(int k) const { return (INEQ && k >= HEAD) ? bnd[2 * NAP + idx(k)] : 0.0; }
+  LFPSQP_DEV double bs(int k) const { return (INEQ && k >= HEAD) ? bnd[3 * NAP + idx(k)] : 0.0; }
+  LFPSQP_DEV double bt(int k) const { return (INEQ && k >= HEAD) ? bnd[4 * NAP + idx(k)] : 0.0; }
   LFPSQP_DEV double sum(double v) const { return gsum<LW>(gmask, v); }
   LFPSQP_DEV double maxr(double v) const { return gmax<LW>(gmask, v); }
   LFPSQP_DEV void sum2(double &a, double &b) const { gsum2<LW>(gmask, a, b); }
   LFPSQP_DEV void sum3(double &a, double &b, double &c) const { gsum3<LW>(gmask, a, b, c); }
 
   // ---------------------------------------------------------------- stash (group-private shared memory, lane-private elements)
-  LFPSQP_DEV double &sx(int v, int k) const { return stash[v * VECD + idx(k)]; }
-  LFPSQP_DEV double &sy(int v, int k) const { return stash[v * VECD + NAP + idx(k)]; }
+  // element e = v VECD + idx(k) of a group's area sits at (e - lane) GPW + group_in_warp LW + lane of its warp's area:
+  // the groups of a warp are interleaved, so one access by the warp covers 32 consecutive doubles (no bank conflict)
+  LFPSQP_DEV double &sx(int v, int k) const { return stash[(v * VECD + k * LW) * GPW]; }
+  LFPSQP_DEV double &sy(int v, int k) const { return stash[(v * VECD + NAP + k * LW) * GPW]; }
   LFPSQP_DEV void put(int v, const Vec &a) const {
     LF_UNROLL for (int k = 0; k < NPL; k++) { sx(v, k) = a.x[k]; if (INEQ) sy(v, k) = a.y[k]; }
   }
@@ -823,11 +834,11 @@ struct RegSolver {
 // Persistent CTAs of REG_NT threads = REG_NT / LW lane groups; every group pulls instance indices from a global counter
 // until the batch is drained (absorbs the per-instance iteration-count variance).  The groups of a warp leave the loop
 // together.  MINB = resident CTAs per SM the register allocation is capped for (3 -> 168 registers, 2 -> 255).
-// SPARSE: see RegSolver.
+// SPARSE, HEAD: see RegSolver.
 constexpr int REG_NT = 128;
-template <class Fam, int LW, int NPL, int ME, bool INEQ, bool SPARSE, int MINB>
+template <class Fam, int LW, int NPL, int ME, bool INEQ, bool SPARSE, int HEAD, int MINB>
 __global__ void __launch_bounds__(REG_NT, MINB) batched_reg_kernel(const BatchedArgs A) {
-  using RS = RegSolver<Fam, LW, NPL, ME, INEQ, SPARSE>;
+  using RS = RegSolver<Fam, LW, NPL, ME, INEQ, SPARSE, HEAD>;
   extern __shared__ double smem[];
   const int lane32 = threadIdx.x & 31;
   int sub = lane32 % LW;
@@ -840,7 +851,7 @@ __global__ void __launch_bounds__(REG_NT, MINB) batched_reg_kernel(const Batched
     bnd[i] = (j < NA) ? A.bnd[a * NA + j] : 0.0;
   }
   __syncthreads();
-  double *stash = smem + NB + (size_t)(threadIdx.x / LW) * RS::STASH_DOUBLES;
+  double *stash = smem + NB + (size_t)(threadIdx.x / 32) * RS::GPW * RS::STASH_DOUBLES + lane32;
   RS S(sub, gmask, A.prm, A.n, A.m, A.p, bnd, stash);
   for (;;) {
     unsigned long long k = 0;
